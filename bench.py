@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo (hand-written sm_100a kernels)
     python bench.py --impl reference --gpus N --steps K ...  # the unmodified reference on the same box
+    python bench.py ... --dump-outputs DIR                   # + what the last timed env.step() returned, as DIR/<name>.npy
 
 One bench "step" = one RL ``env.step()`` of the whole batch = 25 solver (PISO) steps per environment incl.
 jet actuation, advective outflow update, drag/lift integration and sensor sampling.
@@ -195,6 +196,36 @@ def _restore(env, snap):
     env._n_steps = 0
 
 
+DUMP_BYTES = 64 << 20
+
+
+def _step_arrays(result):
+    """The arrays a caller receives from one env.step() -- observation, reward, terminated, truncated, info -- flattened to
+    host float arrays (float64 where float32 would round: double, integer and boolean values)."""
+    import torch
+    obs, reward, terminated, truncated, info = result
+    named = {"reward": reward, "terminated": terminated, "truncated": truncated}
+    named.update({f"obs_{k}": v for k, v in obs.items()} if isinstance(obs, dict) else {"obs": obs})
+    named.update({f"info_{k}": v for k, v in info.items()})
+    out = {}
+    for name, v in named.items():
+        a = v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else np.asarray(v)
+        out[name] = a.astype(np.float32 if a.dtype in (np.float16, np.float32) else np.float64)
+    return out
+
+
+def dump_outputs(arrays, path, tag=""):
+    """Writes ``path/<name><tag>.npy``.  Arrays are sampled at fixed, seeded flat positions where the whole set would exceed
+    DUMP_BYTES, so that two builds run with the same arguments write comparable files."""
+    os.makedirs(path, exist_ok=True)
+    budget = DUMP_BYTES // max(len(arrays), 1)
+    for name, a in sorted(arrays.items()):
+        if a.nbytes > budget:
+            keep = np.sort(np.random.default_rng(0).choice(a.size, budget // a.itemsize, replace=False))
+            a = a.reshape(-1)[keep]
+        np.save(os.path.join(path, f"{name}{tag}.npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------
 def extras(args, rank, world, local, dev):
     """Short records of the other BASELINE.json configs (kept bounded; failures are reported, never fatal):
@@ -316,7 +347,7 @@ def run_ours(args):
     e0.record()
     nsub = 0
     for i in range(args.steps):
-        env.step(actions_dev[args.warmup + i])
+        last = env.step(actions_dev[args.warmup + i])
         nsub += env.last_substeps
     e1.record()
     barrier(world)
@@ -328,6 +359,8 @@ def run_ours(args):
     ms = max_over_ranks(ms_local, world, dev)
     env_substeps = sum_over_ranks(B * nsub, world, dev)
     value = env_substeps / (ms / 1e3)
+    if args.dump_outputs:
+        dump_outputs(_step_arrays(last), args.dump_outputs, "" if world == 1 else f".rank{rank}")
 
     # ---- per-kernel durations for the roofline block: the same steps once more with ONE environment group, so that every
     #      launch runs alone on the GPU and its CUDA-event duration is the kernel's own (in the timed region above the
@@ -634,7 +667,14 @@ def main():
     ap.add_argument("--extra-rbc-envs", type=int, default=1024)
     ap.add_argument("--extra-airfoil-steps", type=int, default=10, help="env.step() of the differentiable airfoil rollout (5 solver steps each)")
     ap.add_argument("--extra-tcf-steps", type=int, default=10)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed env.step() returned (observation, reward, terminated, truncated, info) as "
+                         "DIR/<name>.npy; under torchrun every rank writes DIR/<name>.rank<r>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     # ONE line on stdout: libraries write banners to file descriptor 1 behind python's back (NCCL prints "NCCL version ..." there when
     # the process group comes up), so fd 1 points to stderr while the run is in progress and the JSON line goes to the real stdout

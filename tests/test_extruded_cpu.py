@@ -121,21 +121,11 @@ def test_wall_forces_per_plane_equal_the_reference_force_function(golden):
     """The 3-D cylinder's drag / lift (jet_cylinder_env_3d.py:441-470) are the 2-D wall-traction formula applied in every z plane
     with face areas = face length x plane spacing: our torch statement of k_wall_forces (envs/common.py::_forces_torch, the
     differentiable twin of the CUDA kernel) on the reference's traced 3-D state vs the reference's own ``compute_forces_3d``
-    (envs/util/forces.py:278-377, pure torch) evaluated on the CPU from the installed reference."""
-    import os
-    import sys
+    (envs/util/forces.py:278-377, pure torch) evaluated on the CPU from the installed reference (its stored values elsewhere:
+    tests/reference_values.py)."""
     import torch
-    from conftest import ROOT
-    if not os.path.isdir(os.path.join(ROOT, "baseline", "_ref", "fluidgym")):
-        pytest.skip("unmodified reference not installed (baseline/_ref)")
-    sys.path.insert(0, os.path.join(ROOT, "oracle"))
-    import ref_shims
-    ref_shims.install()
-    try:
-        import fluidgym  # noqa: F401
-        from fluidgym.envs.util.forces import compute_forces_3d
-    except Exception as e:
-        pytest.skip(f"reference not importable here: {e}")
+    import reference_values
+    forces = reference_values.module("fluidgym.envs.util.forces")
     from fluidgym_b200.envs.common import DifferentiableRollout, build_wall_tables
     from fluidgym_b200.envs.cylinder import CylinderJet2DEnv
     from fluidgym_b200.envs.cylinder_domain import make_cylinder_domain
@@ -149,10 +139,11 @@ def test_wall_forces_per_plane_equal_the_reference_force_function(golden):
     u, p, bv = torch.from_numpy(fx["env0_u"]), torch.from_numpy(fx["env0_p"]), torch.from_numpy(fx["env0_bvel"])
     nz, hz = u.shape[1], 0.5
     cell, bface = tab["cell"].long(), tab["bface"].long()
-    ref = compute_forces_3d(u[:, :, cell], bv[:, :, bface], p[:, cell], tab["normal"][:, :, None], tab["tlen"][:, None], tab["dist"][:, None],
-                            tab["flen"] * hz, torch.tensor(float(cd.visc)))                                     # [2, nz]
     env.wall = type("W", (), {"scale": 1.0})()
     mine = torch.stack([DifferentiableRollout._forces_torch(env, u[:, k][None], p[k][None], bv[:, k][None])[0] for k in range(nz)], dim=1) * hz
+    ref = reference_values.value("cylinder3d_wall_forces", forces and (lambda: forces.compute_forces_3d(
+        u[:, :, cell], bv[:, :, bface], p[:, cell], tab["normal"][:, :, None], tab["tlen"][:, None], tab["dist"][:, None],
+        tab["flen"] * hz, torch.tensor(float(cd.visc)))), mine)                                                  # [2, nz]
     assert float(ref.abs().max()) > 1e-2
     assert torch.allclose(mine, ref, rtol=2e-5, atol=1e-6)
 

@@ -1,14 +1,11 @@
 """Moving-window extraction of the multi-agent environments: the cases of the reference's own test file
 (tests/env_utils/test_obs_extraction.py: parametrisations and the property each one checks) applied to the batched
-implementations, plus -- when the unmodified reference is importable here (baseline/_ref, CPU only) -- equality with the
-reference's functions on random fields."""
-import os
-import sys
-
+implementations, plus equality with the reference's functions on random fields (called where the unmodified reference is
+installed, baseline/_ref, CPU only; their stored values elsewhere: tests/reference_values.py)."""
 import pytest
 import torch
 
-from conftest import ROOT
+import reference_values
 from fluidgym_b200.envs.rbc import extract_moving_window_2d
 from fluidgym_b200.envs.rbc3d import extract_moving_window_3d
 from fluidgym_b200.envs.tcf import agent_window_means
@@ -57,51 +54,55 @@ def test_moving_window_2d_x_z(nax, naz, aw, wx, wz, pad_x, pad_z):
     assert torch.allclose(res[pad_x * naz + pad_z], expected)
 
 
-def _reference():
-    if not os.path.isdir(os.path.join(ROOT, "baseline", "_ref", "fluidgym")):
-        pytest.skip("unmodified reference not installed (baseline/_ref)")
-    sys.path.insert(0, os.path.join(ROOT, "oracle"))
-    import ref_shims
-    ref_shims.install()
-    try:
-        import fluidgym  # noqa: F401
-        from fluidgym.envs.util import obs_extraction
-    except Exception as e:  # the compiled extension may not load on a machine without the CUDA runtime libraries
-        pytest.skip(f"reference not importable here: {e}")
-    return obs_extraction
+def _positions(field, out):
+    """where in ``field`` each value of ``out`` comes from: the moving windows only move values, and the values of a random field
+    are distinct, so equality with ``field.flatten()[_positions(field, out)]`` is equality with ``out``"""
+    flat = field.reshape(-1)
+    assert flat.numel() <= 2 ** 15                                # stored as int16
+    order = torch.argsort(flat)
+    pos = order[torch.searchsorted(flat[order], out.reshape(-1)).clamp(max=flat.numel() - 1)]
+    assert torch.equal(flat[pos], out.reshape(-1))
+    return pos.reshape(out.shape).to(torch.int16)
 
 
 def test_equal_to_the_reference_functions():
-    ox = _reference()
+    ox = reference_values.module("fluidgym.envs.util.obs_extraction")
     torch.manual_seed(1)
     for n, w, k in ((8, 12, 1), (8, 12, 3), (12, 8, 11)):
         f = torch.rand(3, 10, n * w)
         mine = extract_moving_window_2d(f, n, w, k)
         for b in range(3):
-            assert torch.equal(mine[b], ox.extract_moving_window_2d(f[b], n_agents=n, agent_width=w, n_agents_per_window=k))
+            pos = reference_values.value(f"window_2d_{n}_{w}_{k}_{b}", ox and (lambda: _positions(f[b], ox.extract_moving_window_2d(
+                f[b], n_agents=n, agent_width=w, n_agents_per_window=k))), _positions(f[b], mine[b]))
+            assert torch.equal(mine[b], f[b].reshape(-1)[pos.long()])
     for nax, naz, aw, wx, wz, px, pz in ((10, 20, 2, 1, 1, 0, 0), (20, 40, 2, 5, 3, 4, 1), (10, 20, 4, 5, 5, 4, 4), (8, 8, 2, 3, 3, 1, 1)):
         f = torch.rand(2, naz * aw, nax * aw)
         mine = agent_window_means(f, nax, naz, aw, wx, wz, px, pz)
         for b in range(2):
-            ref = ox.extract_moving_window_2d_x_z(field=f[b], n_agents_x=nax, n_agents_z=naz, agent_width=aw, n_agents_per_window_x=wx,
-                                                  n_agents_per_window_z=wz, pad_x=px, pad_z=pz)
+            ref = reference_values.value(f"window_2d_x_z_{nax}_{naz}_{aw}_{wx}_{wz}_{px}_{pz}_{b}", ox and (lambda: ox.extract_moving_window_2d_x_z(
+                field=f[b], n_agents_x=nax, n_agents_z=naz, agent_width=aw, n_agents_per_window_x=wx, n_agents_per_window_z=wz,
+                pad_x=px, pad_z=pz)), mine[b])
             assert torch.allclose(mine[b], ref, atol=1e-7)
     for n, w, k in ((4, 3, 1), (4, 3, 3), (6, 2, 5), (8, 4, 3)):
         f = torch.rand(2, n * w, 7, n * w)
         mine = extract_moving_window_3d(f, n, w, k)
         for b in range(2):
-            assert torch.equal(mine[b], ox.extract_moving_window_3d(f[b], n_agents=n, agent_width=w, n_agents_per_window=k))
+            pos = reference_values.value(f"window_3d_{n}_{w}_{k}_{b}", ox and (lambda: _positions(f[b], ox.extract_moving_window_3d(
+                f[b], n_agents=n, agent_width=w, n_agents_per_window=k))), _positions(f[b], mine[b]))
+            assert torch.equal(mine[b], f[b].reshape(-1)[pos.long()])
 
 
 def test_spanwise_local_windows_equal_the_reference():
     """transform_global_to_local_obs_3d (CylinderJet3D / Airfoil3D multi-agent observations)"""
-    ox = _reference()
+    ox = reference_values.module("fluidgym.envs.util.obs_extraction")
     from fluidgym_b200.envs.spanwise import local_obs_windows
     torch.manual_seed(2)
     for n_agents, window in ((8, 3), (8, 1), (6, 5)):
         g = {"velocity": torch.rand(2, n_agents, 2, 3, 11), "pressure": torch.rand(2, n_agents, 2, 11)}
         mine = local_obs_windows(g, window)
         for b in range(2):
-            ref = ox.transform_global_to_local_obs_3d({k: v[b] for k, v in g.items()}, local_obs_window=window, n_agents=n_agents)
+            ref = ox and ox.transform_global_to_local_obs_3d({k: v[b] for k, v in g.items()}, local_obs_window=window, n_agents=n_agents)
             for k in g:
-                assert torch.equal(mine[k][b], ref[k]), (n_agents, window, k)
+                pos = reference_values.value(f"local_obs_{n_agents}_{window}_{b}_{k}", ref and (lambda: _positions(g[k][b], ref[k])),
+                                             _positions(g[k][b], mine[k][b]))
+                assert torch.equal(mine[k][b], g[k][b].reshape(-1)[pos.long()]), (n_agents, window, k)

@@ -1,30 +1,18 @@
 """The static sensor maps (fluidgym_b200/sensors.py) against the reference's own torch re-implementation of its resampling
 kernel (simulation/pict/data/resample.py:361-549, the function its test tests/simulation/test_torch_resample.py compares the
-CUDA kernel with at atol = rtol = 1e-3), run on the CPU from the installed unmodified reference (baseline/_ref).  Skipped where
-the reference is not installed; the GPU goldens (tests/golden/*_steps.npz observations) pin the same maps independently."""
-import os
-import sys
-
+CUDA kernel with at atol = rtol = 1e-3), run on the CPU from the installed unmodified reference (baseline/_ref); its stored values
+where the reference is not installed (tests/reference_values.py).  The GPU goldens (tests/golden/*_steps.npz observations) pin the
+same maps independently."""
 import numpy as np
 import pytest
 import torch
 
-from conftest import ROOT
+import reference_values
 
 
 @pytest.fixture(scope="module")
 def resample():
-    if not os.path.isdir(os.path.join(ROOT, "baseline", "_ref", "fluidgym")):
-        pytest.skip("unmodified reference not installed (baseline/_ref)")
-    sys.path.insert(0, os.path.join(ROOT, "oracle"))
-    import ref_shims
-    ref_shims.install()
-    try:
-        import fluidgym  # noqa: F401
-        from fluidgym.simulation.pict.data import resample as rs
-    except Exception as e:
-        pytest.skip(f"reference not importable here: {e}")
-    return rs
+    return reference_values.module("fluidgym.simulation.pict.data.resample")
 
 
 def test_2d_sensor_tables_equal_the_rendered_pixels(resample):
@@ -42,11 +30,12 @@ def test_2d_sensor_tables_equal_the_rendered_pixels(resample):
     rng = np.random.default_rng(0)
     field = rng.standard_normal((3, info["ny"], info["nx"])).astype(np.float32)
     mine = (w[None] * field.reshape(3, -1)[:, idx]).sum(axis=1)                                   # [3, n_sensors]
-    ref = resample.sample_multi_coords_to_uniform_grid([torch.from_numpy(field)[None]], [torch.from_numpy(vertex)[None]], [nx, ny],
-                                                       fill_max_steps=16, differentiable=True)[0].numpy()      # [3, H, W]
+    ref = reference_values.value("resample_2d_sensors", resample and (lambda: resample.sample_multi_coords_to_uniform_grid(
+        [torch.from_numpy(field)[None]], [torch.from_numpy(vertex)[None]], [nx, ny], fill_max_steps=16,
+        differentiable=True)[0][:, px[1], px[0]]), mine)                                    # [3, H, W] -> [3, n_sensors]
     # white-noise field of unit variance; the torch path computes the voxel coordinates in float64, the kernel (and the map) in
     # float32: observed 2.3e-5 (the reference's own bar between its two implementations is 1e-3)
-    assert np.abs(mine - ref[:, px[1], px[0]]).max() < 1e-4
+    assert np.abs(mine - ref).max() < 1e-4
 
 
 def test_3d_pixel_map_equals_the_trilinear_torch_path(resample, golden):
@@ -60,8 +49,13 @@ def test_3d_pixel_map_equals_the_trilinear_torch_path(resample, golden):
     rng = np.random.default_rng(1)
     field = rng.standard_normal((2, 16, 10, 16)).astype(np.float32)
     mine = (R8 @ field.reshape(2, -1).T.astype(np.float64)).T.reshape(2, Z, H, W)
-    ref = resample.sample_multi_coords_to_uniform_grid([torch.from_numpy(field)[None]], [torch.from_numpy(vertex)[None]], [W, H, Z],
-                                                       fill_max_steps=16, differentiable=True)[0].numpy()
-    assert np.abs(mine - ref).max() < 1e-4
+    ref = resample and resample.sample_multi_coords_to_uniform_grid([torch.from_numpy(field)[None]], [torch.from_numpy(vertex)[None]],
+                                                                    [W, H, Z], fill_max_steps=16, differentiable=True)[0].numpy()
+    assert ref is None or np.abs(mine - ref).max() < 1e-4
+    # stored: a fixed sample of 2048 voxels (all 160 000 would be 1.3 MB)
+    vox = np.sort(np.random.default_rng(3).choice(Z * H * W, 2048, replace=False))
+    mine_s = mine.reshape(2, -1)[:, vox].astype(np.float32)
+    ref_s = reference_values.value("resample_3d_voxel_sample", ref is not None and (lambda: ref.reshape(2, -1)[:, vox]), mine_s)
+    assert np.abs(mine_s - ref_s).max() < 1e-4
     R6, _ = pixel_map_3d(vertex, (W, H, Z), 16)
     assert R6.nnz < R8.nnz and abs((R6 - R8)).max() > 1e-3          # the kernel's 6-corner splat is a different map
