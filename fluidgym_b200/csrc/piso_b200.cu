@@ -2892,6 +2892,117 @@ __global__ void k_sample_sensors(const float *__restrict__ field, int C, int N, 
     out[((size_t)b * C + c) * ns + s] = v;
 }
 
+// rendering (fluidgym_b200/render.py): the full static render map as CSR, rows in image order.  One thread per (pixel,
+// environment), the environment in blockIdx.y so that the tables are read by the whole batch from L2.
+#define RENDER_THREADS 256
+// order-preserving float -> uint32 key (a < b <=> key(a) < key(b)); the range slots hold min key(v) and min ~key(v) so that a
+// single 0xff memset initialises both and both are atomicMin
+__device__ __forceinline__ unsigned int render_key(float v) {
+    const unsigned int u = __float_as_uint(v);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float render_unkey(unsigned int k) {
+    return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
+}
+
+__global__ void __launch_bounds__(RENDER_THREADS) k_render_gather(const float *__restrict__ field, int C, long long chan_stride,
+                                                                  long long env_stride, int mode, const int32_t *__restrict__ rowptr,
+                                                                  const int32_t *__restrict__ col, const float *__restrict__ w, int P,
+                                                                  float *__restrict__ img, unsigned int *__restrict__ range) {
+    const int b = blockIdx.y;
+    const int p = blockIdx.x * RENDER_THREADS + threadIdx.x;
+    float v = 0.f;
+    if (p < P) {
+        const float *f = field + (size_t)b * env_stride;
+        float a[3] = {0.f, 0.f, 0.f};
+        const int k1 = rowptr[p + 1];
+        for (int k = rowptr[p]; k < k1; ++k) {
+            const long long c0 = col[k];
+            const float ww = w[k];
+#pragma unroll
+            for (int c = 0; c < 3; ++c)
+                if (c < C) a[c] += ww * f[c * chan_stride + c0];
+        }
+        v = (mode == FGB_RENDER_NORM) ? sqrtf(a[0] * a[0] + a[1] * a[1] + a[2] * a[2]) : a[0];
+        img[(size_t)b * P + p] = v;
+    }
+    if (!range) return;                                          // uniform over the grid
+    unsigned int lo = 0xffffffffu, hi = 0xffffffffu;
+    if (p < P) { lo = render_key(v); hi = ~lo; }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        lo = min(lo, __shfl_xor_sync(0xffffffffu, lo, o));
+        hi = min(hi, __shfl_xor_sync(0xffffffffu, hi, o));
+    }
+    __shared__ unsigned int red[2][RENDER_THREADS / 32];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (lane == 0) { red[0][warp] = lo; red[1][warp] = hi; }
+    __syncthreads();
+    if (warp == 0) {
+        lo = lane < RENDER_THREADS / 32 ? red[0][lane] : 0xffffffffu;
+        hi = lane < RENDER_THREADS / 32 ? red[1][lane] : 0xffffffffu;
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            lo = min(lo, __shfl_xor_sync(0xffffffffu, lo, o));
+            hi = min(hi, __shfl_xor_sync(0xffffffffu, hi, o));
+        }
+        if (lane == 0) { atomicMin(&range[2 * b], lo); atomicMin(&range[2 * b + 1], hi); }
+    }
+}
+
+// LUT bin of v in [lo, hi]: floor(256 (v - lo) / (hi - lo)) clamped to [0, 255] (NaN -> 0), 128 for an empty range
+__device__ __forceinline__ int render_bin(float v, float lo, float hi) {
+    const float t = hi > lo ? (v - lo) / (hi - lo) : 0.5f;
+    return (int)fminf(fmaxf(t * 256.f, 0.f), 255.f);
+}
+
+// rgb[B*P][3] uint8 from img[B*P] through a 256-entry LUT in shared memory; one thread per 4 consecutive pixels of the flattened
+// batch, whose 12 bytes go out as 3 aligned uint32 stores
+__global__ void __launch_bounds__(RENDER_THREADS) k_render_colour(const float *__restrict__ img, int P, long long total,
+                                                                  const unsigned int *__restrict__ range, float vmin, float vmax,
+                                                                  int symmetric, const uint8_t *__restrict__ lut,
+                                                                  uint8_t *__restrict__ rgb) {
+    __shared__ unsigned int s_lut[256];
+    for (int i = threadIdx.x; i < 256; i += RENDER_THREADS)
+        s_lut[i] = (unsigned int)lut[3 * i] | ((unsigned int)lut[3 * i + 1] << 8) | ((unsigned int)lut[3 * i + 2] << 16);
+    __syncthreads();
+    const long long i0 = 4 * ((long long)blockIdx.x * RENDER_THREADS + threadIdx.x);
+    if (i0 >= total) return;
+    const bool full = i0 + 4 <= total;
+    float v[4];
+    if (full) {
+        const float4 q = *reinterpret_cast<const float4 *>(img + i0);
+        v[0] = q.x; v[1] = q.y; v[2] = q.z; v[3] = q.w;
+    } else {
+        for (int j = 0; j < 4; ++j) v[j] = i0 + j < total ? img[i0 + j] : 0.f;
+    }
+    unsigned int c[4];
+    int bprev = -1;
+    float lo = vmin, hi = vmax;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+        c[j] = 0u;
+        if (i0 + j >= total) continue;
+        const int b = (int)((i0 + j) / P);
+        if (b != bprev) {
+            bprev = b;
+            if (range) { lo = render_unkey(range[2 * b]); hi = render_unkey(~range[2 * b + 1]); }
+            else { lo = vmin; hi = vmax; }
+            if (symmetric) { hi = fmaxf(fabsf(lo), fabsf(hi)); lo = -hi; }
+        }
+        c[j] = s_lut[render_bin(v[j], lo, hi)];
+    }
+    if (full) {
+        unsigned int *o = reinterpret_cast<unsigned int *>(rgb + 3 * i0);
+        o[0] = c[0] | (c[1] << 24);
+        o[1] = (c[1] >> 8) | (c[2] << 16);
+        o[2] = (c[2] >> 16) | (c[3] << 8);
+    } else {
+        for (int j = 0; i0 + j < total; ++j)
+            for (int k = 0; k < 3; ++k) rgb[3 * (i0 + j) + k] = (uint8_t)(c[j] >> (8 * k));
+    }
+}
+
 // ------------------------------------------------------------------------------------------------
 // Reverse-mode adjoint of one PISO substep (replaces the *_GRAD kernels K.cu:3884-4090, 4403-4491,
 // 4982-5130, 5258-5385, 5438-5509, 6265-6309 and the python glue DIFF.py:516-1808).  Specification:
@@ -3965,6 +4076,36 @@ extern "C" int fgb_sample_sensors_n(const float *field, int32_t B, int32_t chann
     dim3 grid((channels * n_sensors + 127) / 128, B);
     k_sample_sensors<<<grid, 128, 0, STREAM(s)>>>(field, channels, N, idx, w, K, n_sensors, out);
     LAUNCH_CHECK("k_sample_sensors");
+    return FGB_OK;
+}
+
+extern "C" int fgb_render_gather(const float *field, int32_t B, int32_t channels, int32_t N, int64_t chan_stride, int64_t env_stride,
+                                 int32_t mode, const int32_t *rowptr, const int32_t *col, const float *w, int32_t P, float *img,
+                                 uint32_t *range, fgb_stream_t s) {
+    if (!field || !rowptr || !col || !w || !img || B <= 0 || B > 65535 || N <= 0 || P <= 0 || chan_stride < 0 || env_stride < 0)
+        return set_err(FGB_E_ARG, "fgb_render_gather: bad argument");
+    if (!((mode == FGB_RENDER_IDENTITY && channels == 1) || (mode == FGB_RENDER_NORM && channels >= 2 && channels <= 3)))
+        return set_err(FGB_E_ARG, "fgb_render_gather: mode IDENTITY takes 1 channel, NORM 2 or 3");
+    if (range) {
+        cudaError_t ce = cudaMemsetAsync(range, 0xff, sizeof(uint32_t) * 2 * (size_t)B, STREAM(s));
+        if (ce != cudaSuccess) return set_err(FGB_E_CUDA, "fgb_render_gather: range initialisation", ce);
+    }
+    dim3 grid((P + RENDER_THREADS - 1) / RENDER_THREADS, B);
+    k_render_gather<<<grid, RENDER_THREADS, 0, STREAM(s)>>>(field, channels, chan_stride, env_stride, mode, rowptr, col, w, P, img, range);
+    LAUNCH_CHECK("k_render_gather");
+    return FGB_OK;
+}
+
+extern "C" int fgb_render_colour(const float *img, int32_t B, int32_t P, const uint32_t *range, float vmin, float vmax,
+                                 int32_t symmetric, const uint8_t *lut, uint8_t *rgb, fgb_stream_t s) {
+    if (!img || !lut || !rgb || B <= 0 || P <= 0) return set_err(FGB_E_ARG, "fgb_render_colour: bad argument");
+    if ((reinterpret_cast<uintptr_t>(img) & 15) || (reinterpret_cast<uintptr_t>(rgb) & 3))
+        return set_err(FGB_E_ARG, "fgb_render_colour: img must be 16-byte and rgb 4-byte aligned");
+    const long long total = (long long)B * P;
+    const long long groups = (total + 3) / 4;
+    k_render_colour<<<(unsigned int)((groups + RENDER_THREADS - 1) / RENDER_THREADS), RENDER_THREADS, 0, STREAM(s)>>>(
+        img, P, total, range, vmin, vmax, symmetric, lut, rgb);
+    LAUNCH_CHECK("k_render_colour");
     return FGB_OK;
 }
 

@@ -16,7 +16,7 @@ from .. import native
 from ..sensors import sensor_tables
 from ..solver import BatchedPISO, _ptr
 from .airfoil_domain import BOT, FRONT, JET_CENTERS, JET_WIDTH, TAIL_LOWER, TAIL_UPPER, TOP, airfoil_polyline, make_airfoil_domain
-from .common import DifferentiableRollout, InitialDomains, build_wall_tables
+from .common import DifferentiableRollout, InitialDomains, Renderable, build_wall_tables
 from .cylinder_domain import jet_profile
 
 AIRFOIL_2D_DEFAULT_CONFIG = {
@@ -41,11 +41,12 @@ def polygon_mask(polygon_xy: np.ndarray, nx: int, ny: int) -> np.ndarray:
     return inside.reshape(ny, nx)
 
 
-class Airfoil2DEnv(DifferentiableRollout, InitialDomains):
+class Airfoil2DEnv(DifferentiableRollout, InitialDomains, Renderable):
     H, L, U_mean, airfoil_length = 1.4, 4.5, 0.3, 1.0
     n_jets = 3
     action_smoothing_alpha = 0.1
     render_shape = (600, 150)
+    render_fields = ("vorticity", "velocity_magnitude", "velocity_x", "velocity_y", "pressure")
     metrics = ["drag", "lift"]
     reference_values = {"cl_cd_ref": ("lift", "mean", "drag", "mean")}
     use_marl = False
@@ -126,6 +127,10 @@ class Airfoil2DEnv(DifferentiableRollout, InitialDomains):
         xy[0] = (xy[0] + 1.5) * (self.render_shape[0] / (self.L + 1.5))
         xy[1] = (xy[1] + self.H / 2) * (self.render_shape[1] / self.H)
         return torch.round(xy).to(torch.int32)
+
+    def _build_render_map(self, plane):
+        from ..render import render_map_2d
+        return render_map_2d([b.vertex for b in self.spec.blocks], self.render_shape, fill_max_steps=128)
 
     def sensor_locations_physical(self) -> torch.Tensor:
         """airfoil_env_base.py:607-656: coarse wake grid, fine near wake, box around the airfoil."""

@@ -32,6 +32,7 @@ AIRFOIL_3D_DEFAULT_CONFIG = {
 
 class Airfoil3DEnv(SpanwiseExtrudedEnv):
     H, L, D, U_mean, airfoil_length = 1.4, 4.5, 1.4, 0.3, 1.0
+    render_fill_steps = 128
     res_z = 96                                                          # airfoil_env_base.py:69
     n_jets = 3                                                          # jets per agent (airfoil_env_base.py:68)
     action_smoothing_alpha = 0.1

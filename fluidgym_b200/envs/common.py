@@ -168,6 +168,103 @@ class DifferentiableRollout:
         return u, p, bv, nsub
 
 
+_SIGNED_FIELDS = ("vorticity", "velocity_x", "velocity_y", "velocity_z", "pressure", "q_criterion")
+
+
+class Renderable:
+    """Mixin: batched images of the flow (the reference's ``render``, fluid_env.py:577-606, for every environment of the batch).
+
+    ``render_field`` resamples one field onto the family's image grid with the static render map of ``fluidgym_b200.render``
+    (``fgb_render_gather``); ``render`` colours it (``fgb_render_colour``): signed fields with the diverging map over a range
+    symmetric about zero, magnitudes and temperature with the sequential one, each environment over its own range unless
+    ``vmin`` / ``vmax`` fix one for the batch.  Both run on the solver's stream under ``no_grad`` and read the solver state
+    only.  The map is built on the first call for a plane and kept by the instance.  ``vorticity`` is the physical omega
+    = dv/dx - du/dy (the reference's 2-D renderer shows -omega).
+
+    A family sets ``render_fields`` (the first is the default) and ``_build_render_map(plane)``; 3-D families also
+    ``_render_planes()`` -> (number of planes, default plane).  Needs ``solver`` (u, p, optionally T / vorticity() /
+    q_criterion()), ``n_envs``, ``device``."""
+
+    render_fields: tuple = ()
+
+    def _render_planes(self):
+        return None
+
+    def _build_render_map(self, plane):
+        raise NotImplementedError
+
+    def _render_map(self, plane):
+        planes = self._render_planes()
+        if planes is None:
+            if plane is not None:
+                raise ValueError(f"{type(self).__name__} renders its 2-D domain: plane must be None, got {plane!r}")
+        else:
+            n, default = planes
+            plane = default if plane is None else plane
+            if not isinstance(plane, (int, np.integer)) or not 0 <= plane < n:
+                raise ValueError(f"plane {plane!r} out of range: valid planes of {type(self).__name__} are 0 .. {n - 1}")
+            plane = int(plane)
+        cache = self.__dict__.setdefault("_render_maps", {})
+        if plane not in cache:
+            m = self._build_render_map(plane)
+            cache[plane] = (tuple(torch.from_numpy(a).to(self.device) for a in (m.rowptr, m.col, m.w)), m.shape)
+        return cache[plane]
+
+    def _render_source(self, field):
+        """-> ([B, C, N] strided view of the field, fgb_render_gather mode)"""
+        from ..render import IDENTITY, NORM
+        if field is None:
+            field = self.render_fields[0]
+        if field not in self.render_fields:
+            raise ValueError(f"unknown render field {field!r}: {type(self).__name__} renders {self.render_fields}")
+        s = self.solver
+        if field == "velocity_magnitude":
+            return s.u, NORM
+        if field.startswith("velocity_"):
+            c = "xyz".index(field[-1])
+            return s.u[:, c:c + 1], IDENTITY
+        src = {"pressure": lambda: s.p, "temperature": lambda: s.T, "vorticity": lambda: s.vorticity(),
+               "q_criterion": lambda: s.q_criterion()}[field]()
+        return src.reshape(self.n_envs, 1, -1), IDENTITY
+
+    def _render_gather(self, field, plane, with_range: bool):
+        with torch.no_grad():
+            src, mode = self._render_source(field)
+            (rowptr, col, w), (H, W) = self._render_map(plane)
+            B, Cn, N = src.shape
+            if src.stride(2) != 1:
+                src = src.contiguous()
+            img = torch.empty(B, H, W, device=self.device)
+            rng = torch.empty(B, 2, dtype=torch.int32, device=self.device) if with_range else None
+            s = self.solver
+            native.check(s.lib.fgb_render_gather(_ptr(src), B, Cn, N, src.stride(1), src.stride(0), mode, _ptr(rowptr), _ptr(col), _ptr(w),
+                                                 H * W, _ptr(img), _ptr(rng), s.stream), "fgb_render_gather")
+        return img, rng
+
+    def render_field(self, field=None, *, plane=None) -> torch.Tensor:
+        """float32 [B, H, W] on the environment's device: ``field`` (default ``render_fields[0]``) resampled onto the image grid;
+        3-D families show the slice ``plane``."""
+        return self._render_gather(field, plane, False)[0]
+
+    def render(self, field=None, *, plane=None, vmin=None, vmax=None) -> torch.Tensor:
+        """uint8 [B, H, W, 3] on the environment's device: ``render_field`` coloured (see the class documentation)."""
+        from ..render import DIVERGING, SEQUENTIAL
+        if (vmin is None) != (vmax is None):
+            raise ValueError("render: give both vmin and vmax (a fixed range for the batch) or neither (each environment's own range)")
+        fixed = vmin is not None
+        img, rng = self._render_gather(field, plane, not fixed)
+        signed = (field or self.render_fields[0]) in _SIGNED_FIELDS
+        luts = self.__dict__.setdefault("_render_luts", {})
+        if signed not in luts:
+            luts[signed] = torch.from_numpy(DIVERGING if signed else SEQUENTIAL).to(self.device)
+        B, H, W = img.shape
+        rgb = torch.empty(B, H, W, 3, dtype=torch.uint8, device=self.device)
+        s = self.solver
+        native.check(s.lib.fgb_render_colour(_ptr(img), B, H * W, _ptr(rng), float(vmin) if fixed else 0.0, float(vmax) if fixed else 0.0,
+                                             int(signed and not fixed), _ptr(luts[signed]), _ptr(rgb), s.stream), "fgb_render_colour")
+        return rgb
+
+
 N_INITIAL_DOMAINS = 10      # envs/fluid_env.py:58
 
 

@@ -18,7 +18,7 @@ import torch
 from .. import native
 from ..sensors import sensor_tables
 from ..solver import BatchedPISO, _ptr
-from .common import DifferentiableRollout, InitialDomains, build_wall_tables
+from .common import DifferentiableRollout, InitialDomains, Renderable, build_wall_tables
 from .cylinder_domain import BOTTOM, LEFT, RIGHT, TOP, WAKE, jet_profile, make_cylinder_domain
 
 CYLINDER_ROT_2D_DEFAULT_CONFIG = {
@@ -82,13 +82,14 @@ def cylinder_sensor_locations(cylinder_diameter: float = 1.0) -> torch.Tensor:
     return torch.concatenate([loc, c1, c2, add], dim=1)
 
 
-class CylinderJet2DEnv(DifferentiableRollout, InitialDomains):
+class CylinderJet2DEnv(DifferentiableRollout, InitialDomains, Renderable):
     H, L, cylinder_diameter, U_mean, cylinder_offset_y = 4.1, 22.0, 1.0, 1.0, 0.05
     n_sensors = 151
     action_smoothing_alpha = 0.1
     jet_angle = 10.0
     metrics = ["drag", "lift"]
     reference_values = {"cd_ref": ("drag", "mean")}
+    render_fields = ("vorticity", "velocity_magnitude", "velocity_x", "velocity_y", "pressure")
     bc_tol = 5e-6            # flux-balance tolerance of the cylinder's outflow hook (cylinder_env_base.py:293-295: tol=5e-6, 2-D and 3-D)
 
     def __init__(self, n_envs: int = 1, reynolds_number=1e2, resolution=24, dt=1e-2, adaptive_cfl=0.8, step_length=0.25,
@@ -154,6 +155,10 @@ class CylinderJet2DEnv(DifferentiableRollout, InitialDomains):
 
     def sensor_locations_physical(self) -> torch.Tensor:
         return cylinder_sensor_locations(self.cylinder_diameter)
+
+    def _build_render_map(self, plane):
+        from ..render import render_map_2d
+        return render_map_2d([b.vertex for b in self.spec.blocks], self.render_shape, fill_max_steps=16)
 
     def _setup_sensors(self):
         pc = self.sensor_locations_physical()

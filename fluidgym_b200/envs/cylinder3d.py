@@ -16,7 +16,7 @@ import numpy as np
 import torch
 
 from ..sensors import sensor_tables_extruded
-from .common import DifferentiableRollout, InitialDomainsExtruded, build_wall_tables
+from .common import DifferentiableRollout, InitialDomainsExtruded, Renderable, build_wall_tables
 from .cylinder import cylinder_jet_templates, cylinder_sensor_locations
 from .cylinder_domain import BOTTOM, LEFT, RIGHT, TOP, WAKE, make_cylinder_domain
 from .spanwise import global_obs_from_samples, local_obs_windows, spanwise_sensor_voxels
@@ -27,7 +27,7 @@ CYLINDER_JET_3D_DEFAULT_CONFIG = {
 }
 
 
-class SpanwiseExtrudedEnv(InitialDomainsExtruded):
+class SpanwiseExtrudedEnv(InitialDomainsExtruded, Renderable):
     """What the environments on z-extruded domains with agents lined up along the span share (CylinderJet3D, Airfoil3D): the
     reference-shaped API, reset (zero field + inflow -> projection, or an on-disk initial domain), the solver-step loop with action
     smoothing, per-plane wall forces, voxel sensors, multi-agent windows and the local / global reward mix.  A subclass provides the
@@ -37,6 +37,16 @@ class SpanwiseExtrudedEnv(InitialDomainsExtruded):
     action_smoothing_alpha = 0.1
     bc_tol = 5e-6
     metrics = ["drag", "lift"]
+    render_fields = ("velocity_magnitude", "velocity_x", "velocity_y", "velocity_z", "pressure")
+    render_fill_steps = 16                  # the hole-filling sweeps of the family's sensors
+
+    def _render_planes(self):
+        Z = self.render_shape[2]
+        return Z, Z // 2
+
+    def _build_render_map(self, plane):
+        from ..render import render_map_extruded
+        return render_map_extruded([b.vertex for b in self.spec.blocks], self.z_vertices, self.render_shape, plane, self.render_fill_steps)
 
     @property
     def n_sensors_z(self):

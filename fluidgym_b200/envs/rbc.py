@@ -15,7 +15,7 @@ import torch
 from .. import native
 from ..sensors import sensor_tables
 from ..solver import BatchedPISO, _ptr
-from .common import InitialDomains
+from .common import InitialDomains, Renderable
 from .rbc_domain import make_rbc_domain
 
 RBC_2D_DEFAULT_CONFIG = {
@@ -38,12 +38,13 @@ def extract_moving_window_2d(field: torch.Tensor, n_agents: int, agent_width: in
     return win.reshape(*lead, n_agents, Y, n_agents_per_window * agent_width)
 
 
-class RBC2DEnv(InitialDomains):
+class RBC2DEnv(InitialDomains, Renderable):
     T_cold, T_hot, heater_limit = 0.0, 1.0, 0.75
     n_sensors_y, n_sensors_per_heater = 8, 4
     buoyancy_factor = 1.0
     metrics = ["nusselt"]
     reference_values = {"nu_ref": ("nusselt", "p50")}
+    render_fields = ("temperature", "velocity_magnitude", "vorticity", "pressure")
 
     def __init__(self, n_envs: int = 1, rayleigh_number=8e4, prandtl_number=0.7, n_heaters=12, resolution=8, dt=0.05,
                  adaptive_cfl=0.8, step_length=1.0, episode_length=200, local_obs_window=11, local_reward_weight=0.2,
@@ -88,6 +89,10 @@ class RBC2DEnv(InitialDomains):
     @property
     def n_sensors_x(self):
         return self.n_heaters * self.n_sensors_per_heater
+
+    def _build_render_map(self, plane):
+        from ..render import render_map_2d
+        return render_map_2d([b.vertex for b in self.spec.blocks], self.render_shape, fill_max_steps=16)
 
     def _setup_sensors(self):
         nx, ny = self.render_shape

@@ -18,7 +18,7 @@ from ..box3d import BatchedPISO3D, Box3DDomain
 from ..grids import wall_refined_ortho_grid
 from ..sensors import sensor_tables_3d
 from ..solver import _ptr
-from .common import InitialDomains3D
+from .common import InitialDomains3D, Renderable
 
 RBC_3D_DEFAULT_CONFIG = {
     "rayleigh_number": 2e3, "prandtl_number": 0.7, "n_heaters": 8, "resolution": 8, "dt": 0.05, "adaptive_cfl": 0.8,
@@ -54,7 +54,7 @@ def extract_moving_window_3d(field: torch.Tensor, n_agents: int, agent_width: in
     return fzx.reshape(*lead, n_agents * n_agents, cells.shape[1], Y, cells.shape[1])
 
 
-class RBC3DEnv(InitialDomains3D):
+class RBC3DEnv(InitialDomains3D, Renderable):
     T_cold, T_hot, heater_limit = 0.0, 1.0, 0.75
     n_sensors_y, n_sensors_per_heater = 8, 4
     buoyancy_factor = 1.0
@@ -62,6 +62,7 @@ class RBC3DEnv(InitialDomains3D):
     resolution_scale_y, grid_base = 2.0, 1.02
     metrics = ["nusselt"]
     reference_values = {"nu_ref": ("nusselt", "mean")}
+    render_fields = ("temperature", "velocity_magnitude", "q_criterion", "pressure")
 
     def __init__(self, n_envs: int = 1, rayleigh_number=2e3, prandtl_number=0.7, n_heaters=8, resolution=8, dt=0.05,
                  adaptive_cfl=0.8, step_length=1.0, episode_length=200, local_obs_window=3, local_reward_weight=0.0015,
@@ -114,6 +115,14 @@ class RBC3DEnv(InitialDomains3D):
     @property
     def n_sensors_x(self):
         return self.n_heaters * self.n_sensors_per_heater
+
+    def _render_planes(self):
+        Z = self.render_shape[2]
+        return Z, Z // 2
+
+    def _build_render_map(self, plane):
+        from ..render import render_map_box3d
+        return render_map_box3d(self.dom.vertex, self.render_shape, plane, fill_max_steps=16)
 
     def _setup_sensors(self):
         """rbc_env_base.py:445-470 + rbc_env_3d.py:183-203: (x, y) sensor voxels x-major, every pair repeated over z."""

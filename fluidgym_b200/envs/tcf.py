@@ -11,7 +11,7 @@ import torch
 
 from ..box3d import BatchedPISO3D, Box3DDomain
 from ..grids import channel_vertex_grid
-from .common import InitialDomains3D
+from .common import InitialDomains3D, Renderable
 
 SMALL_TCF_3D_DEFAULT_CONFIG = {
     "resolution_y": 65, "resolution_x_z": 64, "actor_size": 2, "L": np.pi, "D": np.pi / 2, "reynolds_number_wall": 180,
@@ -39,11 +39,12 @@ def agent_window_means(field, n_agents_x, n_agents_z, agent_width, wx, wz, pad_x
     return win.reshape(*lead, n_agents_x * n_agents_z, wz, wx)
 
 
-class TCF3DEnv(InitialDomains3D):
+class TCF3DEnv(InitialDomains3D, Renderable):
     delta, H = 1.0, 2.0
     y_obs_wall = 15.0
     metrics = ["wall_stress", "wall_stress_bottom", "wall_stress_top"]
     both_walls = False
+    render_fields = ("velocity_x", "velocity_magnitude", "pressure", "q_criterion")
 
     def __init__(self, n_envs: int = 1, resolution_y=65, resolution_x_z=64, actor_size=2, L=np.pi, D=np.pi / 2, reynolds_number_wall=180,
                  adaptive_cfl=0.1, step_length=0.6, episode_length=1000, local_obs_window=1, local_reward_weight=0.0, use_marl=True,
@@ -244,6 +245,14 @@ class TCF3DEnv(InitialDomains3D):
             oy = torch.flip(oy, dims=[3]) * -1
             op = torch.flip(op, dims=[2])
         return {"velocity": torch.stack((ox, oy), dim=-1), "pressure": op}
+
+    def _render_planes(self):
+        return self.ny, self.y_obs_bottom_idx
+
+    def _build_render_map(self, plane):
+        """the wall-parallel cell plane y = ``plane``, shown [z, x]: x and z are uniform, so the map is the identity"""
+        from ..render import render_map_cell_plane
+        return render_map_cell_plane(self.x, self.ny, self.z, plane)
 
     def q_criterion(self):
         """_get_q_criterion (tcf_env.py:586-644) on the cell grid [B, nz, ny, nx]: Q = (|Omega|^2 - |S|^2) / 2 from

@@ -40,12 +40,18 @@ def _device(env):
     return getattr(env, "device", None) or getattr(env, "cuda_device")
 
 
+def _check_render_mode(render_mode):
+    if render_mode is not None and render_mode != "rgb_array":
+        raise ValueError(f"Unsupported render mode: {render_mode}. Only 'rgb_array' is supported.")
+
+
 class VecFluidEnv(_SB3VecEnv):
     """SB3 ``VecEnv`` protocol over a batched environment: slot ``e * n_agents + a`` = agent ``a`` of environment ``e``."""
 
     metadata = {"render_modes": ["rbg_array"]}
 
-    def __init__(self, env, auto_reset: bool = True):
+    def __init__(self, env, auto_reset: bool = True, render_mode: str | None = None):
+        _check_render_mode(render_mode)
         self._env = env
         self._auto_reset = auto_reset
         self.n_envs_batch = int(getattr(env, "n_envs", 1))
@@ -54,7 +60,7 @@ class VecFluidEnv(_SB3VecEnv):
         self.observation_space = env.observation_space
         self.action_space = env.action_space
         self._actions = None
-        self.render_mode = None
+        self.render_mode = render_mode
 
     # --- layout helpers -----------------------------------------------------------------------------
     def _flat(self, x):
@@ -121,6 +127,14 @@ class VecFluidEnv(_SB3VecEnv):
     def env_method(self, method_name: str, *method_args, indices=None, **method_kwargs):
         raise NotImplementedError
 
+    def get_images(self) -> list:
+        """One uint8 [H, W, 3] image per slot (the agents of an environment share its image); ``None`` per slot unless
+        ``render_mode == "rgb_array"``.  One batched ``env.render()`` and one device->host copy."""
+        if self.render_mode != "rgb_array":
+            return [None] * self.num_envs
+        imgs = _np(self._env.render())
+        return [imgs[i // self.n_agents] for i in range(self.num_envs)]
+
     def seed(self, seed: int | None = None):
         if seed is not None:
             self._env.seed(seed)
@@ -156,8 +170,7 @@ class GymFluidEnv:
     def __init__(self, env, render_mode: str | None = None):
         if getattr(env, "use_marl", False):
             raise ValueError("GymFluidEnv does not support multi-agent environments. Please use a single-agent environment.")
-        if render_mode is not None and render_mode != "rgb_array":
-            raise ValueError(f"Unsupported render mode: {render_mode}. Only 'rgb_array' is supported.")
+        _check_render_mode(render_mode)
         _single(env, "GymFluidEnv")
         self.render_mode = render_mode
         self._env = env
@@ -177,6 +190,12 @@ class GymFluidEnv:
     def reset(self, *, seed: int | None = None, options: dict | None = None, randomize: bool | None = None):
         obs, info = self._env.reset(seed=seed, randomize=randomize)
         return self._squeeze(obs), {k: _np(v) for k, v in info.items()}
+
+    def render(self):
+        """uint8 [H, W, 3] numpy image of the environment with ``render_mode == "rgb_array"``, otherwise ``None``."""
+        if self.render_mode != "rgb_array":
+            return None
+        return _np(self._env.render()[0])
 
     def close(self):
         pass
@@ -278,11 +297,13 @@ class TorchRLFluidEnv(_TorchRLEnvBase):
     batch, torchrl.py:87-100).  A batched environment is a real batch: batch size ``(n_envs,)`` or ``(n_envs, n_agents)``, all
     tensors stay on the environment's device (no numpy round trip).  Same ``_step / _reset / _set_seed`` protocol and the same
     spec layout (observation keys as a Composite, reward / done / terminated / truncated with a trailing unit dimension).
-    ``from_pixels`` needs the reference's renderer and is not supported (rendering is outside the solver path)."""
+    ``from_pixels`` adds ``"pixels"``, the environment's ``render()`` as uint8 ``(*batch_size, H, W, 3)``, to
+    the observation spec and to every reset / step; the agents of one environment share its image (an expanded view)."""
 
     def __init__(self, env, from_pixels: bool = False):
-        if from_pixels:
-            raise NotImplementedError("from_pixels: rendering is not part of fluidgym_b200")
+        if from_pixels and not callable(getattr(env, "render", None)):
+            raise NotImplementedError(f"from_pixels: {type(env).__name__} has no render()")
+        self._from_pixels = bool(from_pixels)
         n_envs = int(getattr(env, "n_envs", 1))
         self._n_agents = int(env.n_agents) if getattr(env, "use_marl", False) else None
         batch = (n_envs,) if self._n_agents is None else (n_envs, self._n_agents)
@@ -306,6 +327,11 @@ class TorchRLFluidEnv(_TorchRLEnvBase):
         obs_space = self._env.observation_space
         sub = obs_space.spaces if hasattr(obs_space, "spaces") else {"observation": obs_space}
         obs = {k: self._box(v, lead) for k, v in sub.items()}
+        if self._from_pixels:
+            H, W = self._pixels().shape[-3:-1]
+            shape = torch.Size((*lead, H, W, 3))
+            obs["pixels"] = _Bounded(low=0, high=255, shape=shape, dtype=torch.uint8, device=self.device) if _HAVE_TORCHRL else \
+                SpecLike(shape, dtype=torch.uint8, low=0, high=255, device=self.device)
         flag = (lambda: SpecLike((*lead, 1), dtype=torch.bool, device=self.device)) if not _HAVE_TORCHRL else \
             (lambda: _Categorical(n=2, shape=torch.Size((*lead, 1)), dtype=torch.bool, device=self.device))
         if _HAVE_TORCHRL:                                # pragma: no cover
@@ -320,6 +346,17 @@ class TorchRLFluidEnv(_TorchRLEnvBase):
             self.done_spec = {"done": flag(), "terminated": flag(), "truncated": flag()}
         self.action_spec = self._box(self._env.action_space, lead)
 
+    def _pixels(self) -> torch.Tensor:
+        img = self._env.render()                                        # [n_envs, H, W, 3]
+        if self._n_agents is not None:
+            img = img[:, None].expand(img.shape[0], self._n_agents, *img.shape[1:])
+        return img
+
+    def _observe(self, obs) -> dict:
+        if not isinstance(obs, dict):
+            obs = {"observation": obs}
+        return {**obs, "pixels": self._pixels()} if self._from_pixels else obs
+
     def _td(self, data: dict):
         return _TensorDict(data, batch_size=self.batch_size) if _HAVE_TORCHRL else dict(data)
 
@@ -329,17 +366,14 @@ class TorchRLFluidEnv(_TorchRLEnvBase):
     def _step(self, tensordict):                          # torchrl.py:205-244
         with torch.no_grad():
             obs, reward, term, trunc, _ = self._env.step(tensordict["action"])
-        if not isinstance(obs, dict):
-            obs = {"observation": obs}
+            obs = self._observe(obs)
         reward = reward.reshape(*self.batch_size, 1)
         return self._td({**obs, "reward": reward, "done": self._flag(term or trunc), "terminated": self._flag(term),
                          "truncated": self._flag(trunc)})
 
     def _reset(self, tensordict=None, **kwargs):          # torchrl.py:246-268
         obs, _ = self._env.reset()
-        if not isinstance(obs, dict):
-            obs = {"observation": obs}
-        return self._td(obs)
+        return self._td(self._observe(obs))
 
     def _set_seed(self, seed: int) -> None:               # torchrl.py:270-278
         self._env.seed(seed)

@@ -85,7 +85,7 @@ EXPORTS = ["fgb_last_error", "fgb_version", "fgb_workspace_bytes", "fgb_batch_cr
            "fgb_ortho3_solve_pressure", "fgb_ortho3_correct_velocity", "fgb_ortho3_piso_substep", "fgb_ortho3_make_divergence_free",
            "fgb_ortho3_sim_step", "fgb_ortho3_wall_rows", "fgb_ipc_alloc", "fgb_ipc_open", "fgb_ipc_close", "fgb_ipc_free",
            "fgb_ortho3_set_slab", "fgb_ortho3_slab_error", "fgb_ortho3_set_scalar", "fgb_ortho3_advect_scalar", "fgb_ortho3_set_sgs", "fgb_ortho3_sgs_viscosity", "fgb_ortho3_velocity_gradients", "fgb_ortho3_piso_substep_record", "fgb_ortho3_adjoint_workspace_bytes", "fgb_ortho3_piso_substep_backward", "fgb_ortho3_piso_substep_record_scalar", "fgb_ortho3_piso_substep_backward_scalar", "fgb_extruded3_piso_substep_record", "fgb_extruded3_adjoint_workspace_bytes", "fgb_extruded3_piso_substep_backward", "fgb_sample_sensors_n", "fgb_extruded3_piso_substep", "fgb_extruded3_make_divergence_free",
-           "fgb_extruded3_balance_fluxes", "fgb_extruded3_update_outflow", "fgb_extruded3_max_velocity", "fgb_extruded3_wall_forces", "fgb_extruded3_apply_jets"]
+           "fgb_extruded3_balance_fluxes", "fgb_extruded3_update_outflow", "fgb_extruded3_max_velocity", "fgb_extruded3_wall_forces", "fgb_extruded3_apply_jets", "fgb_render_gather", "fgb_render_colour"]
 
 
 def lib_path() -> str:
@@ -165,6 +165,8 @@ def load():
     L.fgb_wall_forces.argtypes = [vp, C.POINTER(Wall), vp, vp, vp, vp, vp]
     L.fgb_sample_sensors.argtypes = [vp, vp, i32, vp, vp, i32, i32, vp, vp]
     L.fgb_sample_sensors_n.argtypes = [vp, i32, i32, i32, vp, vp, i32, i32, vp, vp]
+    L.fgb_render_gather.argtypes = [vp, i32, i32, i32, C.c_int64, C.c_int64, i32, vp, vp, vp, i32, vp, vp, vp]
+    L.fgb_render_colour.argtypes = [vp, i32, i32, vp, f32, f32, i32, vp, vp, vp]
     L.fgb_profile_enable.argtypes = [vp, i32]
     L.fgb_profile_read.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(C.c_int64), i32]
     L.fgb_launch_count.argtypes = [vp]

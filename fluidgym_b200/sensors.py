@@ -320,22 +320,31 @@ def _splat_matrix(centres, lower, upper, out_shape, n_corners):
 def _pixel_map_from_centres(centres, lower, upper, out_shape, fill_max_steps, n_corners):
     W, H, Z = out_shape
     S, wsum = _splat_matrix(centres, lower, upper, out_shape, n_corners)
-    npx = W * H * Z
+    return normalise_and_fill(S, wsum, (Z, H, W), fill_max_steps)
+
+
+def normalise_and_fill(S, wsum, grid_shape, fill_max_steps):
+    """Rendered-pixel map R [pixels, cells] from the raw splat ``S`` and its row sums: rows with weight normalised, then up to
+    ``fill_max_steps`` hole-filling sweeps R <- R + A R, where A gives every still empty pixel the mean of its face neighbours
+    (2 per axis of ``grid_shape``, C order = pixel order) that were valid before the sweep (resampling.cu:191-293).
+    Returns (R csr, fill level per pixel: 0 = splat, k = filled in sweep k, -1 = never)."""
+    npx = S.shape[0]
+    nd = len(grid_shape)
     valid = wsum > 1e-8
     level = np.where(valid, 0, -1).astype(np.int32)
     inv = np.zeros(npx)
     inv[valid] = 1.0 / wsum[valid]
     R = sp.diags(inv) @ S
-    grid = np.arange(npx).reshape(Z, H, W)
+    grid = np.arange(npx).reshape(grid_shape)
     for k in range(1, int(fill_max_steps) + 1):
         if valid.all():
             break
-        v3 = valid.reshape(Z, H, W)
+        v3 = valid.reshape(grid_shape)
         src_l, dst_l = [], []
-        for ax in range(3):
+        for ax in range(nd):
             for sh in (1, -1):
-                a = [slice(None)] * 3
-                b = [slice(None)] * 3
+                a = [slice(None)] * nd
+                b = [slice(None)] * nd
                 a[ax] = slice(1, None) if sh == 1 else slice(0, -1)
                 b[ax] = slice(0, -1) if sh == 1 else slice(1, None)
                 m = (~v3[tuple(a)]) & v3[tuple(b)]

@@ -246,6 +246,22 @@ int fgb_sample_sensors(fgb_batch *b, const float *field, int32_t channels, const
 int fgb_sample_sensors_n(const float *field, int32_t B, int32_t channels, int32_t N, const int32_t *idx, const float *w, int32_t K,
                          int32_t n_sensors, float *out, fgb_stream_t s);
 
+/* ---- rendering (fluidgym_b200/render.py; no solver handle) --------------------------------------------------------------- */
+#define FGB_RENDER_IDENTITY 0   /* img = the resampled channel (channels = 1)                    */
+#define FGB_RENDER_NORM 1       /* img = |resampled vector| over 2 or 3 channels                  */
+/* env.render / render_field (fluid_env.py:577-606 -> resample.py:300-358, resampling.cu:191-364): img[B][P] float32 = the CSR
+ * render map (rowptr [P+1], col, w; splat + normalise + fill sweeps, rows in image order) applied to channel c of environment b at
+ * field + b * env_stride + c * chan_stride, combined by ``mode``.  range (optional) [B][2] receives order-preserving uint32 keys
+ * of each environment's min and max for fgb_render_colour; it is initialised by this call.  No host synchronisation. */
+int fgb_render_gather(const float *field, int32_t B, int32_t channels, int32_t N, int64_t chan_stride, int64_t env_stride,
+                      int32_t mode, const int32_t *rowptr, const int32_t *col, const float *w, int32_t P, float *img,
+                      uint32_t *range, fgb_stream_t s);
+/* the colour step of env.render: rgb[B][P][3] uint8 = lut[256][3] at bin floor(256 (v - lo) / (hi - lo)) clamped to [0, 255] (128
+ * when hi <= lo); [lo, hi] = the environment's range from fgb_render_gather, or [vmin, vmax] for the whole batch when range is
+ * NULL; symmetric != 0 widens it to [-m, m], m = max(|lo|, |hi|).  img 16-byte, rgb 4-byte aligned. */
+int fgb_render_colour(const float *img, int32_t B, int32_t P, const uint32_t *range, float vmin, float vmax, int32_t symmetric,
+                      const uint8_t *lut, uint8_t *rgb, fgb_stream_t s);
+
 /* ---- differentiability (torch.autograd is layered on top in fluidgym_b200/autograd.py) ----------------- */
 /* Tape of one substep: device buffers owned by the caller, filled by fgb_piso_substep_record.  Replaces the
  * tensors the reference's autograd.Functions save per native op (DIFF.py:624-1808). */
