@@ -16,7 +16,7 @@ from .. import native
 from ..sensors import sensor_tables
 from ..solver import BatchedPISO, _ptr
 from .airfoil_domain import BOT, FRONT, JET_CENTERS, JET_WIDTH, TAIL_LOWER, TAIL_UPPER, TOP, airfoil_polyline, make_airfoil_domain
-from .common import DifferentiableRollout, InitialDomains, Renderable, build_wall_tables
+from .common import DifferentiableRollout, EpisodeLifecycle, InitialDomains, Renderable, build_wall_tables
 from .cylinder_domain import jet_profile
 
 AIRFOIL_2D_DEFAULT_CONFIG = {
@@ -41,7 +41,7 @@ def polygon_mask(polygon_xy: np.ndarray, nx: int, ny: int) -> np.ndarray:
     return inside.reshape(ny, nx)
 
 
-class Airfoil2DEnv(DifferentiableRollout, InitialDomains, Renderable):
+class Airfoil2DEnv(EpisodeLifecycle, DifferentiableRollout, InitialDomains, Renderable):
     H, L, U_mean, airfoil_length = 1.4, 4.5, 0.3, 1.0
     n_jets = 3
     action_smoothing_alpha = 0.1
@@ -65,7 +65,6 @@ class Airfoil2DEnv(DifferentiableRollout, InitialDomains, Renderable):
         self.cl_cd_ref = float(cl_cd_ref)
         self.randomize_initial_state, self.enable_actions = randomize_initial_state, enable_actions
         self.differentiable = bool(differentiable)
-        self._dstate = None
         self.load_domain_on_reset, self.initial_domains_path = bool(load_initial_domain), initial_domains_path
         self.device = torch.device(device)
         if compiled is None:
@@ -92,7 +91,6 @@ class Airfoil2DEnv(DifferentiableRollout, InitialDomains, Renderable):
         self.last_control = torch.zeros(B, self.n_jets, device=dev)
         self._acc = torch.zeros(B, 2, device=dev)
         self._zero_action = torch.zeros(B, self.n_jets, device=dev)
-        self._reset_called, self._seed, self._n_steps, self.last_substeps = False, None, 0, 0
 
     # ---- static tables ---------------------------------------------------------------------------
     def _setup_jets(self, out_mask):
@@ -165,10 +163,6 @@ class Airfoil2DEnv(DifferentiableRollout, InitialDomains, Renderable):
         return f"airfoil_2D_Re{int(self.reynolds_number)}"
 
     @property
-    def n_sim_steps(self):
-        return max(1, int(self.step_length / self.dt))
-
-    @property
     def observation_space(self):
         from .. import spaces
         inf, ns = float("inf"), int(self.sens_idx.shape[1])
@@ -179,21 +173,10 @@ class Airfoil2DEnv(DifferentiableRollout, InitialDomains, Renderable):
         from .. import spaces
         return spaces.Box(-1.0, 1.0, shape=(self.n_jets,))
 
-    def seed(self, seed: int):
-        self._seed = seed
-        self._np_rng = np.random.default_rng(seed)
-        self._torch_rng = torch.Generator(device=self.device).manual_seed(seed)
-
-    def sample_action(self):
-        if self._seed is None:
-            raise RuntimeError("Environment must be seeded before sampling actions")
-        return torch.rand(self.n_envs, self.n_jets, device=self.device, generator=self._torch_rng) * 2 - 1
-
     def set_state(self, u, p, bvel, last_control=None):
         s = self.solver
         for dst, src in ((s.u, u), (s.p, p), (s.bvel, bvel)):
-            src = torch.as_tensor(src, dtype=torch.float32, device=self.device)
-            dst.copy_(src if src.dim() == dst.dim() else src.unsqueeze(0).expand_as(dst))
+            self._copy_state(dst, src)
         if last_control is not None:
             self.last_control.copy_(torch.as_tensor(last_control, device=self.device).expand_as(self.last_control))
         self._dstate = None
@@ -204,11 +187,7 @@ class Airfoil2DEnv(DifferentiableRollout, InitialDomains, Renderable):
         return dict(u=s.u.clone(), p=s.p.clone(), bvel=s.bvel.clone(), last_control=self.last_control.clone())
 
     def reset(self, seed: int | None = None, randomize: bool | None = None):
-        if seed is None:
-            if self._seed is None:
-                raise ValueError("Seed must be provided either during reset or by calling seed().")
-        else:
-            self.seed(seed)
+        self._begin_reset(seed)
         s = self.solver
         if self.load_domain_on_reset:
             self._load_initial_domains_on_reset(self.randomize_initial_state if randomize is None else randomize)
@@ -260,16 +239,7 @@ class Airfoil2DEnv(DifferentiableRollout, InitialDomains, Renderable):
                                                      s.stream), "fgb_sample_sensors")
         return {"velocity": vel.permute(0, 2, 1).contiguous(), "pressure": prs[:, 0]}
 
-    def step(self, action):
-        if not self._reset_called:
-            raise RuntimeError("Environment must be reset before stepping. Call 'reset()' before'step()'.")
-        action = torch.as_tensor(action, dtype=torch.float32, device=self.device)
-        if action.shape != self._zero_action.shape:
-            raise ValueError(f"Action shape {action.shape} does not match expected shape {self._zero_action.shape}.")
-        if self._n_steps >= self.episode_length:
-            raise RuntimeError("Episode has already terminated. Call 'reset()' first.")
-        if self.differentiable:
-            return self._step_differentiable(action)
+    def _advance(self, action):
         s = self.solver
         self._acc.zero_()
         nsub = 0
@@ -282,18 +252,12 @@ class Airfoil2DEnv(DifferentiableRollout, InitialDomains, Renderable):
             native.check(self.lib.fgb_wall_forces(s.handle, C.byref(self.wall), _ptr(s.u), _ptr(s.p), _ptr(s.bvel), _ptr(self._acc),
                                                   s.stream), "fgb_wall_forces")
         self.last_substeps = nsub
-        return self._finish(self._acc / self.n_sim_steps)
+        return self._acc
 
-    def _finish(self, mean):
-        obs = self._get_obs()
-        cd, cl = mean[:, 0], mean[:, 1]
-        reward = cl / cd - self.cl_cd_ref
-        self._n_steps += 1
-        self._watch_linear_solves()
-        truncated = self._n_steps >= self.episode_length
-        return obs, reward, False, truncated, {"drag": cd.detach(), "lift": cl.detach()}
+    def _reward(self, cd, cl):
+        return cl / cd - self.cl_cd_ref
 
-    def _step_differentiable(self, action):
+    def _advance_differentiable(self, action):
         s = self.solver
         if self._dstate is None:
             self._dstate = (s.u.clone(), s.p.clone(), s.bvel.clone(), self.last_control.clone())
@@ -314,4 +278,4 @@ class Airfoil2DEnv(DifferentiableRollout, InitialDomains, Renderable):
             s.u.copy_(u); s.p.copy_(p); s.bvel.copy_(bv)
             self.last_control = last.detach().clone()
         self.last_substeps = nsub
-        return self._finish(acc / self.n_sim_steps)
+        return acc

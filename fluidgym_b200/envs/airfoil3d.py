@@ -96,7 +96,6 @@ class Airfoil3DEnv(SpanwiseExtrudedEnv):
         self.last_control = torch.zeros(B, self.n_span, self.n_jets, device=dev)
         self._zero_action = torch.zeros(B, self.n_span, self.n_jets, device=dev)
         self._bvel0 = torch.from_numpy(np.ascontiguousarray(cd.bvel0[:, :cd.NB])).to(dev)
-        self._reset_called, self._seed, self._n_steps, self.last_substeps = False, None, 0, 0
 
     # ---- static tables ---------------------------------------------------------------------------------------------------
     @property

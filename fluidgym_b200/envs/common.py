@@ -1,4 +1,5 @@
-"""Pieces shared by the bluff-body environments (cylinder, airfoil): wall-force tables, and the differentiable
+"""Pieces shared by the environment families: the episode lifecycle, initial domains, domain statistics, the linear-solve
+watch and rendering.  For the bluff-body environments (cylinder, airfoil) also the wall-force tables and the differentiable
 rollout in which the PISO substep is one autograd node backed by the CUDA adjoint (``fluidgym_b200.autograd``)
 while the few boundary / reward formulas around it are tiny torch expressions over the same static tables the
 kernels use -- so gradients flow from the reward to the action, the cell velocities and the boundary values as in
@@ -12,7 +13,7 @@ import torch
 
 from .. import native
 from ..sensors import cell_centres
-from ..solver import _ptr
+from ..solver import _ptr, cfl_substeps
 
 
 def build_wall_tables(cd, spec, ring, device, scale: float):
@@ -67,13 +68,82 @@ def build_wall_tables(cd, spec, ring, device, scale: float):
     return tab, w
 
 
-class DifferentiableRollout:
-    """Mixin: needs ``solver, cd, device, lib, n_envs, dt, cfl, char_vel, wall, _wall_t, _dstate``."""
+class EpisodeLifecycle:
+    """Mixin: the episode lifecycle of the reference's ``FluidEnv`` (fluid_env.py) with its error strings, shared by every
+    family: seeding, action sampling, the checks at the start of ``reset`` and ``step``, the end of a step and ``detach``.
+    Needs ``device, dt, step_length, episode_length, _zero_action`` and ``_watch_linear_solves`` (LinearSolveWatch)."""
+
+    _reset_called = False
+    _seed = None
+    _n_steps = 0
+    last_substeps = 0
+    _dstate = None          # differentiable mode: the state tensors carried with their autograd history
+
+    @property
+    def n_sim_steps(self):
+        return max(1, int(self.step_length / self.dt))
+
+    def seed(self, seed: int):
+        self._seed = seed
+        self._np_rng = np.random.default_rng(seed)
+        self._torch_rng = torch.Generator(device=self.device).manual_seed(seed)
+
+    def sample_action(self):
+        if self._seed is None:
+            raise RuntimeError("Environment must be seeded before sampling actions")
+        return torch.rand(self._zero_action.shape, device=self.device, generator=self._torch_rng) * 2 - 1
+
+    def _begin_reset(self, seed):
+        """First thing of every ``reset``: seed, or check that ``seed()`` was called."""
+        if seed is None:
+            if self._seed is None:
+                raise ValueError("Seed must be provided either during reset or by calling seed().")
+        else:
+            self.seed(seed)
+
+    def _begin_step(self, action) -> torch.Tensor:
+        """First thing of every ``step``: the checks of the reference, returns the action as float32 on the device."""
+        if not self._reset_called:
+            raise RuntimeError("Environment must be reset before stepping. Call 'reset()' before'step()'.")
+        action = torch.as_tensor(action, dtype=torch.float32, device=self.device)
+        if action.shape != self._zero_action.shape:
+            raise ValueError(f"Action shape {action.shape} does not match expected shape {self._zero_action.shape}.")
+        if self._n_steps >= self.episode_length:
+            raise RuntimeError("Episode has already terminated. Call 'reset()' first.")
+        return action
+
+    def _end_step(self) -> bool:
+        """Counts the step, watches its linear solves; returns ``truncated``."""
+        self._n_steps += 1
+        self._watch_linear_solves()
+        return self._n_steps >= self.episode_length
+
+    def _copy_state(self, dst: torch.Tensor, src):
+        """``set_state``: ``src`` is one environment's field (copied into every environment) or the whole batch's."""
+        src = torch.as_tensor(src, dtype=torch.float32, device=self.device)
+        dst.copy_(src if src.dim() == dst.dim() else src.unsqueeze(0).expand_as(dst))
 
     def detach(self):
         """fluid_env.py ``detach()``: cut the autograd graph at the current state."""
         if self._dstate is not None:
             self._dstate = tuple(t.detach() for t in self._dstate)
+
+
+class DifferentiableRollout:
+    """Mixin of the 2-D bluff-body families (cylinder, airfoil): ``env.step`` and the differentiable rollout.  Needs ``solver,
+    cd, device, lib, n_envs, dt, cfl, char_vel, wall, _wall_t, _dstate`` and, for ``step``, ``_advance(action)`` /
+    ``_advance_differentiable(action)`` (-> the [B, 2] drag / lift coefficients summed over the solver steps), ``_get_obs()`` and
+    ``_reward(cd, cl)``."""
+
+    def step(self, action):
+        action = self._begin_step(action)
+        acc = self._advance_differentiable(action) if self.differentiable else self._advance(action)
+        obs = self._get_obs()
+        mean = acc / self.n_sim_steps
+        cd, cl = mean[:, 0], mean[:, 1]
+        reward = self._reward(cd, cl)
+        truncated = self._end_step()
+        return obs, reward, False, truncated, {"drag": cd.detach(), "lift": cl.detach()}
 
     def _diff_tables(self):
         if getattr(self, "_dt_tab", None) is None:
@@ -150,20 +220,16 @@ class DifferentiableRollout:
         used for the batch (the most restrictive environment decides)."""
         from ..autograd import piso_substep
         s = self.solver
-        remaining, nsub = float(self.dt), 0
         mvb = torch.empty(self.n_envs, device=self.device)
-        while remaining > 0.0 and not abs(remaining) <= 1e-8:
+
+        def max_velocity():
             native.check(self.lib.fgb_max_velocity(s.handle, _ptr(u.detach().contiguous()), _ptr(bv.detach().contiguous()), _ptr(mvb),
                                                    s.stream), "fgb_max_velocity")
-            mv = float(mvb.max())
-            if abs(mv) <= 1e-8:
-                ts = remaining
-            else:
-                mts = np.float32(self.cfl) / np.float32(mv)
-                ts = remaining if float(mts) >= remaining else remaining / float(np.ceil(np.float32(remaining) / mts))
-            remaining -= ts
-            bv = self._outflow_torch(u, bv, float(np.float32(ts)), getattr(self, "bc_tol", 1e-5))
-            u, p = piso_substep(s, u, p, bv, float(np.float32(ts)))
+            return float(mvb.max())
+        nsub = 0
+        for ts in cfl_substeps(self.dt, self.cfl, max_velocity):
+            bv = self._outflow_torch(u, bv, ts, getattr(self, "bc_tol", 1e-5))
+            u, p = piso_substep(s, u, p, bv, ts)
             nsub += 1
         return u, p, bv, nsub
 

@@ -18,7 +18,7 @@ import torch
 from .. import native
 from ..sensors import sensor_tables
 from ..solver import BatchedPISO, _ptr
-from .common import DifferentiableRollout, InitialDomains, Renderable, build_wall_tables
+from .common import DifferentiableRollout, EpisodeLifecycle, InitialDomains, Renderable, build_wall_tables
 from .cylinder_domain import BOTTOM, LEFT, RIGHT, TOP, WAKE, jet_profile, make_cylinder_domain
 
 CYLINDER_ROT_2D_DEFAULT_CONFIG = {
@@ -82,7 +82,7 @@ def cylinder_sensor_locations(cylinder_diameter: float = 1.0) -> torch.Tensor:
     return torch.concatenate([loc, c1, c2, add], dim=1)
 
 
-class CylinderJet2DEnv(DifferentiableRollout, InitialDomains, Renderable):
+class CylinderJet2DEnv(EpisodeLifecycle, DifferentiableRollout, InitialDomains, Renderable):
     H, L, cylinder_diameter, U_mean, cylinder_offset_y = 4.1, 22.0, 1.0, 1.0, 0.05
     n_sensors = 151
     action_smoothing_alpha = 0.1
@@ -105,7 +105,6 @@ class CylinderJet2DEnv(DifferentiableRollout, InitialDomains, Renderable):
         self.randomize_initial_state = randomize_initial_state
         self.enable_actions = enable_actions
         self.differentiable = bool(differentiable)
-        self._dstate = None
         self.load_domain_on_reset, self.initial_domains_path = bool(load_initial_domain), initial_domains_path
         self.reynolds_number = float(reynolds_number)
         self.device = torch.device(device)
@@ -130,10 +129,6 @@ class CylinderJet2DEnv(DifferentiableRollout, InitialDomains, Renderable):
         self.last_control = torch.zeros(B, device=dev)
         self._acc = torch.zeros(B, 2, device=dev)
         self._zero_action = torch.zeros(B, 1, device=dev)
-        self._reset_called = False
-        self._seed = None
-        self._n_steps = 0
-        self.last_substeps = 0
 
     # ---- static tables ---------------------------------------------------------------------------
     def _setup_jets(self):
@@ -182,10 +177,6 @@ class CylinderJet2DEnv(DifferentiableRollout, InitialDomains, Renderable):
         """cylinder_env_base.py:823-828"""
         return f"cylinder_2D_Re{int(self.reynolds_number)}_Res{self.resolution}"
 
-    @property
-    def n_sim_steps(self):
-        return max(1, int(self.step_length / self.dt))
-
     use_marl = False
 
     @property
@@ -201,21 +192,10 @@ class CylinderJet2DEnv(DifferentiableRollout, InitialDomains, Renderable):
         from .. import spaces
         return spaces.Box(-1.0, 1.0, shape=(1,))
 
-    def seed(self, seed: int):
-        self._seed = seed
-        self._np_rng = np.random.default_rng(seed)
-        self._torch_rng = torch.Generator(device=self.device).manual_seed(seed)
-
-    def sample_action(self):
-        if self._seed is None:
-            raise RuntimeError("Environment must be seeded before sampling actions")
-        return torch.rand(self.n_envs, 1, device=self.device, generator=self._torch_rng) * 2 - 1
-
     def set_state(self, u, p, bvel, last_control=None):
         s = self.solver
         for dst, src in ((s.u, u), (s.p, p), (s.bvel, bvel)):
-            src = torch.as_tensor(src, dtype=torch.float32, device=self.device)
-            dst.copy_(src if src.dim() == dst.dim() else src.unsqueeze(0).expand_as(dst))
+            self._copy_state(dst, src)
         if last_control is not None:
             self.last_control.copy_(torch.as_tensor(last_control, device=self.device).expand_as(self.last_control))
         self._dstate = None
@@ -226,11 +206,7 @@ class CylinderJet2DEnv(DifferentiableRollout, InitialDomains, Renderable):
         return dict(u=s.u.clone(), p=s.p.clone(), bvel=s.bvel.clone(), last_control=self.last_control.clone())
 
     def reset(self, seed: int | None = None, randomize: bool | None = None):
-        if seed is None:
-            if self._seed is None:
-                raise ValueError("Seed must be provided either during reset or by calling seed().")
-        else:
-            self.seed(seed)
+        self._begin_reset(seed)
         s = self.solver
         randomize = self.randomize_initial_state if randomize is None else randomize
         if self.load_domain_on_reset:
@@ -284,16 +260,7 @@ class CylinderJet2DEnv(DifferentiableRollout, InitialDomains, Renderable):
                                                  s.stream), "fgb_sample_sensors")
         return {"velocity": vel.permute(0, 2, 1).contiguous(), "pressure": prs[:, 0]}
 
-    def step(self, action):
-        if not self._reset_called:
-            raise RuntimeError("Environment must be reset before stepping. Call 'reset()' before'step()'.")
-        action = torch.as_tensor(action, dtype=torch.float32, device=self.device)
-        if action.shape != self._zero_action.shape:
-            raise ValueError(f"Action shape {action.shape} does not match expected shape {self._zero_action.shape}.")
-        if self._n_steps >= self.episode_length:
-            raise RuntimeError("Episode has already terminated. Call 'reset()' first.")
-        if self.differentiable:
-            return self._step_differentiable(action)
+    def _advance(self, action):
         s = self.solver
         self._acc.zero_()
         nsub = 0
@@ -304,21 +271,18 @@ class CylinderJet2DEnv(DifferentiableRollout, InitialDomains, Renderable):
             native.check(self.lib.fgb_wall_forces(s.handle, C.byref(self.wall), _ptr(s.u), _ptr(s.p), _ptr(s.bvel), _ptr(self._acc),
                                                   s.stream), "fgb_wall_forces")
         self.last_substeps = nsub
-        obs = self._get_obs()
-        mean = self._acc / self.n_sim_steps
-        cd, cl = mean[:, 0], mean[:, 1]
-        reward = self.cd_ref - cd - self.lift_penalty * torch.abs(cl)
-        self._n_steps += 1
-        self._watch_linear_solves()
-        truncated = self._n_steps >= self.episode_length
-        return obs, reward, False, truncated, {"drag": cd.detach(), "lift": cl.detach()}
+        return self._acc
+
+    def _reward(self, cd, cl):
+        """cylinder_env_base.py:769"""
+        return self.cd_ref - cd - self.lift_penalty * torch.abs(cl)
 
     # ---- differentiable mode (fluid_env.py:154,232; examples/interfaces/gradient_based_methods.py) -----------------
     # The PISO substep is one autograd node backed by the CUDA adjoint (fluidgym_b200.autograd); the few boundary
     # and reward formulas around it are tiny torch expressions over the same static tables the kernels use, so
     # gradients flow from the reward to the action, the block velocities and the boundary values exactly as in
     # the reference, where those parts are torch code as well (SIM.py:188-393, forces.py:193-275).
-    def _step_differentiable(self, action):
+    def _advance_differentiable(self, action):
         s = self.solver
         if self._dstate is None:
             self._dstate = (s.u.clone(), s.p.clone(), s.bvel.clone(), self.last_control.clone())
@@ -337,14 +301,7 @@ class CylinderJet2DEnv(DifferentiableRollout, InitialDomains, Renderable):
         with torch.no_grad():                      # keep the solver's own state in step for obs / get_state
             s.u.copy_(u); s.p.copy_(p); s.bvel.copy_(bv); self.last_control.copy_(last)
         self.last_substeps = nsub
-        obs = self._get_obs()
-        mean = acc / self.n_sim_steps
-        cd, cl = mean[:, 0], mean[:, 1]
-        reward = self.cd_ref - cd - self.lift_penalty * torch.abs(cl)
-        self._n_steps += 1
-        self._watch_linear_solves()
-        truncated = self._n_steps >= self.episode_length
-        return obs, reward, False, truncated, {"drag": cd.detach(), "lift": cl.detach()}
+        return acc
 
 
 class CylinderRot2DEnv(CylinderJet2DEnv):

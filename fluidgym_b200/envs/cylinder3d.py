@@ -16,7 +16,8 @@ import numpy as np
 import torch
 
 from ..sensors import sensor_tables_extruded
-from .common import DifferentiableRollout, InitialDomainsExtruded, Renderable, build_wall_tables
+from ..solver import cfl_substeps
+from .common import DifferentiableRollout, EpisodeLifecycle, InitialDomainsExtruded, Renderable, build_wall_tables
 from .cylinder import cylinder_jet_templates, cylinder_sensor_locations
 from .cylinder_domain import BOTTOM, LEFT, RIGHT, TOP, WAKE, make_cylinder_domain
 from .spanwise import global_obs_from_samples, local_obs_windows, spanwise_sensor_voxels
@@ -27,7 +28,7 @@ CYLINDER_JET_3D_DEFAULT_CONFIG = {
 }
 
 
-class SpanwiseExtrudedEnv(InitialDomainsExtruded, Renderable):
+class SpanwiseExtrudedEnv(EpisodeLifecycle, InitialDomainsExtruded, Renderable):
     """What the environments on z-extruded domains with agents lined up along the span share (CylinderJet3D, Airfoil3D): the
     reference-shaped API, reset (zero field + inflow -> projection, or an on-disk initial domain), the solver-step loop with action
     smoothing, per-plane wall forces, voxel sensors, multi-agent windows and the local / global reward mix.  A subclass provides the
@@ -57,10 +58,6 @@ class SpanwiseExtrudedEnv(InitialDomainsExtruded, Renderable):
         return self.n_span if self.use_marl else 1
 
     @property
-    def n_sim_steps(self):
-        return max(1, int(self.step_length / self.dt))
-
-    @property
     def observation_space(self):
         """jet_cylinder_env_3d.py:205-258 (per environment, per agent with use_marl)"""
         from .. import spaces
@@ -73,22 +70,11 @@ class SpanwiseExtrudedEnv(InitialDomainsExtruded, Renderable):
             vs, ps = (self.n_span, spa, 3, nxy), (self.n_span, spa, nxy)
         return spaces.Dict({"velocity": spaces.Box(-inf, inf, shape=vs), "pressure": spaces.Box(-inf, inf, shape=ps)})
 
-    def seed(self, seed: int):
-        self._seed = seed
-        self._np_rng = np.random.default_rng(seed)
-        self._torch_rng = torch.Generator(device=self.device).manual_seed(seed)
-
-    def sample_action(self):
-        if self._seed is None:
-            raise RuntimeError("Environment must be seeded before sampling actions")
-        return torch.rand(self._zero_action.shape, device=self.device, generator=self._torch_rng) * 2 - 1
-
     def set_state(self, u, p, bvel, last_control=None):
         s = self.solver
         for dst, src in ((s.u, u), (s.p, p), (s.bvel, bvel)):
             src = torch.as_tensor(src, dtype=torch.float32, device=self.device)
-            src = src.reshape(dst.shape[1:]) if src.numel() == dst[0].numel() else src.reshape(dst.shape)
-            dst.copy_(src if src.dim() == dst.dim() else src.unsqueeze(0).expand_as(dst))
+            self._copy_state(dst, src.reshape(dst.shape[1:]) if src.numel() == dst[0].numel() else src.reshape(dst.shape))
         if last_control is not None:
             self.last_control.copy_(torch.as_tensor(last_control, device=self.device).expand_as(self.last_control))
         self._reset_called = True
@@ -98,11 +84,7 @@ class SpanwiseExtrudedEnv(InitialDomainsExtruded, Renderable):
         return dict(u=s.u.clone(), p=s.p.clone(), bvel=s.bvel.clone(), last_control=self.last_control.clone())
 
     def reset(self, seed: int | None = None, randomize: bool | None = None):
-        if seed is None:
-            if self._seed is None:
-                raise ValueError("Seed must be provided either during reset or by calling seed().")
-        else:
-            self.seed(seed)
+        self._begin_reset(seed)
         s = self.solver
         randomize = self.randomize_initial_state if randomize is None else randomize
         if self.load_domain_on_reset:
@@ -180,11 +162,6 @@ class SpanwiseExtrudedEnv(InitialDomainsExtruded, Renderable):
     # cuts it: update_advective_boundaries runs entirely under no_grad (SIM.py:232), balance_boundary_fluxes computes its scale under
     # no_grad and applies it outside (SIM.py:191-224).  One common substep size for the batch (the most restrictive environment decides).
     differentiable = False
-    _dstate = None
-
-    def detach(self):
-        if self._dstate is not None:
-            self._dstate = tuple(t.detach() for t in self._dstate)
 
     def mark_state_differentiable(self):
         """envs/util/diff_tools.py:8-22: the velocity leaf of the incoming state [B, 3, nz * N2]"""
@@ -220,20 +197,16 @@ class SpanwiseExtrudedEnv(InitialDomainsExtruded, Renderable):
         from ..autograd import piso_substep_extruded
         s = self.solver
         st = s._st
-        remaining, nsub = float(self.dt), 0
-        while remaining > 0.0 and not abs(remaining) <= 1e-8:                                     # SIM.py:2004-2031
+
+        def max_velocity():
             with torch.no_grad():
                 u4, mi, bm = u.view(self.n_envs, 3, self.nz, s.N2), st["minv"], st["b_minv"]
-                mv = float(torch.stack([(mi[0] * u4[:, 0] + mi[1] * u4[:, 1]).abs().max(), (mi[2] * u4[:, 0] + mi[3] * u4[:, 1]).abs().max(),
-                                        u4[:, 2].abs().max() / s.hz, (bm[0] * bv[:, 0] + bm[1] * bv[:, 1]).abs().max(),
-                                        (bm[2] * bv[:, 0] + bm[3] * bv[:, 1]).abs().max(), bv[:, 2].abs().max() / s.hz]).max())
-            if abs(mv) <= 1e-8:
-                ts = remaining
-            else:
-                mts = np.float32(self.cfl) / np.float32(mv)
-                ts = remaining if float(mts) >= remaining else remaining / float(int(np.ceil(np.float32(remaining) / mts)))
-            remaining -= ts
-            dtv = torch.full((self.n_envs,), float(np.float32(ts)), device=self.device)
+                return float(torch.stack([(mi[0] * u4[:, 0] + mi[1] * u4[:, 1]).abs().max(), (mi[2] * u4[:, 0] + mi[3] * u4[:, 1]).abs().max(),
+                                          u4[:, 2].abs().max() / s.hz, (bm[0] * bv[:, 0] + bm[1] * bv[:, 1]).abs().max(),
+                                          (bm[2] * bv[:, 0] + bm[3] * bv[:, 1]).abs().max(), bv[:, 2].abs().max() / s.hz]).max())
+        nsub = 0
+        for ts in cfl_substeps(self.dt, self.cfl, max_velocity):                                   # SIM.py:2004-2031
+            dtv = torch.full((self.n_envs,), ts, device=self.device)
             bv = self._outflow_fn(u, bv, dtv, self.bc_tol)
             u, p = piso_substep_extruded(s, u, p, bv, dtv)
             nsub += 1
@@ -268,13 +241,7 @@ class SpanwiseExtrudedEnv(InitialDomainsExtruded, Renderable):
         return cds, cls_
 
     def step(self, action):
-        if not self._reset_called:
-            raise RuntimeError("Environment must be reset before stepping. Call 'reset()' before'step()'.")
-        action = torch.as_tensor(action, dtype=torch.float32, device=self.device)
-        if action.shape != self._zero_action.shape:
-            raise ValueError(f"Action shape {action.shape} does not match expected shape {self._zero_action.shape}.")
-        if self._n_steps >= self.episode_length:
-            raise RuntimeError("Episode has already terminated. Call 'reset()' first.")
+        action = self._begin_step(action)
         if self.use_marl and self.local_reward_weight is None:
             raise ValueError("local_reward_weight must be set for multi-agent step.")
         s = self.solver
@@ -297,9 +264,7 @@ class SpanwiseExtrudedEnv(InitialDomainsExtruded, Renderable):
         all_cds, all_cls = cds / self.n_sim_steps, cls_ / self.n_sim_steps
         cd, cl = all_cds.sum(dim=1) / self.D, all_cls.sum(dim=1) / self.D                        # jet_cylinder_env_3d.py:431-452
         reward = self._reward(cd, cl)
-        self._n_steps += 1
-        self._watch_linear_solves()
-        truncated = self._n_steps >= self.episode_length
+        truncated = self._end_step()
         info = {"drag": cd, "lift": cl}
         if not self.use_marl:
             info["all_cds"], info["all_cls"] = all_cds, all_cls
@@ -374,7 +339,6 @@ class CylinderJet3DEnv(SpanwiseExtrudedEnv):
         self.last_control = torch.zeros(B, self.n_jets, device=dev)
         self._zero_action = torch.zeros(B, self.n_jets, 1, device=dev)
         self._bvel0 = torch.from_numpy(np.ascontiguousarray(cd.bvel0[:, :cd.NB])).to(dev)
-        self._reset_called, self._seed, self._n_steps, self.last_substeps = False, None, 0, 0
 
     @property
     def render_shape(self):

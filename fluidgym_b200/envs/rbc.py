@@ -14,8 +14,8 @@ import torch
 
 from .. import native
 from ..sensors import sensor_tables
-from ..solver import BatchedPISO, _ptr
-from .common import InitialDomains, Renderable
+from ..solver import BatchedPISO, _ptr, cfl_substeps
+from .common import EpisodeLifecycle, InitialDomains, Renderable
 from .rbc_domain import make_rbc_domain
 
 RBC_2D_DEFAULT_CONFIG = {
@@ -38,7 +38,7 @@ def extract_moving_window_2d(field: torch.Tensor, n_agents: int, agent_width: in
     return win.reshape(*lead, n_agents, Y, n_agents_per_window * agent_width)
 
 
-class RBC2DEnv(InitialDomains, Renderable):
+class RBC2DEnv(EpisodeLifecycle, InitialDomains, Renderable):
     T_cold, T_hot, heater_limit = 0.0, 1.0, 0.75
     n_sensors_y, n_sensors_per_heater = 8, 4
     buoyancy_factor = 1.0
@@ -60,7 +60,6 @@ class RBC2DEnv(InitialDomains, Renderable):
         self.use_marl, self.nu_ref = bool(use_marl), float(nu_ref)
         self.enable_actions = enable_actions
         self.differentiable = bool(differentiable)
-        self._dstate = None          # (u, p, T, sbval) carried with their autograd history in differentiable mode
         self.randomize_initial_state = randomize_initial_state
         self.load_domain_on_reset, self.initial_domains_path = bool(load_initial_domain), initial_domains_path
         self.prandtl_number, self.rayleigh_number = prandtl_number, rayleigh_number
@@ -77,8 +76,6 @@ class RBC2DEnv(InitialDomains, Renderable):
         self._bottom = slice(int(self.cd.boff[0, 2]), int(self.cd.boff[0, 2]) + self.nx)
         self._setup_sensors()
         self._zero_action = torch.zeros(self.n_envs, self.n_heaters, 1, device=self.device)
-        self._reset_called, self._seed, self._n_steps = False, None, 0
-        self.last_substeps = 0
 
     # ---- static tables ---------------------------------------------------------------------------
     @property
@@ -111,10 +108,6 @@ class RBC2DEnv(InitialDomains, Renderable):
         return self.n_heaters if self.use_marl else 1
 
     @property
-    def n_sim_steps(self):
-        return max(1, int(self.step_length / self.dt))
-
-    @property
     def initial_domain_id(self):
         """rbc_env_base.py:606-611"""
         return f"rbc_2d_Ra{self.rayleigh_number}_Pr{self.prandtl_number}_NH{self.n_heaters}_HW{self.heater_width}"
@@ -134,41 +127,24 @@ class RBC2DEnv(InitialDomains, Renderable):
         from .. import spaces
         return spaces.Box(-1.0, 1.0, shape=(1,) if self.use_marl else (self.n_heaters, 1))
 
-    def seed(self, seed: int):
-        self._seed = seed
-        self._np_rng = np.random.default_rng(seed)
-        self._torch_rng = torch.Generator(device=self.device).manual_seed(seed)
-
-    def sample_action(self):
-        if self._seed is None:
-            raise RuntimeError("Environment must be seeded before sampling actions")
-        return torch.rand(self._zero_action.shape, device=self.device, generator=self._torch_rng) * 2 - 1
-
     def set_state(self, u, p, T, sbval=None, ures=None):
         s = self.solver
         for dst, src in ((s.u, u), (s.p, p), (s.T, T)):
-            src = torch.as_tensor(src, dtype=torch.float32, device=self.device)
-            dst.copy_(src if src.dim() == dst.dim() else src.unsqueeze(0).expand_as(dst))
+            self._copy_state(dst, src)
         if sbval is not None:
-            sb = torch.as_tensor(sbval, dtype=torch.float32, device=self.device)
-            s.sbval.copy_(sb if sb.dim() == 2 else sb.unsqueeze(0).expand_as(s.sbval))
+            self._copy_state(s.sbval, sbval)
         ur = s.buffer("ures")
         if ures is None:
             ur.zero_()
         else:
-            ures = torch.as_tensor(ures, dtype=torch.float32, device=self.device)
-            ur.copy_(ures if ures.dim() == 3 else ures.unsqueeze(0).expand_as(ur))
+            self._copy_state(ur, ures)
         self._reset_called = True
         self._dstate = None
 
     def reset(self, seed: int | None = None, randomize: bool | None = None):
         """rbc_env_base.py:190-278: linear temperature profile + 0.1 N(0,1) clamped to [T_cold, T_hot],
         velocity 0.05 N(0,1) (per environment streams of one generator)."""
-        if seed is None:
-            if self._seed is None:
-                raise ValueError("Seed must be provided either during reset or by calling seed().")
-        else:
-            self.seed(seed)
+        self._begin_reset(seed)
         s = self.solver
         B, nx, ny = self.n_envs, self.nx, self.ny
         self._dstate = None
@@ -287,11 +263,7 @@ class RBC2DEnv(InitialDomains, Renderable):
     # One autograd node per substep (scalar transport + buoyancy + PISO, fluidgym_b200.autograd.PISOSubstepScalar backed by
     # the CUDA adjoint); the heater profile (rbc_env_2d.py:210-282) and the Nusselt sums (rbc_env_base.py:491-539) around it
     # are torch expressions, as in the reference.  The CFL plan is taken from detached maxima with one common substep size
-    # for the batch (the most restrictive environment decides), like envs/common.py::_single_step_differentiable.
-    def detach(self):
-        if self._dstate is not None:
-            self._dstate = tuple(t.detach() for t in self._dstate)
-
+    # for the batch (the most restrictive environment decides): solver.cfl_substeps.
     def _advance_differentiable(self, action):
         from ..autograd import piso_substep_scalar
         s = self.solver
@@ -303,20 +275,14 @@ class RBC2DEnv(InitialDomains, Renderable):
             sb = sb.index_copy(1, torch.arange(self._bottom.start, self._bottom.stop, device=self.device), ctrl)
         bv = s.bvel
         mvb = torch.empty(self.n_envs, device=self.device)
+
+        def max_velocity():
+            native.check(self.lib.fgb_max_velocity(s.handle, _ptr(u.detach().contiguous()), _ptr(bv), _ptr(mvb), s.stream), "fgb_max_velocity")
+            return float(mvb.max())
         nsub = 0
         for _ in range(self.n_sim_steps):
-            remaining = float(self.dt)
-            while remaining > 0.0 and not abs(remaining) <= 1e-8:            # SIM.py:2004-2031
-                native.check(self.lib.fgb_max_velocity(s.handle, _ptr(u.detach().contiguous()), _ptr(bv), _ptr(mvb), s.stream),
-                             "fgb_max_velocity")
-                mv = float(mvb.max())
-                if abs(mv) <= 1e-8:
-                    ts = remaining
-                else:
-                    mts = np.float32(self.cfl) / np.float32(mv)
-                    ts = remaining if float(mts) >= remaining else remaining / float(np.ceil(np.float32(remaining) / mts))
-                remaining -= ts
-                u, p, T = piso_substep_scalar(s, u, p, bv, T, sb, float(np.float32(ts)), self.buoyancy_factor)
+            for ts in cfl_substeps(self.dt, self.cfl, max_velocity):                 # SIM.py:2004-2031
+                u, p, T = piso_substep_scalar(s, u, p, bv, T, sb, ts, self.buoyancy_factor)
                 nsub += 1
         self._dstate = (u, p, T, sb)
         with torch.no_grad():                      # keep the solver's own state in step for observations / get_state
@@ -332,13 +298,7 @@ class RBC2DEnv(InitialDomains, Renderable):
         return self._det_t
 
     def step(self, action):
-        if not self._reset_called:
-            raise RuntimeError("Environment must be reset before stepping. Call 'reset()' before'step()'.")
-        action = torch.as_tensor(action, dtype=torch.float32, device=self.device)
-        if action.shape != self._zero_action.shape:
-            raise ValueError(f"Action shape {action.shape} does not match expected shape {self._zero_action.shape}.")
-        if self._n_steps >= self.episode_length:
-            raise RuntimeError("Episode has already terminated. Call 'reset()' first.")
+        action = self._begin_step(action)
         if self.differentiable:
             cs = self._advance_differentiable(action)
         else:
@@ -352,9 +312,7 @@ class RBC2DEnv(InitialDomains, Renderable):
         nu = self.compute_global_nusselt(cs)
         reward = self.nu_ref - nu
         info = {"nusselt": nu.detach()}
-        self._n_steps += 1
-        self._watch_linear_solves()
-        truncated = self._n_steps >= self.episode_length
+        truncated = self._end_step()
         if not self.use_marl:
             return self._get_global_obs(), reward, False, truncated, info
         lw = self.local_reward_weight

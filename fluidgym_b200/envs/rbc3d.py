@@ -17,8 +17,8 @@ from .. import native
 from ..box3d import BatchedPISO3D, Box3DDomain
 from ..grids import wall_refined_ortho_grid
 from ..sensors import sensor_tables_3d
-from ..solver import _ptr
-from .common import InitialDomains3D, Renderable
+from ..solver import _ptr, cfl_substeps
+from .common import EpisodeLifecycle, InitialDomains3D, Renderable
 
 RBC_3D_DEFAULT_CONFIG = {
     "rayleigh_number": 2e3, "prandtl_number": 0.7, "n_heaters": 8, "resolution": 8, "dt": 0.05, "adaptive_cfl": 0.8,
@@ -54,7 +54,7 @@ def extract_moving_window_3d(field: torch.Tensor, n_agents: int, agent_width: in
     return fzx.reshape(*lead, n_agents * n_agents, cells.shape[1], Y, cells.shape[1])
 
 
-class RBC3DEnv(InitialDomains3D, Renderable):
+class RBC3DEnv(EpisodeLifecycle, InitialDomains3D, Renderable):
     T_cold, T_hot, heater_limit = 0.0, 1.0, 0.75
     n_sensors_y, n_sensors_per_heater = 8, 4
     buoyancy_factor = 1.0
@@ -71,7 +71,6 @@ class RBC3DEnv(InitialDomains3D, Renderable):
                  differentiable=False):
         self.n_envs = int(n_envs)
         self.differentiable = bool(differentiable)
-        self._dstate = None          # (u, p, T, sbval) carried with their autograd history in differentiable mode
         self.load_domain_on_reset, self.initial_domains_path = bool(load_initial_domain), initial_domains_path
         self.rayleigh_number, self.prandtl_number = rayleigh_number, prandtl_number
         self.Ra, self.Pr = float(rayleigh_number), float(prandtl_number)
@@ -104,7 +103,6 @@ class RBC3DEnv(InitialDomains3D, Renderable):
         self._setup_sensors()
         self._zero_action = torch.zeros(self.n_envs, self.n_heaters ** 2, 1, device=self.device) if self.use_marl else \
             torch.zeros(self.n_envs, self.n_heaters, self.n_heaters, 1, device=self.device)
-        self._reset_called, self._seed, self._n_steps, self.last_substeps = False, None, 0, 0
 
     # ---- static tables ---------------------------------------------------------------------------
     @property
@@ -147,10 +145,6 @@ class RBC3DEnv(InitialDomains3D, Renderable):
         return self.n_heaters ** 2 if self.use_marl else 1
 
     @property
-    def n_sim_steps(self):
-        return max(1, int(self.step_length / self.dt))
-
-    @property
     def initial_domain_id(self):
         """rbc_env_base.py:606-611"""
         return f"rbc_3d_Ra{self.rayleigh_number}_Pr{self.prandtl_number}_NH{self.n_heaters}_HW{self.heater_width}"
@@ -169,40 +163,23 @@ class RBC3DEnv(InitialDomains3D, Renderable):
         from .. import spaces
         return spaces.Box(-1.0, 1.0, shape=(1,) if self.use_marl else (self.n_heaters, self.n_heaters, 1))
 
-    def seed(self, seed: int):
-        self._seed = seed
-        self._np_rng = np.random.default_rng(seed)
-        self._torch_rng = torch.Generator(device=self.device).manual_seed(seed)
-
-    def sample_action(self):
-        if self._seed is None:
-            raise RuntimeError("Environment must be seeded before sampling actions")
-        return torch.rand(self._zero_action.shape, device=self.device, generator=self._torch_rng) * 2 - 1
-
     def set_state(self, u, p, T, sbval=None, ures=None):
         s = self.solver
         for dst, src in ((s.u, u), (s.p, p), (s.T, T)):
-            src = torch.as_tensor(src, dtype=torch.float32, device=self.device)
-            dst.copy_(src if src.dim() == dst.dim() else src.unsqueeze(0).expand_as(dst))
+            self._copy_state(dst, src)
         if sbval is not None:
-            sb = torch.as_tensor(sbval, dtype=torch.float32, device=self.device)
-            s.sbval.copy_(sb if sb.dim() == 2 else sb.unsqueeze(0).expand_as(s.sbval))
+            self._copy_state(s.sbval, sbval)
         ur = s.buffer("ures")
         if ures is None:
             ur.zero_()
         else:
-            ures = torch.as_tensor(ures, dtype=torch.float32, device=self.device)
-            ur.copy_(ures if ures.dim() == 3 else ures.unsqueeze(0).expand_as(ur))
+            self._copy_state(ur, ures)
         self._reset_called = True
 
     def reset(self, seed: int | None = None, randomize: bool | None = None):
         """rbc_env_base.py:190-278 with ndims = 3: linear temperature profile + 0.1 N(0,1) clamped to [T_cold, T_hot], velocity
         0.05 N(0,1); ``randomize`` adds the mirror / shift / noise / settling of rbc_env_base.py:336-393 per environment."""
-        if seed is None:
-            if self._seed is None:
-                raise ValueError("Seed must be provided either during reset or by calling seed().")
-        else:
-            self.seed(seed)
+        self._begin_reset(seed)
         s = self.solver
         B, nx, ny, nz = self.n_envs, self.nx, self.ny, self.nz
         randomize = self.randomize_initial_state if randomize is None else randomize
@@ -336,10 +313,6 @@ class RBC3DEnv(InitialDomains3D, Renderable):
     # ---- differentiable mode: one autograd node per substep (autograd.PISOSubstepScalar3D, CUDA adjoint of the D = 3 box path); the
     # heater profile and the Nusselt integrals around it are torch expressions, as in the reference.  The CFL plan is taken from
     # detached maxima with one common substep size for the batch (the most restrictive environment decides).
-    def detach(self):
-        if self._dstate is not None:
-            self._dstate = tuple(t.detach() for t in self._dstate)
-
     def mark_state_differentiable(self):
         """envs/util/diff_tools.py:8-22: (velocity, temperature) leaves of the incoming state"""
         s = self.solver
@@ -358,19 +331,14 @@ class RBC3DEnv(InitialDomains3D, Renderable):
             sb = sb.index_copy(1, torch.arange(self._bottom.start, self._bottom.stop, device=self.device), ctrl)
         bv = s.bvel
         minv, b_minv = s._tab["minv"].reshape(1, 3, -1), s._tab["b_minv"].reshape(1, 3, -1)
+
+        def max_velocity():
+            with torch.no_grad():
+                return float(torch.maximum((minv * u).abs().max(), (b_minv * bv).abs().max()))
         nsub = 0
         for _ in range(self.n_sim_steps):
-            remaining = float(self.dt)
-            while remaining > 0.0 and not abs(remaining) <= 1e-8:            # SIM.py:2004-2031
-                with torch.no_grad():
-                    mv = float(torch.maximum((minv * u).abs().max(), (b_minv * bv).abs().max()))
-                if abs(mv) <= 1e-8:
-                    ts = remaining
-                else:
-                    mts = np.float32(self.cfl) / np.float32(mv)
-                    ts = remaining if float(mts) >= remaining else remaining / float(int(np.ceil(np.float32(remaining) / mts)))
-                remaining -= ts
-                u, p, T = piso_substep_scalar_3d(s, u, p, bv, T, sb, float(np.float32(ts)))
+            for ts in cfl_substeps(self.dt, self.cfl, max_velocity):                 # SIM.py:2004-2031
+                u, p, T = piso_substep_scalar_3d(s, u, p, bv, T, sb, ts)
                 nsub += 1
         self._dstate = (u, p, T, sb)
         with torch.no_grad():                      # keep the solver's own state in step for observations / get_state
@@ -379,13 +347,7 @@ class RBC3DEnv(InitialDomains3D, Renderable):
         return u, T
 
     def step(self, action):
-        if not self._reset_called:
-            raise RuntimeError("Environment must be reset before stepping. Call 'reset()' before'step()'.")
-        action = torch.as_tensor(action, dtype=torch.float32, device=self.device)
-        if action.shape != self._zero_action.shape:
-            raise ValueError(f"Action shape {action.shape} does not match expected shape {self._zero_action.shape}.")
-        if self._n_steps >= self.episode_length:
-            raise RuntimeError("Episode has already terminated. Call 'reset()' first.")
+        action = self._begin_step(action)
         if self.differentiable:
             self._dfields = self._advance_differentiable(action)
         else:
@@ -399,9 +361,7 @@ class RBC3DEnv(InitialDomains3D, Renderable):
         nu = self.compute_global_nusselt()
         reward = self.nu_ref - nu
         info = {"nusselt": nu.detach()}
-        self._n_steps += 1
-        self._watch_linear_solves()
-        truncated = self._n_steps >= self.episode_length
+        truncated = self._end_step()
         if not self.use_marl:
             return self._get_global_obs(), reward, False, truncated, info
         lw = self.local_reward_weight

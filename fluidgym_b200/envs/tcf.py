@@ -11,7 +11,8 @@ import torch
 
 from ..box3d import BatchedPISO3D, Box3DDomain
 from ..grids import channel_vertex_grid
-from .common import InitialDomains3D, Renderable
+from ..solver import cfl_substeps
+from .common import EpisodeLifecycle, InitialDomains3D, Renderable
 
 SMALL_TCF_3D_DEFAULT_CONFIG = {
     "resolution_y": 65, "resolution_x_z": 64, "actor_size": 2, "L": np.pi, "D": np.pi / 2, "reynolds_number_wall": 180,
@@ -39,7 +40,7 @@ def agent_window_means(field, n_agents_x, n_agents_z, agent_width, wx, wz, pad_x
     return win.reshape(*lead, n_agents_x * n_agents_z, wz, wx)
 
 
-class TCF3DEnv(InitialDomains3D, Renderable):
+class TCF3DEnv(EpisodeLifecycle, InitialDomains3D, Renderable):
     delta, H = 1.0, 2.0
     y_obs_wall = 15.0
     metrics = ["wall_stress", "wall_stress_bottom", "wall_stress_top"]
@@ -111,16 +112,11 @@ class TCF3DEnv(InitialDomains3D, Renderable):
         self._acc = torch.zeros(self.n_envs, 2, device=dev)
         shape = (self.n_agents, 1)
         self._zero_action = torch.zeros(self.n_envs, *shape, device=dev)
-        self._reset_called, self._seed, self._n_steps, self.last_substeps = False, None, 0, 0
 
     # ---- reference-shaped API ---------------------------------------------------------------------
     @property
     def n_agents(self):
         return self.nax * self.naz * (2 if self.both_walls else 1)
-
-    @property
-    def n_sim_steps(self):
-        return max(1, int(self.step_length / self.dt))
 
     @property
     def initial_domain_id(self):
@@ -141,21 +137,10 @@ class TCF3DEnv(InitialDomains3D, Renderable):
         from .. import spaces
         return spaces.Box(-1.0, 1.0, shape=(1,) if self.use_marl else (self.n_agents, 1))
 
-    def seed(self, seed: int):
-        self._seed = seed
-        self._np_rng = np.random.default_rng(seed)
-        self._torch_rng = torch.Generator(device=self.device).manual_seed(seed)
-
-    def sample_action(self):
-        if self._seed is None:
-            raise RuntimeError("Environment must be seeded before sampling actions")
-        return torch.rand(self._zero_action.shape, device=self.device, generator=self._torch_rng) * 2 - 1
-
     def set_state(self, u, p, bvel=None):
         s = self.solver
         for dst, src in ((s.u, u), (s.p, p)) + (((s.bvel, bvel),) if bvel is not None else ()):
-            src = torch.as_tensor(src, dtype=torch.float32, device=self.device)
-            dst.copy_(src if src.dim() == dst.dim() else src.unsqueeze(0).expand_as(dst))
+            self._copy_state(dst, src)
         self._reset_called = True
 
     def get_state(self):
@@ -163,11 +148,7 @@ class TCF3DEnv(InitialDomains3D, Renderable):
         return dict(u=s.u.clone(), p=s.p.clone(), bvel=s.bvel.clone())
 
     def reset(self, seed: int | None = None, randomize: bool | None = None):
-        if seed is None:
-            if self._seed is None:
-                raise ValueError("Seed must be provided either during reset or by calling seed().")
-        else:
-            self.seed(seed)
+        self._begin_reset(seed)
         s = self.solver
         randomize = self.randomize_initial_state if randomize is None else randomize
         if self.load_domain_on_reset:                      # fluid_env.py:519-551
@@ -296,17 +277,13 @@ class TCF3DEnv(InitialDomains3D, Renderable):
         s = self.solver
         minv = s._tab["minv"].reshape(1, 3, -1)
         b_minv = s._tab["b_minv"].reshape(1, 3, -1)
-        remaining, nsub = float(self.dt), 0
-        while remaining > 0.0 and not abs(remaining) <= 1e-8:
+
+        def max_velocity():
             with torch.no_grad():
-                mv = float(torch.maximum((minv * u).abs().max(), (b_minv * bv).abs().max()))
-            if abs(mv) <= 1e-8:
-                ts = remaining
-            else:
-                mts = np.float32(self.cfl) / np.float32(mv)
-                ts = remaining if float(mts) >= remaining else remaining / float(int(np.ceil(np.float32(remaining) / mts)))
-            remaining -= ts
-            u, p = piso_substep_3d(s, u, p, bv, float(np.float32(ts)), self._forcing_torch(u))
+                return float(torch.maximum((minv * u).abs().max(), (b_minv * bv).abs().max()))
+        nsub = 0
+        for ts in cfl_substeps(self.dt, self.cfl, max_velocity):
+            u, p = piso_substep_3d(s, u, p, bv, ts, self._forcing_torch(u))
             nsub += 1
         return u, p, nsub
 
@@ -318,7 +295,7 @@ class TCF3DEnv(InitialDomains3D, Renderable):
     def detach(self):
         self._du = None
 
-    def _step_differentiable(self, action):
+    def _advance_differentiable(self, action):
         s = self.solver
         u = self._du if getattr(self, "_du", None) is not None else s.u.detach().clone()
         p = s.p.detach().clone()
@@ -346,26 +323,8 @@ class TCF3DEnv(InitialDomains3D, Renderable):
         tau_bottom, tau_top = torch.stack(tb).mean(dim=0), torch.stack(tt).mean(dim=0)
         return tau_bottom, tau_top
 
-    def step(self, action):
-        if not self._reset_called:
-            raise RuntimeError("Environment must be reset before stepping. Call 'reset()' before'step()'.")
-        action = torch.as_tensor(action, dtype=torch.float32, device=self.device)
-        if action.shape != self._zero_action.shape:
-            raise ValueError(f"Action shape {action.shape} does not match expected shape {self._zero_action.shape}.")
-        if self._n_steps >= self.episode_length:
-            raise RuntimeError("Episode has already terminated. Call 'reset()' first.")
-        if self.differentiable:
-            tau_bottom, tau_top = self._step_differentiable(action)
-            tau_total = 0.5 * (tau_bottom + tau_top)
-            reward = 1 - (tau_total if self.both_walls else tau_bottom) / self.tau_ref
-            info = {"wall_stress": tau_total, "wall_stress_bottom": tau_bottom, "wall_stress_top": tau_top}
-            self._n_steps += 1
-            self._watch_linear_solves()
-            obs = self._get_obs()
-            if self.use_marl:
-                info["global_reward"] = reward
-                reward = reward[:, None] * torch.ones(self.n_envs, self.n_agents, device=self.device)
-            return obs, reward, False, self._n_steps >= self.episode_length, info
+    def _advance(self, action):
+        """-> (tau_bottom, tau_top) [B]: the wall shear stresses averaged over the solver steps"""
         if self.enable_actions:
             self._apply_action(action)
         s = self.solver
@@ -376,13 +335,15 @@ class TCF3DEnv(InitialDomains3D, Renderable):
             s.wall_rows(self.rows, self.d_lo, self.d_hi, set_forcing=False, acc=self._acc)
         self.last_substeps = nsub
         tau = self._acc / self.n_sim_steps
-        tau_bottom, tau_top = tau[:, 0], tau[:, 1]
+        return tau[:, 0], tau[:, 1]
+
+    def step(self, action):
+        action = self._begin_step(action)
+        tau_bottom, tau_top = self._advance_differentiable(action) if self.differentiable else self._advance(action)
         tau_total = 0.5 * (tau_bottom + tau_top)
         reward = 1 - (tau_total if self.both_walls else tau_bottom) / self.tau_ref
         info = {"wall_stress": tau_total, "wall_stress_bottom": tau_bottom, "wall_stress_top": tau_top}
-        self._n_steps += 1
-        self._watch_linear_solves()
-        truncated = self._n_steps >= self.episode_length
+        truncated = self._end_step()
         obs = self._get_obs()
         if self.use_marl:
             info["global_reward"] = reward

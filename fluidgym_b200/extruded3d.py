@@ -16,7 +16,7 @@ import torch
 
 from . import native
 from .domain import CompiledDomain
-from .solver import _TABLE_FIELDS, _ptr
+from .solver import _TABLE_FIELDS, _ptr, cfl_substep
 
 
 def extruded_neighbours(nbr2: np.ndarray, nz: int) -> np.ndarray:
@@ -106,13 +106,8 @@ class ExtrudedStepping:
             mv = self.max_velocity().detach().cpu().numpy().astype(np.float32)
             ts = np.zeros(B, dtype=np.float64)
             for b in np.nonzero(act)[0]:
-                rem = remaining[b]
-                if abs(mv[b]) <= 1e-8:
-                    ts[b] = rem
-                else:
-                    mts = np.float32(cfl) / mv[b]
-                    ts[b] = rem if float(mts) >= rem else rem / float(np.ceil(np.float32(rem) / mts))
-                remaining[b] = rem - ts[b]
+                ts[b] = cfl_substep(float(remaining[b]), cfl, float(mv[b]))
+                remaining[b] -= ts[b]
             keep = None
             if not act.all():                       # finished environments ride along with a dummy step and are restored afterwards
                 idle = torch.from_numpy(np.nonzero(~act)[0]).to(self.device)

@@ -24,6 +24,26 @@ def _ptr(t):
     return C.c_void_p(t.data_ptr()) if t is not None else None
 
 
+def cfl_substep(remaining: float, cfl: float, max_vel: float) -> float:
+    """Size of the next substep of the adaptive CFL plan (SIM.py:2004-2031), in k_plan_substep's precision: the CFL-limited
+    step cfl / max_vel is formed in float32, ``remaining`` stays float64 and is split into equal parts when it is longer."""
+    if abs(max_vel) <= 1e-8:
+        return remaining
+    mts = np.float32(cfl) / np.float32(max_vel)
+    return remaining if float(mts) >= remaining else remaining / float(np.ceil(np.float32(remaining) / mts))
+
+
+def cfl_substeps(dt: float, cfl: float, max_velocity):
+    """The substeps of one solver step of length ``dt``: yields each size rounded to float32 (what the substep kernels take).
+    ``max_velocity()`` returns the maximum velocity of the batch as a Python float and is called before every substep, so one
+    common size serves the whole batch (the most restrictive environment decides)."""
+    remaining = float(dt)
+    while remaining > 0.0 and not abs(remaining) <= 1e-8:
+        ts = cfl_substep(remaining, cfl, max_velocity())
+        remaining -= ts
+        yield float(np.float32(ts))
+
+
 def cluster_shape(N: int, cg_impl: int = 6):
     """(cluster size, cells per CTA incl. padding) the on-chip Krylov launchers pick for a grid of N cells
     (cg_cluster_mb_any in csrc/piso_b200.cu): smallest cluster whose CTAs hold ceil(N/CS) cells."""
