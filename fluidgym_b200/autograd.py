@@ -9,6 +9,11 @@ pressure ``p`` (enters through the deferred non-orthogonal correction) and the D
 ``bvel`` (jets / inflow); geometry and viscosity are constants, like the transforms in the reference.
 ``PISOSubstepScalar`` is the same node for domains with a passive scalar and buoyancy (RBC): additional
 differentiable inputs are the temperature field and the boundary temperatures (heaters).
+
+Every node takes an optional ``active`` mask (int32 ``[B]`` on the solver's device, 0 = skip; ``None`` = every environment): a
+skipped environment is the identity in both directions -- its outputs are its inputs bit for bit, its cotangents pass through
+unchanged and its boundary values get none.  Per-environment CFL plans (``solver.cfl_substeps_per_env``) use it for environments
+that have already used up their time.
 """
 from __future__ import annotations
 
@@ -32,6 +37,19 @@ def _new_tape(solver: BatchedPISO):
                 pmean=torch.empty(C_ * n_p, B, **f32), u1=torch.empty(max(C_ - 1, 1), B, 2, N, **f32))
 
 
+def _ctape(cls, tape: dict, active):
+    """the C tape of the buffers in ``tape`` (native.Tape / native.Ortho3Tape) with the environment mask ``active`` (or None)"""
+    return cls(*[tape[k].data_ptr() for k, _ in cls._fields_ if k != "active"], active.data_ptr() if active is not None else None)
+
+
+def _mask(solver, active):
+    if active is None:
+        return None
+    if active.dtype != torch.int32 or tuple(active.shape) != (solver.B,) or active.device.type != solver.device.type:
+        raise ValueError(f"active must be an int32 tensor of shape ({solver.B},) on {solver.device}")
+    return active.contiguous()
+
+
 def _adjoint_workspace(solver: BatchedPISO):
     nbytes = solver.lib.fgb_adjoint_workspace_bytes(C.byref(solver.tables), solver.B)
     ws = getattr(solver, "_adj_ws", None)
@@ -44,16 +62,17 @@ class PISOSubstep(torch.autograd.Function):
     """(u [B,2,N], p [B,N], bvel [B,2,NB]) -> (u_next, p_next) for one substep of ``dt`` (tensor [B] or float)."""
 
     @staticmethod
-    def forward(ctx, u, p, bvel, solver: BatchedPISO, dt):
+    def forward(ctx, u, p, bvel, solver: BatchedPISO, dt, active=None):
         dtc = solver._dt(dt)
+        active = _mask(solver, active)
         tape = _new_tape(solver)
-        ct = native.Tape(*[tape[k].data_ptr() for k, _ in native.Tape._fields_])
+        ct = _ctape(native.Tape, tape, active)
         u_out = u.detach().clone().contiguous()
         p_out = p.detach().clone().contiguous()
         bv = bvel.detach().contiguous()
         native.check(solver.lib.fgb_piso_substep_record(solver.handle, _ptr(u_out), _ptr(p_out), _ptr(bv), _ptr(dtc), C.byref(ct),
                                                         solver.stream), "fgb_piso_substep_record")
-        ctx.solver, ctx.tape = solver, tape
+        ctx.solver, ctx.tape, ctx.active = solver, tape, active
         return u_out, p_out
 
     @staticmethod
@@ -61,14 +80,14 @@ class PISOSubstep(torch.autograd.Function):
         solver, tape = ctx.solver, ctx.tape
         B, N, NB = solver.B, solver.N, solver.NB
         f32 = dict(device=solver.device, dtype=torch.float32)
-        ct = native.Tape(*[tape[k].data_ptr() for k, _ in native.Tape._fields_])
+        ct = _ctape(native.Tape, tape, ctx.active)
         ub, pb, bvb = torch.empty(B, 2, N, **f32), torch.empty(B, N, **f32), torch.empty(B, 2, NB, **f32)
         ws, nbytes = _adjoint_workspace(solver)
         uo = (u_out_bar if u_out_bar is not None else torch.zeros(B, 2, N, **f32)).contiguous()
         po = (p_out_bar if p_out_bar is not None else torch.zeros(B, N, **f32)).contiguous()
         native.check(solver.lib.fgb_piso_substep_backward(solver.handle, C.byref(ct), _ptr(uo), _ptr(po), _ptr(ub), _ptr(pb), _ptr(bvb),
                                                           ws, nbytes, solver.stream), "fgb_piso_substep_backward")
-        return ub, pb, bvb, None, None
+        return ub, pb, bvb, None, None, None
 
 
 class PISOSubstepScalar(torch.autograd.Function):
@@ -76,13 +95,14 @@ class PISOSubstepScalar(torch.autograd.Function):
     incoming velocity, buoyancy source ``(0, beta T_next)``, PISO substep (SIM.py:1471-1657, rbc_env_base.py:280-304)."""
 
     @staticmethod
-    def forward(ctx, u, p, bvel, T, sbval, solver: BatchedPISO, dt, beta):
+    def forward(ctx, u, p, bvel, T, sbval, solver: BatchedPISO, dt, beta, active=None):
         dtc = solver._dt(dt)
+        active = _mask(solver, active)
         tape = _new_tape(solver)
         f32 = dict(device=solver.device, dtype=torch.float32)
         stape = dict(T_in=torch.empty(solver.B, solver.N, **f32), T_out=torch.empty(solver.B, solver.N, **f32),
                      sbval_in=torch.empty(solver.B, solver.NB, **f32))
-        ct = native.Tape(*[tape[k].data_ptr() for k, _ in native.Tape._fields_])
+        ct = _ctape(native.Tape, tape, active)
         cs = native.ScalarTape(*[stape[k].data_ptr() for k, _ in native.ScalarTape._fields_])
         u_out, p_out, T_out = (x.detach().clone().contiguous() for x in (u, p, T))
         bv, sb = bvel.detach().contiguous(), sbval.detach().contiguous()
@@ -90,7 +110,7 @@ class PISOSubstepScalar(torch.autograd.Function):
         sc = native.Scalar(T_out.data_ptr(), sb.data_ptr(), float(beta), src.data_ptr())
         native.check(solver.lib.fgb_piso_substep_record_scalar(solver.handle, _ptr(u_out), _ptr(p_out), _ptr(bv), _ptr(dtc), C.byref(sc),
                                                                C.byref(ct), C.byref(cs), solver.stream), "fgb_piso_substep_record_scalar")
-        ctx.solver, ctx.tape, ctx.stape, ctx.beta = solver, tape, stape, float(beta)
+        ctx.solver, ctx.tape, ctx.stape, ctx.beta, ctx.active = solver, tape, stape, float(beta), active
         return u_out, p_out, T_out
 
     @staticmethod
@@ -98,7 +118,7 @@ class PISOSubstepScalar(torch.autograd.Function):
         solver, tape, stape = ctx.solver, ctx.tape, ctx.stape
         B, N, NB = solver.B, solver.N, solver.NB
         f32 = dict(device=solver.device, dtype=torch.float32)
-        ct = native.Tape(*[tape[k].data_ptr() for k, _ in native.Tape._fields_])
+        ct = _ctape(native.Tape, tape, ctx.active)
         cs = native.ScalarTape(*[stape[k].data_ptr() for k, _ in native.ScalarTape._fields_])
         ub, pb, bvb = torch.empty(B, 2, N, **f32), torch.empty(B, N, **f32), torch.empty(B, 2, NB, **f32)
         Tb, sbb = torch.empty(B, N, **f32), torch.empty(B, NB, **f32)
@@ -109,17 +129,18 @@ class PISOSubstepScalar(torch.autograd.Function):
         native.check(solver.lib.fgb_piso_substep_backward_scalar(solver.handle, C.byref(ct), C.byref(cs), ctx.beta, _ptr(uo), _ptr(po),
                                                                  _ptr(To), _ptr(ub), _ptr(pb), _ptr(bvb), _ptr(Tb), _ptr(sbb), ws, nbytes,
                                                                  solver.stream), "fgb_piso_substep_backward_scalar")
-        return ub, pb, bvb, Tb, sbb, None, None, None
+        return ub, pb, bvb, Tb, sbb, None, None, None, None
 
 
-def piso_substep_scalar(solver: BatchedPISO, u, p, bvel, T, sbval, dt, beta=1.0):
-    """Differentiable substep of a domain with passive scalar + buoyancy (functional form)."""
-    return PISOSubstepScalar.apply(u, p, bvel, T, sbval, solver, dt, beta)
+def piso_substep_scalar(solver: BatchedPISO, u, p, bvel, T, sbval, dt, beta=1.0, active=None):
+    """Differentiable substep of a domain with passive scalar + buoyancy (functional form); ``active``: optional int32 [B] mask."""
+    return PISOSubstepScalar.apply(u, p, bvel, T, sbval, solver, dt, beta, active)
 
 
-def piso_substep(solver: BatchedPISO, u, p, bvel, dt):
-    """Differentiable PISO substep (functional form: inputs are not modified)."""
-    return PISOSubstep.apply(u, p, bvel, solver, dt)
+def piso_substep(solver: BatchedPISO, u, p, bvel, dt, active=None):
+    """Differentiable PISO substep (functional form: inputs are not modified); ``active``: optional int32 [B] mask of the
+    environments that take the substep, the others pass through unchanged."""
+    return PISOSubstep.apply(u, p, bvel, solver, dt, active)
 
 
 # ---- D = 3 structured boxes (turbulent channel): fgb_ortho3_piso_substep_record / _backward ------------------------------------------
@@ -147,16 +168,17 @@ class PISOSubstep3D(torch.autograd.Function):
     ``torch.tensor``).  The previous pressure gets no gradient: every recorded solve starts from zero."""
 
     @staticmethod
-    def forward(ctx, u, p, bvel, solver, dt, src):
+    def forward(ctx, u, p, bvel, solver, dt, src, active=None):
         dtc = solver._dt(dt)
+        active = _mask(solver, active)
         tape = _new_tape3(solver)
-        ct = native.Ortho3Tape(*[tape[k].data_ptr() for k, _ in native.Ortho3Tape._fields_])
+        ct = _ctape(native.Ortho3Tape, tape, active)
         u_out, p_out = u.detach().clone().contiguous(), p.detach().clone().contiguous()
         bv = bvel.detach().contiguous()
         srcc = None if src is None else src.detach().contiguous()
         native.check(solver.lib.fgb_ortho3_piso_substep_record(solver.handle, _ptr(u_out), _ptr(p_out), _ptr(bv), _ptr(srcc), _ptr(dtc),
                                                                C.byref(ct), solver.stream), "fgb_ortho3_piso_substep_record")
-        ctx.solver, ctx.tape = solver, tape
+        ctx.solver, ctx.tape, ctx.active = solver, tape, active
         return u_out, p_out
 
     @staticmethod
@@ -164,19 +186,19 @@ class PISOSubstep3D(torch.autograd.Function):
         solver, tape = ctx.solver, ctx.tape
         B, N, NB = solver.B, solver.N, max(solver.NB, 1)
         f32 = dict(device=solver.device, dtype=torch.float32)
-        ct = native.Ortho3Tape(*[tape[k].data_ptr() for k, _ in native.Ortho3Tape._fields_])
+        ct = _ctape(native.Ortho3Tape, tape, ctx.active)
         ub, bvb = torch.empty(B, 3, N, **f32), torch.empty(B, 3, NB, **f32)
         ws, nbytes = _adjoint_workspace3(solver)
         uo = (u_out_bar if u_out_bar is not None else torch.zeros(B, 3, N, **f32)).contiguous()
         po = (p_out_bar if p_out_bar is not None else torch.zeros(B, N, **f32)).contiguous()
         native.check(solver.lib.fgb_ortho3_piso_substep_backward(solver.handle, C.byref(ct), _ptr(uo), _ptr(po), _ptr(ub), _ptr(bvb), ws, nbytes,
                                                                  solver.stream), "fgb_ortho3_piso_substep_backward")
-        return ub, None, bvb, None, None, None
+        return ub, None, bvb, None, None, None, None
 
 
-def piso_substep_3d(solver, u, p, bvel, dt, src=None):
-    """Differentiable substep of a structured 3-D box (functional form: inputs are not modified)."""
-    return PISOSubstep3D.apply(u, p, bvel, solver, dt, src)
+def piso_substep_3d(solver, u, p, bvel, dt, src=None, active=None):
+    """Differentiable substep of a structured 3-D box (functional form: inputs are not modified); ``active``: optional int32 [B] mask."""
+    return PISOSubstep3D.apply(u, p, bvel, solver, dt, src, active)
 
 
 class PISOSubstepScalar3D(torch.autograd.Function):
@@ -184,20 +206,21 @@ class PISOSubstepScalar3D(torch.autograd.Function):
     passive scalar + buoyancy (RBC3D; ``BatchedPISO3D.attach_scalar``).  The solver's own scalar buffers are used as scratch."""
 
     @staticmethod
-    def forward(ctx, u, p, bvel, T, sbval, solver, dt):
+    def forward(ctx, u, p, bvel, T, sbval, solver, dt, active=None):
         dtc = solver._dt(dt)
+        active = _mask(solver, active)
         tape = _new_tape3(solver)
         f32 = dict(device=solver.device, dtype=torch.float32)
         stape = dict(T_in=torch.empty(solver.B, solver.N, **f32), T_out=torch.empty(solver.B, solver.N, **f32),
                      sbval_in=torch.empty(solver.B, max(solver.NB, 1), **f32))
-        ct = native.Ortho3Tape(*[tape[k].data_ptr() for k, _ in native.Ortho3Tape._fields_])
+        ct = _ctape(native.Ortho3Tape, tape, active)
         cs = native.ScalarTape(*[stape[k].data_ptr() for k, _ in native.ScalarTape._fields_])
         u_out, p_out = u.detach().clone().contiguous(), p.detach().clone().contiguous()
         bv = bvel.detach().contiguous()
         solver.T.copy_(T.detach()); solver.sbval.copy_(sbval.detach())
         native.check(solver.lib.fgb_ortho3_piso_substep_record_scalar(solver.handle, _ptr(u_out), _ptr(p_out), _ptr(bv), None, _ptr(dtc), C.byref(ct),
                                                                       C.byref(cs), solver.stream), "fgb_ortho3_piso_substep_record_scalar")
-        ctx.solver, ctx.tape, ctx.stape = solver, tape, stape
+        ctx.solver, ctx.tape, ctx.stape, ctx.active = solver, tape, stape, active
         return u_out, p_out, solver.T.clone()
 
     @staticmethod
@@ -205,7 +228,7 @@ class PISOSubstepScalar3D(torch.autograd.Function):
         solver, tape, stape = ctx.solver, ctx.tape, ctx.stape
         B, N, NB = solver.B, solver.N, max(solver.NB, 1)
         f32 = dict(device=solver.device, dtype=torch.float32)
-        ct = native.Ortho3Tape(*[tape[k].data_ptr() for k, _ in native.Ortho3Tape._fields_])
+        ct = _ctape(native.Ortho3Tape, tape, ctx.active)
         cs = native.ScalarTape(*[stape[k].data_ptr() for k, _ in native.ScalarTape._fields_])
         ub, bvb, Tb, sbb = torch.empty(B, 3, N, **f32), torch.empty(B, 3, NB, **f32), torch.empty(B, N, **f32), torch.empty(B, NB, **f32)
         ws, nbytes = _adjoint_workspace3(solver)
@@ -215,12 +238,13 @@ class PISOSubstepScalar3D(torch.autograd.Function):
         native.check(solver.lib.fgb_ortho3_piso_substep_backward_scalar(solver.handle, C.byref(ct), C.byref(cs), _ptr(uo), _ptr(po), _ptr(To), _ptr(ub),
                                                                         _ptr(bvb), _ptr(Tb), _ptr(sbb), ws, nbytes, solver.stream),
                      "fgb_ortho3_piso_substep_backward_scalar")
-        return ub, None, bvb, Tb, sbb, None, None
+        return ub, None, bvb, Tb, sbb, None, None, None
 
 
-def piso_substep_scalar_3d(solver, u, p, bvel, T, sbval, dt):
-    """Differentiable substep of a structured 3-D box with passive scalar + buoyancy (functional form)."""
-    return PISOSubstepScalar3D.apply(u, p, bvel, T, sbval, solver, dt)
+def piso_substep_scalar_3d(solver, u, p, bvel, T, sbval, dt, active=None):
+    """Differentiable substep of a structured 3-D box with passive scalar + buoyancy (functional form); ``active``: optional int32 [B]
+    mask."""
+    return PISOSubstepScalar3D.apply(u, p, bvel, T, sbval, solver, dt, active)
 
 
 # ---- z-extruded multi-block grids (CylinderJet3D / Airfoil3D): fgb_extruded3_piso_substep_record / _backward -----------------------------
@@ -228,8 +252,9 @@ class PISOSubstepExtruded(torch.autograd.Function):
     """(u [B,3,N3], p [B,N3], bvel [B,3,nz,NB2]) -> (u_next, p_next) for one substep of an ``ExtrudedPISO3D`` solver"""
 
     @staticmethod
-    def forward(ctx, u, p, bvel, solver, dt):
+    def forward(ctx, u, p, bvel, solver, dt, active=None):
         B, N3, nz, NB = solver.B, solver.N, solver.nz, max(solver.NB2, 1)
+        active = _mask(solver, active)
         f32 = dict(device=solver.device, dtype=torch.float32)
         o = solver.options
         C_, n_adv, n_p = int(o.corrector_steps), int(o.adv_nonortho_steps), int(o.p_nonortho_steps)
@@ -237,13 +262,13 @@ class PISOSubstepExtruded(torch.autograd.Function):
                     dt=torch.empty(B, **f32), Coff=torch.empty(B, 6, N3, **f32), A=torch.empty(B, N3, **f32),
                     ustar=torch.empty(n_adv, B, 3, N3, **f32), hb=torch.empty(C_, B, 3, N3, **f32), p=torch.empty(C_ * n_p, B, N3, **f32),
                     pmean=torch.empty(C_ * n_p, B, **f32), u1=torch.empty(max(C_ - 1, 1), B, 3, N3, **f32))
-        ct = native.Tape(*[tape[k].data_ptr() for k, _ in native.Tape._fields_])
+        ct = _ctape(native.Tape, tape, active)
         dtc = dt.to(solver.device, torch.float32).contiguous() if isinstance(dt, torch.Tensor) else torch.full((B,), float(dt), **f32)
         u_out, p_out = u.detach().clone().contiguous(), p.detach().clone().contiguous()
         bv = bvel.detach().contiguous()
         native.check(solver.lib.fgb_extruded3_piso_substep_record(solver.handle, C.byref(solver.xtables), _ptr(u_out), _ptr(p_out), _ptr(bv), _ptr(dtc),
                                                                   C.byref(ct), solver.stream), "fgb_extruded3_piso_substep_record")
-        ctx.solver, ctx.tape = solver, tape
+        ctx.solver, ctx.tape, ctx.active = solver, tape, active
         return u_out, p_out
 
     @staticmethod
@@ -251,7 +276,7 @@ class PISOSubstepExtruded(torch.autograd.Function):
         solver, tape = ctx.solver, ctx.tape
         B, N3, nz, NB = solver.B, solver.N, solver.nz, max(solver.NB2, 1)
         f32 = dict(device=solver.device, dtype=torch.float32)
-        ct = native.Tape(*[tape[k].data_ptr() for k, _ in native.Tape._fields_])
+        ct = _ctape(native.Tape, tape, ctx.active)
         ub, pb, bvb = torch.empty(B, 3, N3, **f32), torch.empty(B, N3, **f32), torch.empty(B, 3, nz, NB, **f32)
         nbytes = solver.lib.fgb_extruded3_adjoint_workspace_bytes(C.byref(solver.xtables), B)
         ws = getattr(solver, "_adj_ws", None)
@@ -262,9 +287,9 @@ class PISOSubstepExtruded(torch.autograd.Function):
         po = (p_out_bar if p_out_bar is not None else torch.zeros(B, N3, **f32)).contiguous()
         native.check(solver.lib.fgb_extruded3_piso_substep_backward(solver.handle, C.byref(solver.xtables), C.byref(ct), _ptr(uo), _ptr(po), _ptr(ub),
                                                                     _ptr(pb), _ptr(bvb), wsp, nbytes, solver.stream), "fgb_extruded3_piso_substep_backward")
-        return ub, pb, bvb, None, None
+        return ub, pb, bvb, None, None, None
 
 
-def piso_substep_extruded(solver, u, p, bvel, dt):
-    """Differentiable substep of a z-extruded multi-block grid (functional form)."""
-    return PISOSubstepExtruded.apply(u, p, bvel, solver, dt)
+def piso_substep_extruded(solver, u, p, bvel, dt, active=None):
+    """Differentiable substep of a z-extruded multi-block grid (functional form); ``active``: optional int32 [B] mask."""
+    return PISOSubstepExtruded.apply(u, p, bvel, solver, dt, active)

@@ -215,35 +215,35 @@ X3_HD void x3_correct_cell(const X3Tab &x, int k, int g, const float *hb, const 
 // run the Krylov iterations.
 // ------------------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) kx3_setup_advection(X3Tab x, const float *U, const float *Ures, const float *Bvel, const float *dtv,
-                                                          float *Coff, float *A, float *Rhs, int with_matrix) {
+                                                          float *Coff, float *A, float *Rhs, int with_matrix, const int32_t *active) {
     const int b = blockIdx.z, k = blockIdx.y, g = blockIdx.x * blockDim.x + threadIdx.x;
-    if (g >= x.t.N) return;
+    if (g >= x.t.N || (active && !active[b])) return;
     const size_t N3 = (size_t)x.t.N * x.nz;
     x3_setup_advection_cell(x, k, g, U + b * 3 * N3, Ures + b * 3 * N3, Bvel + (size_t)b * 3 * x.nz * x.t.NB, dtv[b], Coff + b * 6 * N3,
                             A + b * N3, Rhs + b * 3 * N3, with_matrix);
 }
-__global__ void __launch_bounds__(256) kx3_pressure_matrix(X3Tab x, const float *A, float *Poff, float *Pdiag) {
+__global__ void __launch_bounds__(256) kx3_pressure_matrix(X3Tab x, const float *A, float *Poff, float *Pdiag, const int32_t *active) {
     const int b = blockIdx.z, k = blockIdx.y, g = blockIdx.x * blockDim.x + threadIdx.x;
-    if (g >= x.t.N) return;
+    if (g >= x.t.N || (active && !active[b])) return;
     const size_t N3 = (size_t)x.t.N * x.nz;
     x3_pressure_matrix_cell(x, k, g, A + b * N3, Poff + b * 6 * N3, Pdiag + b * N3);
 }
 __global__ void __launch_bounds__(256) kx3_hbya(X3Tab x, const float *U, const float *Ures, const float *Bvel, const float *Coff, const float *A,
-                                               const float *dtv, float *Hb) {
+                                               const float *dtv, float *Hb, const int32_t *active) {
     const int b = blockIdx.z, k = blockIdx.y, g = blockIdx.x * blockDim.x + threadIdx.x;
-    if (g >= x.t.N) return;
+    if (g >= x.t.N || (active && !active[b])) return;
     const size_t N3 = (size_t)x.t.N * x.nz;
     x3_hbya_cell(x, k, g, U + b * 3 * N3, Ures + b * 3 * N3, Bvel + (size_t)b * 3 * x.nz * x.t.NB, Coff + b * 6 * N3, A + b * N3, dtv[b], Hb + b * 3 * N3);
 }
-__global__ void __launch_bounds__(256) kx3_divergence(X3Tab x, const float *Hb, const float *Bvel, const float *Pprev, const float *A, float *Div) {
+__global__ void __launch_bounds__(256) kx3_divergence(X3Tab x, const float *Hb, const float *Bvel, const float *Pprev, const float *A, float *Div, const int32_t *active) {
     const int b = blockIdx.z, k = blockIdx.y, g = blockIdx.x * blockDim.x + threadIdx.x;
-    if (g >= x.t.N) return;
+    if (g >= x.t.N || (active && !active[b])) return;
     const size_t N3 = (size_t)x.t.N * x.nz;
     x3_divergence_cell(x, k, g, Hb + b * 3 * N3, Bvel + (size_t)b * 3 * x.nz * x.t.NB, Pprev ? Pprev + b * N3 : nullptr, A + b * N3, Div + b * N3);
 }
-__global__ void __launch_bounds__(256) kx3_correct(X3Tab x, const float *Hb, const float *P, const float *A, float *Uout) {
+__global__ void __launch_bounds__(256) kx3_correct(X3Tab x, const float *Hb, const float *P, const float *A, float *Uout, const int32_t *active) {
     const int b = blockIdx.z, k = blockIdx.y, g = blockIdx.x * blockDim.x + threadIdx.x;
-    if (g >= x.t.N) return;
+    if (g >= x.t.N || (active && !active[b])) return;
     const size_t N3 = (size_t)x.t.N * x.nz;
     x3_correct_cell(x, k, g, Hb + b * 3 * N3, P + b * N3, A + b * N3, Uout + b * 3 * N3);
 }
@@ -261,23 +261,23 @@ extern "C" int fgb_extruded3_piso_substep(fgb_ortho3 *b, const fgb_extruded3_tab
     int rc;
     for (int ns = 0; ns < o.adv_nonortho_steps; ++ns) {
         b->launches++;
-        kx3_setup_advection<<<grid, 256, 0, st>>>(x, u, ns == 0 ? u : b->ures, bvel, dt, b->Coff, b->A, b->rhs, ns == 0);
+        kx3_setup_advection<<<grid, 256, 0, st>>>(x, u, ns == 0 ? u : b->ures, bvel, dt, b->Coff, b->A, b->rhs, ns == 0, nullptr);
         LAUNCH_CHECK("kx3_setup_advection");
         if ((rc = fgb_ortho3_solve_advection(b, ns == 0, nullptr, s))) return rc;
     }
     for (int cs = 0; cs < o.corrector_steps; ++cs) {
         b->launches += 2;
-        if (cs == 0) { kx3_pressure_matrix<<<grid, 256, 0, st>>>(x, b->A, b->Poff, b->Pdiag); LAUNCH_CHECK("kx3_pressure_matrix"); }
-        kx3_hbya<<<grid, 256, 0, st>>>(x, u, b->ures, bvel, b->Coff, b->A, dt, b->hbya);
+        if (cs == 0) { kx3_pressure_matrix<<<grid, 256, 0, st>>>(x, b->A, b->Poff, b->Pdiag, nullptr); LAUNCH_CHECK("kx3_pressure_matrix"); }
+        kx3_hbya<<<grid, 256, 0, st>>>(x, u, b->ures, bvel, b->Coff, b->A, dt, b->hbya, nullptr);
         LAUNCH_CHECK("kx3_hbya");
         for (int ps = 0; ps < o.p_nonortho_steps; ++ps) {
             b->launches++;
-            kx3_divergence<<<grid, 256, 0, st>>>(x, b->hbya, bvel, p, b->A, b->div);
+            kx3_divergence<<<grid, 256, 0, st>>>(x, b->hbya, bvel, p, b->A, b->div, nullptr);
             LAUNCH_CHECK("kx3_divergence");
             if ((rc = fgb_ortho3_solve_pressure(b, p, ps == 0, 100, o.max_iter, cs * o.p_nonortho_steps + ps, nullptr, s))) return rc;
         }
         b->launches++;
-        kx3_correct<<<grid, 256, 0, st>>>(x, b->hbya, p, b->A, b->ures);
+        kx3_correct<<<grid, 256, 0, st>>>(x, b->hbya, p, b->A, b->ures, nullptr);
         LAUNCH_CHECK("kx3_correct");
     }
     cudaError_t ce = cudaMemcpyAsync(u, b->ures, (size_t)b->B * 3 * b->t.N * sizeof(float), cudaMemcpyDeviceToDevice, st);
@@ -319,13 +319,14 @@ __device__ __forceinline__ void x3_fluxes_adjoint(const fgb_tables &t, int g, co
     const int b = blockIdx.z, k = blockIdx.y, g = blockIdx.x * blockDim.x + threadIdx.x; \
     const fgb_tables &t = x.t; \
     const int N = t.N, nz = x.nz; \
-    if (g >= N) return; \
+    if (g >= N || (active && !active[b])) return;    /* skipped environment: identity cotangents from k_adj_inactive */ \
     const size_t N3 = (size_t)N * nz, g3 = (size_t)k * N + g; \
     const int kl = (k + nz - 1) % nz, ku = (k + 1) % nz; \
     (void)kl; (void)ku; (void)N3; (void)g3;
 
 __global__ void __launch_bounds__(256) kx3_adj_correct(X3Tab x, const float *__restrict__ Unb, const float *__restrict__ P, const float *__restrict__ A,
-                                                       float *__restrict__ Hbb, float *__restrict__ rAb, float *__restrict__ Pb) {
+                                                       float *__restrict__ Hbb, float *__restrict__ rAb, float *__restrict__ Pb,
+                                                       const int32_t *__restrict__ active) {
     X3_ADJ_PROLOGUE
     const float *p = P + b * N3, *pk = p + (size_t)k * N;
     float *pb = Pb + b * N3, *pbk = pb + (size_t)k * N;
@@ -358,7 +359,8 @@ __global__ void __launch_bounds__(256) kx3_adj_correct(X3Tab x, const float *__r
 // adjoint of  div = hz (fluxdiv2(hb) + NOp(p_prev, rA)) + det2 D_z(hb_z)  and of  x = P^-1 div  w.r.t. P(rA):  given lam = P^-T x_bar
 __global__ void __launch_bounds__(256) kx3_adj_pressure_rhs(X3Tab x, const float *__restrict__ Lam, const float *__restrict__ Pm, const float *__restrict__ Pmean,
                                                             const float *__restrict__ Pprev, const float *__restrict__ A, float *__restrict__ Hbb,
-                                                            float *__restrict__ Fbb, float *__restrict__ rAb, float *__restrict__ Pprevb) {
+                                                            float *__restrict__ Fbb, float *__restrict__ rAb, float *__restrict__ Pprevb,
+                                                            const int32_t *__restrict__ active) {
     X3_ADJ_PROLOGUE
     const int NB = t.NB;
     const float hz = x.hz, lam = Lam[b * N3 + g3], mean = Pmean[b];
@@ -409,7 +411,7 @@ __global__ void __launch_bounds__(256) kx3_adj_pressure_rhs(X3Tab x, const float
 __global__ void __launch_bounds__(256) kx3_adj_hbya(X3Tab x, const float *__restrict__ Hbb, const float *__restrict__ Hb, const float *__restrict__ A,
                                                     const float *__restrict__ Coff, const float *__restrict__ Uprev, const float *__restrict__ dtv,
                                                     float *__restrict__ rAb, float *__restrict__ Ub, float *__restrict__ Sbb, float *__restrict__ Coffb,
-                                                    float *__restrict__ Uprevb) {
+                                                    float *__restrict__ Uprevb, const int32_t *__restrict__ active) {
     X3_ADJ_PROLOGUE
     const float dt = dtv[b], Ag = A[b * N3 + g3], rA = 1.0f / Ag, det = t.det[g];
     const float *coff = Coff + b * 6 * N3;
@@ -443,7 +445,7 @@ __global__ void __launch_bounds__(256) kx3_adj_hbya(X3Tab x, const float *__rest
 __global__ void __launch_bounds__(256) kx3_adj_advection(X3Tab x, const float *__restrict__ Mu, const float *__restrict__ X, const float *__restrict__ rAb,
                                                          const float *__restrict__ A, const float *__restrict__ dtv, float *__restrict__ Ab,
                                                          float *__restrict__ Coffb, float *__restrict__ Ub, float *__restrict__ Sbb, float *__restrict__ Bvb,
-                                                         float *__restrict__ NoTarget, int first) {
+                                                         float *__restrict__ NoTarget, int first, const int32_t *__restrict__ active) {
     X3_ADJ_PROLOGUE
     const int NB = t.NB;
     const float dt = dtv[b], det = t.det[g], Ag = A[b * N3 + g3];
@@ -474,7 +476,8 @@ __global__ void __launch_bounds__(256) kx3_adj_advection(X3Tab x, const float *_
 }
 // adjoint of the assembly (A, Coff from the in-plane face fluxes and the z fluxes) and of the boundary sources
 __global__ void __launch_bounds__(256) kx3_adj_assemble(X3Tab x, const float *__restrict__ Ab, const float *__restrict__ Coffb, const float *__restrict__ Sbb,
-                                                        const float *__restrict__ Bvel, float *__restrict__ Ub, float *__restrict__ Bvb, float *__restrict__ Fbb) {
+                                                        const float *__restrict__ Bvel, float *__restrict__ Ub, float *__restrict__ Bvb, float *__restrict__ Fbb,
+                                                        const int32_t *__restrict__ active) {
     X3_ADJ_PROLOGUE
     const int NB = t.NB;
     const float det = t.det[g], ab = Ab[b * N3 + g3], diagb = ab / det, hz = x.hz;
@@ -510,11 +513,11 @@ __global__ void __launch_bounds__(256) kx3_adj_assemble(X3Tab x, const float *__
     atomicAdd(&ub[2 * N3 + (size_t)ku * N + g], 0.5f * fzp);
 }
 // adjoint of the in-plane boundary flux Fb(bx, by): one thread per (boundary face, plane, environment)
-__global__ void kx3_adj_bflux(X3Tab x, const float *__restrict__ Fbb, float *__restrict__ Bvb) {
+__global__ void kx3_adj_bflux(X3Tab x, const float *__restrict__ Fbb, float *__restrict__ Bvb, const int32_t *__restrict__ active) {
     const int b = blockIdx.z, k = blockIdx.y, j = blockIdx.x * blockDim.x + threadIdx.x;
     const fgb_tables &t = x.t;
     const int NB = t.NB, nz = x.nz;
-    if (j >= NB) return;
+    if (j >= NB || (active && !active[b])) return;
     const int ax = t.b_face[j] >> 1;
     const float f = Fbb[((size_t)b * nz + k) * NB + j] * t.b_det[j];
     Bvb[((size_t)b * 3 + 0) * nz * NB + (size_t)k * NB + j] += f * t.b_minv[(2 * ax) * NB + j];
@@ -529,7 +532,8 @@ static int x3_copy(void *dst, const void *src, size_t bytes, cudaStream_t st) {
     cudaError_t ce = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, st);
     return ce == cudaSuccess ? FGB_OK : set_err(FGB_E_CUDA, "cudaMemcpyAsync (extruded tape)", ce);
 }
-// fgb_extruded3_piso_substep that additionally records the tape of the backward pass (zero-started solves, no CG residual reset)
+// fgb_extruded3_piso_substep that additionally records the tape of the backward pass (zero-started solves, no CG residual reset), for the
+// environments of tp->active (NULL: all); a skipped environment keeps u and p bit for bit
 extern "C" int fgb_extruded3_piso_substep_record(fgb_ortho3 *b, const fgb_extruded3_tables *xt, float *u, float *p, const float *bvel, const float *dt,
                                                  const fgb_tape *tp, fgb_stream_t s) {
     if (!b || !xt || !u || !p || !bvel || !dt || !tp) return set_err(FGB_E_ARG, "fgb_extruded3_piso_substep_record: null argument");
@@ -541,6 +545,7 @@ extern "C" int fgb_extruded3_piso_substep_record(fgb_ortho3 *b, const fgb_extrud
     cudaStream_t st = STREAM(s);
     const dim3 grid((unsigned)((x.t.N + 255) / 256), (unsigned)x.nz, (unsigned)b->B);
     const size_t B = b->B, BN = B * b->t.N, BNB = B * (size_t)x.nz * (x.t.NB > 0 ? x.t.NB : 1);
+    const int32_t *act = tp->active;
     int rc;
     if ((rc = x3_copy(tp->u_in, u, 3 * BN * 4, st))) return rc;
     if ((rc = x3_copy(tp->p_in, p, BN * 4, st))) return rc;
@@ -548,43 +553,44 @@ extern "C" int fgb_extruded3_piso_substep_record(fgb_ortho3 *b, const fgb_extrud
     if ((rc = x3_copy(tp->dt, dt, B * 4, st))) return rc;
     for (int ns = 0; ns < n_adv; ++ns) {
         b->launches++;
-        kx3_setup_advection<<<grid, 256, 0, st>>>(x, u, ns == 0 ? u : b->ures, bvel, dt, b->Coff, b->A, b->rhs, ns == 0);
+        kx3_setup_advection<<<grid, 256, 0, st>>>(x, u, ns == 0 ? u : b->ures, bvel, dt, b->Coff, b->A, b->rhs, ns == 0, act);
         LAUNCH_CHECK("kx3_setup_advection");
-        if ((rc = fgb_ortho3_solve_advection(b, 1, nullptr, s))) return rc;
+        if ((rc = fgb_ortho3_solve_advection(b, 1, act, s))) return rc;
         if ((rc = x3_copy(tp->ustar + (size_t)ns * 3 * BN, b->ures, 3 * BN * 4, st))) return rc;
     }
     if ((rc = x3_copy(tp->Coff, b->Coff, 6 * BN * 4, st))) return rc;
     if ((rc = x3_copy(tp->A, b->A, BN * 4, st))) return rc;
     b->launches++;
-    kx3_pressure_matrix<<<grid, 256, 0, st>>>(x, b->A, b->Poff, b->Pdiag);
+    kx3_pressure_matrix<<<grid, 256, 0, st>>>(x, b->A, b->Poff, b->Pdiag, act);
     LAUNCH_CHECK("kx3_pressure_matrix");
     for (int cs = 0; cs < C; ++cs) {
         b->launches++;
-        kx3_hbya<<<grid, 256, 0, st>>>(x, u, b->ures, bvel, b->Coff, b->A, dt, b->hbya);
+        kx3_hbya<<<grid, 256, 0, st>>>(x, u, b->ures, bvel, b->Coff, b->A, dt, b->hbya, act);
         LAUNCH_CHECK("kx3_hbya");
         for (int ps = 0; ps < n_p; ++ps) {
             const int q = cs * n_p + ps, slot = q > 4 ? 4 : q;
             b->launches += 2;
-            kx3_divergence<<<grid, 256, 0, st>>>(x, b->hbya, bvel, p, b->A, b->div);
+            kx3_divergence<<<grid, 256, 0, st>>>(x, b->hbya, bvel, p, b->A, b->div, act);
             LAUNCH_CHECK("kx3_divergence");
-            if ((rc = fgb_ortho3_solve_pressure(b, p, 1, 0, o.max_iter, slot, nullptr, s))) return rc;
+            if ((rc = fgb_ortho3_solve_pressure(b, p, 1, 0, o.max_iter, slot, act, s))) return rc;
             if ((rc = x3_copy(tp->p + (size_t)q * BN, p, BN * 4, st))) return rc;
             kx3_take_mean<<<(unsigned)((B + 127) / 128), 128, 0, st>>>((int)B, b->pmean, slot, tp->pmean + (size_t)q * B);
             LAUNCH_CHECK("kx3_take_mean");
         }
         if ((rc = x3_copy(tp->hb + (size_t)cs * 3 * BN, b->hbya, 3 * BN * 4, st))) return rc;
         b->launches++;
-        kx3_correct<<<grid, 256, 0, st>>>(x, b->hbya, p, b->A, b->ures);
+        kx3_correct<<<grid, 256, 0, st>>>(x, b->hbya, p, b->A, b->ures, act);
         LAUNCH_CHECK("kx3_correct");
         if (cs + 1 < C && (rc = x3_copy(tp->u1 + (size_t)cs * 3 * BN, b->ures, 3 * BN * 4, st))) return rc;
     }
-    return x3_copy(u, b->ures, 3 * BN * 4, st);
+    return o3_copy_active(b, u, b->ures, 3 * BN, act, st);
 }
 extern "C" size_t fgb_extruded3_adjoint_workspace_bytes(const fgb_extruded3_tables *xt, int32_t B) {
     const size_t BN = (size_t)B * xt->plane.N * xt->nz, BNB = (size_t)B * xt->nz * (xt->plane.NB > 0 ? xt->plane.NB : 1);
     return (size_t)(3 + 3 + 1 + 6 + 3 + 1 + 1 + 1 + 3 + 1 + 3 + 1 + 3) * align_up(BN * 4) + align_up(BNB * 4) + 8192;
 }
-// (u_out_bar, p_out_bar) -> (u_bar, p_prev_bar, bvel_bar), all overwritten
+// (u_out_bar, p_out_bar) -> (u_bar, p_prev_bar, bvel_bar), all overwritten; environments tp->active skips are skipped by every adjoint
+// kernel and transposed solve and get the identity cotangents (k_adj_inactive)
 extern "C" int fgb_extruded3_piso_substep_backward(fgb_ortho3 *b, const fgb_extruded3_tables *xt, const fgb_tape *tp, const float *u_out_bar,
                                                    const float *p_out_bar, float *u_bar, float *p_prev_bar, float *bvel_bar, void *ws, size_t ws_bytes,
                                                    fgb_stream_t s) {
@@ -600,6 +606,7 @@ extern "C" int fgb_extruded3_piso_substep_backward(fgb_ortho3 *b, const fgb_extr
     cudaStream_t st = STREAM(s);
     const dim3 grid((unsigned)((x.t.N + 255) / 256), (unsigned)x.nz, (unsigned)b->B);
     const size_t B = b->B, NBz = (size_t)x.nz * (x.t.NB > 0 ? x.t.NB : 1), BN = B * b->t.N;
+    const int32_t *act = tp->active;
     Carver c{(char *)ws, 0};
     float *unb = c.take<float>(3 * BN), *hbb = c.take<float>(3 * BN), *rAb = c.take<float>(BN), *Coffb = c.take<float>(6 * BN);
     float *Sbb = c.take<float>(3 * BN), *pb = c.take<float>(BN), *xb = c.take<float>(BN), *lam = c.take<float>(BN);
@@ -612,36 +619,36 @@ extern "C" int fgb_extruded3_piso_substep_backward(fgb_ortho3 *b, const fgb_extr
     if ((rc = x3_copy(unb, u_out_bar, 3 * BN * 4, st))) return rc;
     if ((rc = x3_copy(pb, p_out_bar, BN * 4, st))) return rc;
     b->launches++;
-    kx3_pressure_matrix<<<grid, 256, 0, st>>>(x, tp->A, b->Poff, b->Pdiag);
+    kx3_pressure_matrix<<<grid, 256, 0, st>>>(x, tp->A, b->Poff, b->Pdiag, act);
     LAUNCH_CHECK("kx3_pressure_matrix (backward)");
     for (int cs = C - 1; cs >= 0; --cs) {
         const float *hb_c = tp->hb + (size_t)cs * 3 * BN;
         const float *uprev = cs == 0 ? tp->ustar + (size_t)(n_adv - 1) * 3 * BN : tp->u1 + (size_t)(cs - 1) * 3 * BN;
         b->launches++;
-        kx3_adj_correct<<<grid, 256, 0, st>>>(x, unb, tp->p + (size_t)(cs * n_p + n_p - 1) * BN, tp->A, hbb, rAb, pb);
+        kx3_adj_correct<<<grid, 256, 0, st>>>(x, unb, tp->p + (size_t)(cs * n_p + n_p - 1) * BN, tp->A, hbb, rAb, pb, act);
         LAUNCH_CHECK("kx3_adj_correct");
         for (int ps = n_p - 1; ps >= 0; --ps) {
             const int q = cs * n_p + ps;
             const float *pprev = q == 0 ? tp->p_in : tp->p + (size_t)(q - 1) * BN;
             b->launches += 3;
-            k3_adj_remove_mean<<<b->B, 1024, 0, st>>>(b->t.N, b->t.N, pb, xb);
+            k3_adj_remove_mean<<<b->B, 1024, 0, st>>>(b->t.N, b->t.N, pb, xb, act);
             LAUNCH_CHECK("k3_adj_remove_mean");
             {   // lam = P^-T x_bar: the forward CG kernel on the transposed operator, zero start, no residual reset
                 T3 t = b->t; O3Slab sl = b->slab; int Bi = b->B; const float *poff = b->Poff, *pd = b->Pdiag, *rhs = xb; float *work = b->kry, *part = b->part;
-                float tol = b->opt.p_tol; int max_iter = b->opt.max_iter, zero_init = 1, reset_steps = 0, slot = 4; const int32_t *active = nullptr;
+                float tol = b->opt.p_tol; int max_iter = b->opt.max_iter, zero_init = 1, reset_steps = 0, slot = 4; const int32_t *active = act;
                 int32_t *iters = b->iters; float *resid = b->resid; unsigned long long *itot = b->iter_total; float *out = lam, *pmean = b->pmean;
                 void *args[] = {&t, &sl, &Bi, &poff, &pd, &rhs, &out, &work, &part, &max_iter, &tol, &zero_init, &reset_steps, &slot, &active, &iters, &resid, &itot, &pmean};
                 ce = cudaLaunchCooperativeKernel((void *)k3_cg<1>, dim3(o3_coop_blocks(b)), dim3(O3_CT), args, 0, st);
                 if (ce != cudaSuccess) return set_err(FGB_E_CUDA, "cudaLaunchCooperativeKernel(k3_cg<1>, backward)", ce);
             }
             ZEROX(pb2, BN);                 // becomes the gradient w.r.t. pprev
-            kx3_adj_pressure_rhs<<<grid, 256, 0, st>>>(x, lam, tp->p + (size_t)q * BN, tp->pmean + (size_t)q * B, pprev, tp->A, hbb, Fbb, rAb, pb2);
+            kx3_adj_pressure_rhs<<<grid, 256, 0, st>>>(x, lam, tp->p + (size_t)q * BN, tp->pmean + (size_t)q * B, pprev, tp->A, hbb, Fbb, rAb, pb2, act);
             LAUNCH_CHECK("kx3_adj_pressure_rhs");
             float *tmp = pb; pb = pb2; pb2 = tmp;      // the previous iterate enters only through the deferred term
         }
         ZEROX(uprevb, 3 * BN);
         b->launches++;
-        kx3_adj_hbya<<<grid, 256, 0, st>>>(x, hbb, hb_c, tp->A, tp->Coff, uprev, tp->dt, rAb, u_bar, Sbb, Coffb, uprevb);
+        kx3_adj_hbya<<<grid, 256, 0, st>>>(x, hbb, hb_c, tp->A, tp->Coff, uprev, tp->dt, rAb, u_bar, Sbb, Coffb, uprevb, act);
         LAUNCH_CHECK("kx3_adj_hbya");
         float *tmp = unb; unb = uprevb; uprevb = tmp;   // gradient w.r.t. the velocity entering this corrector
     }
@@ -650,7 +657,7 @@ extern "C" int fgb_extruded3_piso_substep_backward(fgb_ortho3 *b, const fgb_extr
     for (int k = n_adv - 1; k >= 0; --k) {
         {   // mu = C^-T x_k_bar
             T3 t = b->t; O3Slab sl = b->slab; int Bi = b->B; const float *coff = tp->Coff, *a = tp->A, *rhs = xb_cur; float *xo = mu, *work = b->kry, *part = b->part;
-            int maxit = b->opt.max_iter, zero_init = 1, transposed = 1; float tol = b->opt.adv_tol; const int32_t *active = nullptr;
+            int maxit = b->opt.max_iter, zero_init = 1, transposed = 1; float tol = b->opt.adv_tol; const int32_t *active = act;
             int32_t *iters = b->iters; float *resid = b->resid; unsigned long long *itot = b->iter_total;
             void *args[] = {&t, &sl, &Bi, &coff, &a, &rhs, &xo, &work, &part, &maxit, &tol, &zero_init, &active, &iters, &resid, &itot, &transposed};
             b->launches++;
@@ -660,19 +667,20 @@ extern "C" int fgb_extruded3_piso_substep_backward(fgb_ortho3 *b, const fgb_extr
         if (k > 0) ZEROX(xb_prev, 3 * BN);
         b->launches++;
         kx3_adj_advection<<<grid, 256, 0, st>>>(x, mu, tp->ustar + (size_t)k * 3 * BN, rAb, tp->A, tp->dt, Ab, Coffb, u_bar, Sbb, bvel_bar,
-                                                k > 0 ? xb_prev : u_bar, k == n_adv - 1);
+                                                k > 0 ? xb_prev : u_bar, k == n_adv - 1, act);
         LAUNCH_CHECK("kx3_adj_advection");
         float *tmp = xb_cur; xb_cur = xb_prev; xb_prev = tmp;
     }
     b->launches += 2;
-    kx3_adj_assemble<<<grid, 256, 0, st>>>(x, Ab, Coffb, Sbb, tp->bvel_in, u_bar, bvel_bar, Fbb);
+    kx3_adj_assemble<<<grid, 256, 0, st>>>(x, Ab, Coffb, Sbb, tp->bvel_in, u_bar, bvel_bar, Fbb, act);
     LAUNCH_CHECK("kx3_adj_assemble");
     if (x.t.NB > 0) {
-        kx3_adj_bflux<<<dim3((unsigned)((x.t.NB + 127) / 128), (unsigned)x.nz, (unsigned)b->B), 128, 0, st>>>(x, Fbb, bvel_bar);
+        kx3_adj_bflux<<<dim3((unsigned)((x.t.NB + 127) / 128), (unsigned)x.nz, (unsigned)b->B), 128, 0, st>>>(x, Fbb, bvel_bar, act);
         LAUNCH_CHECK("kx3_adj_bflux");
     }
 #undef ZEROX
-    return FGB_OK;
+    if (act) b->launches++;
+    return launch_adj_inactive(act, b->B, 3, b->t.N, u_out_bar, u_bar, p_out_bar, p_prev_bar, nullptr, nullptr, (int)(3 * NBz), bvel_bar, 0, nullptr, st);
 }
 
 // Simulation.make_divergence_free on an extruded domain (SIM.py:1320-1430): A = 1, the velocity itself is the pressure right-hand
@@ -691,16 +699,16 @@ extern "C" int fgb_extruded3_make_divergence_free(fgb_ortho3 *b, const fgb_extru
     b->launches += 2;
     k_fill<<<(unsigned)((BN + 255) / 256), 256, 0, st>>>(b->A, 1.0f, BN);
     LAUNCH_CHECK("k_fill");
-    kx3_pressure_matrix<<<grid, 256, 0, st>>>(x, b->A, b->Poff, b->Pdiag);
+    kx3_pressure_matrix<<<grid, 256, 0, st>>>(x, b->A, b->Poff, b->Pdiag, nullptr);
     LAUNCH_CHECK("kx3_pressure_matrix");
     for (int ps = 0; ps < b->opt.p_nonortho_steps; ++ps) {
         b->launches++;
-        kx3_divergence<<<grid, 256, 0, st>>>(x, u, bvel, p, b->A, b->div);
+        kx3_divergence<<<grid, 256, 0, st>>>(x, u, bvel, p, b->A, b->div, nullptr);
         LAUNCH_CHECK("kx3_divergence");
         if ((rc = fgb_ortho3_solve_pressure(b, p, ps == 0, 0 /* no residual reset here, SIM.py:1387-1396 */, max_iter > 0 ? max_iter : b->opt.max_iter, ps, nullptr, s))) return rc;
     }
     b->launches++;
-    kx3_correct<<<grid, 256, 0, st>>>(x, u, p, b->A, b->ures);
+    kx3_correct<<<grid, 256, 0, st>>>(x, u, p, b->A, b->ures, nullptr);
     LAUNCH_CHECK("kx3_correct");
     cudaError_t ce = cudaMemcpyAsync(u, b->ures, 3 * BN * sizeof(float), cudaMemcpyDeviceToDevice, st);
     if (ce != cudaSuccess) return set_err(FGB_E_CUDA, "fgb_extruded3_make_divergence_free: copy", ce);

@@ -1231,9 +1231,9 @@ __device__ __forceinline__ void o3_fluxes_adjoint(const T3 &t, int g, const int 
 }
 // adjoint of the corrector u_next = hb - rA * minv_d * dp_d:  hbb = unb ; rAb -= sum_d dp_d minv_d unb_d ; pb += D^T(-rA minv_d unb_d)
 __global__ void __launch_bounds__(O3_T) k3_adj_correct(T3 t, const float *__restrict__ Unb, const float *__restrict__ P, const float *__restrict__ A,
-                                                       float *__restrict__ Hbb, float *__restrict__ rAb, float *__restrict__ Pb) {
+                                                       float *__restrict__ Hbb, float *__restrict__ rAb, float *__restrict__ Pb, const int32_t *__restrict__ active) {
     const int b = blockIdx.y, g = blockIdx.x * blockDim.x + threadIdx.x, NS = t.NS;
-    if (g >= t.N) return;
+    if (g >= t.N || (active && !active[b])) return;
     const float *p = P + (size_t)b * NS;
     float *pb = Pb + (size_t)b * NS;
     const float pc = p[g], rA = 1.0f / A[(size_t)b * NS + g];
@@ -1255,9 +1255,10 @@ __global__ void __launch_bounds__(O3_T) k3_adj_correct(T3 t, const float *__rest
     atomicAdd(&rAb[(size_t)b * NS + g], accr);
 }
 // x_bar = p_bar - mean(p_bar)   (adjoint of the mean removal), one CTA per environment
-__global__ void __launch_bounds__(1024) k3_adj_remove_mean(int N, int NS, const float *__restrict__ Pb, float *__restrict__ Xb) {
+__global__ void __launch_bounds__(1024) k3_adj_remove_mean(int N, int NS, const float *__restrict__ Pb, float *__restrict__ Xb, const int32_t *__restrict__ active) {
     __shared__ double red[32 * 2 + 2];
     const int b = blockIdx.x;
+    if (active && !active[b]) return;
     float acc[2] = {0.f, 0.f};
     for (int g = threadIdx.x; g < N; g += 1024) acc[0] += Pb[(size_t)b * NS + g];
     block_reduce_sum<2>(acc, red);
@@ -1267,9 +1268,9 @@ __global__ void __launch_bounds__(1024) k3_adj_remove_mean(int N, int NS, const 
 // adjoint of  div = fluxdiv(hb)  and of  x = P^-1 div  w.r.t. P(rA):  given lam = P^-1 x_bar (P is symmetric on these grids)
 //   P_ij = 1/2 (alpha_i rA_i + alpha_j rA_j) across face (i, j), P_ii = - sum_j P_ij,  P_bar_ij = -lam_i x_j
 __global__ void __launch_bounds__(O3_T) k3_adj_pressure_rhs(T3 t, const float *__restrict__ Lam, const float *__restrict__ X, float *__restrict__ Hbb,
-                                                            float *__restrict__ Fbb, float *__restrict__ rAb) {
+                                                            float *__restrict__ Fbb, float *__restrict__ rAb, const int32_t *__restrict__ active) {
     const int b = blockIdx.y, g = blockIdx.x * blockDim.x + threadIdx.x, NS = t.NS;
-    if (g >= t.N) return;
+    if (g >= t.N || (active && !active[b])) return;
     const float lam = Lam[(size_t)b * NS + g];
     const float *x = X + (size_t)b * NS;
     float *ra = rAb + (size_t)b * NS;
@@ -1295,9 +1296,9 @@ __global__ void __launch_bounds__(O3_T) k3_adj_pressure_rhs(T3 t, const float *_
 __global__ void __launch_bounds__(O3_T) k3_adj_hbya(T3 t, const float *__restrict__ Hbb, const float *__restrict__ Hb /*saved hb*/,
                                                     const float *__restrict__ A, const float *__restrict__ Coff, const float *__restrict__ Uprev,
                                                     const float *__restrict__ dtv, float *__restrict__ rAb, float *__restrict__ Ub,
-                                                    float *__restrict__ Sbb, float *__restrict__ Coffb, float *__restrict__ Uprevb) {
+                                                    float *__restrict__ Sbb, float *__restrict__ Coffb, float *__restrict__ Uprevb, const int32_t *__restrict__ active) {
     const int b = blockIdx.y, g = blockIdx.x * blockDim.x + threadIdx.x, NS = t.NS;
-    if (g >= t.N) return;
+    if (g >= t.N || (active && !active[b])) return;
     const float dt = dtv[b], Ag = A[(size_t)b * NS + g], rA = 1.0f / Ag, det = t.det[g];
     int nb6[6];
     o3_nbrs(t, g, nb6);
@@ -1324,9 +1325,9 @@ __global__ void __launch_bounds__(O3_T) k3_adj_hbya(T3 t, const float *__restric
 // adjoint of the predictor  C ustar = rhs,  rhs = u/dt + Sb/det + src,  C = A I + Coff:  given mu = C^-T ustar_bar
 __global__ void __launch_bounds__(O3_T) k3_adj_advection(T3 t, const float *__restrict__ Mu, const float *__restrict__ Ustar, const float *__restrict__ rAb,
                                                          const float *__restrict__ A, const float *__restrict__ dtv, float *__restrict__ Ab,
-                                                         float *__restrict__ Coffb, float *__restrict__ Ub, float *__restrict__ Sbb) {
+                                                         float *__restrict__ Coffb, float *__restrict__ Ub, float *__restrict__ Sbb, const int32_t *__restrict__ active) {
     const int b = blockIdx.y, g = blockIdx.x * blockDim.x + threadIdx.x, NS = t.NS;
-    if (g >= t.N) return;
+    if (g >= t.N || (active && !active[b])) return;
     const float dt = dtv[b], det = t.det[g], Ag = A[(size_t)b * NS + g];
     int nb6[6];
     o3_nbrs(t, g, nb6);
@@ -1346,9 +1347,9 @@ __global__ void __launch_bounds__(O3_T) k3_adj_advection(T3 t, const float *__re
 // adjoint of the assembly (A, Coff from the face fluxes; constant viscosity) and of the boundary sources Sb
 __global__ void __launch_bounds__(O3_T) k3_adj_assemble(T3 t, const float *__restrict__ Ab, const float *__restrict__ Coffb, const float *__restrict__ Sbb,
                                                         const float *__restrict__ Bvel, float *__restrict__ Ub, float *__restrict__ Bvb, float *__restrict__ Fbb,
-                                                        const float *__restrict__ Visc /* [B][NS] taped per-cell viscosity or null */) {
+                                                        const float *__restrict__ Visc /* [B][NS] taped per-cell viscosity or null */, const int32_t *__restrict__ active) {
     const int b = blockIdx.y, g = blockIdx.x * blockDim.x + threadIdx.x, NS = t.NS, NB = t.NB;
-    if (g >= t.N) return;
+    if (g >= t.N || (active && !active[b])) return;
     const float det = t.det[g], diagb = Ab[(size_t)b * NS + g] / det;
     const float *bv = Bvel + (size_t)b * 3 * NB;
     int nb6[6];
@@ -1377,18 +1378,18 @@ __global__ void __launch_bounds__(O3_T) k3_adj_assemble(T3 t, const float *__res
 }
 // Passive scalar + buoyancy (RBC3D).  The source (0, beta T_new, 0) enters the predictor right-hand side and HbyA next to S_b / det, so
 // its adjoint is det * S_b_bar:  T_new_bar = T_out_bar + beta * det * S_b_bar[1]
-__global__ void __launch_bounds__(O3_T) k3_adj_buoyancy(T3 t, const float *__restrict__ Sbb, const float *__restrict__ Toutb, float beta, float *__restrict__ Tnb) {
+__global__ void __launch_bounds__(O3_T) k3_adj_buoyancy(T3 t, const float *__restrict__ Sbb, const float *__restrict__ Toutb, float beta, float *__restrict__ Tnb, const int32_t *__restrict__ active) {
     const int b = blockIdx.y, g = blockIdx.x * blockDim.x + threadIdx.x, NS = t.NS;
-    if (g >= t.N) return;
+    if (g >= t.N || (active && !active[b])) return;
     Tnb[(size_t)b * NS + g] = Toutb[(size_t)b * NS + g] + beta * t.det[g] * Sbb[((size_t)b * 3 + 1) * NS + g];
 }
 // adjoint of k3_setup_scalar + the scalar solve, given lam = C_s^-T T_new_bar:  A_s_bar = -lam T_new, Coff_s_bar[f] = -lam T_new[nb_f];
 // rhs_s = r / det with r = det T_in / dt + sum_{prescribed f} sb (-(sig F_b) + 2 kappa alpha_b)
 __global__ void __launch_bounds__(O3_T) k3_adj_scalar(T3 t, const float *__restrict__ Lam, const float *__restrict__ Tnew, const float *__restrict__ Bvel,
                                                       const float *__restrict__ Sbval, float kappa, const float *__restrict__ dtv,
-                                                      float *__restrict__ Tinb, float *__restrict__ Sbvalb, float *__restrict__ Fbb, float *__restrict__ Ub) {
+                                                      float *__restrict__ Tinb, float *__restrict__ Sbvalb, float *__restrict__ Fbb, float *__restrict__ Ub, const int32_t *__restrict__ active) {
     const int b = blockIdx.y, g = blockIdx.x * blockDim.x + threadIdx.x, NS = t.NS, NB = t.NB;
-    if (g >= t.N) return;
+    if (g >= t.N || (active && !active[b])) return;
     const float *tn = Tnew + (size_t)b * NS, *bv = Bvel + (size_t)b * 3 * NB, *sb = Sbval + (size_t)b * NB;
     const float lam = Lam[(size_t)b * NS + g], det = t.det[g], rb = lam / det;
     Tinb[(size_t)b * NS + g] = lam / dtv[b];
@@ -1411,9 +1412,9 @@ __global__ void __launch_bounds__(O3_T) k3_adj_scalar(T3 t, const float *__restr
     o3_fluxes_adjoint(t, g, nb6, flb, Ub + (size_t)b * 3 * NS, nullptr);
 }
 // adjoint of the boundary flux Fb_j = b_det minv_d bv_d (d = axis of the face): one thread per (boundary face, environment)
-__global__ void k3_adj_bflux(T3 t, const float *__restrict__ Fbb, float *__restrict__ Bvb) {
+__global__ void k3_adj_bflux(T3 t, const float *__restrict__ Fbb, float *__restrict__ Bvb, const int32_t *__restrict__ active) {
     const int b = blockIdx.y, j = blockIdx.x * blockDim.x + threadIdx.x, NB = t.NB;
-    if (j >= NB) return;
+    if (j >= NB || (active && !active[b])) return;
     const int cnt[3] = {t.ny * t.nz, t.nx * t.nz, t.nx * t.ny};
     int d = -1;
 #pragma unroll
@@ -1426,6 +1427,14 @@ static int o3_copy(void *dst, const void *src, size_t bytes, cudaStream_t st) {
     cudaError_t ce = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, st);
     return ce == cudaSuccess ? FGB_OK : set_err(FGB_E_CUDA, "cudaMemcpyAsync (D = 3 tape)", ce);
 }
+// dst <- src ([B][n / B] floats) for the environments of active (NULL: a plain copy of everything)
+static int o3_copy_active(fgb_ortho3 *b, float *dst, const float *src, size_t n, const int32_t *active, cudaStream_t st) {
+    if (!active) return o3_copy(dst, src, n * 4, st);
+    b->launches++;
+    k3_copy_active<<<dim3((unsigned)((n / b->B + 255) / 256), (unsigned)b->B), 256, 0, st>>>(src, dst, n / b->B, active);
+    LAUNCH_CHECK("k3_copy_active");
+    return FGB_OK;
+}
 static int o3_adjoint_supported(const fgb_ortho3 *b, bool with_scalar) {
     if (b->slab.on || b->t.NS != b->t.N) return set_err(FGB_E_ARG, "D = 3 reverse mode: single GPU only (no slabs)");
     if (b->t.nx <= 0) return set_err(FGB_E_ARG, "D = 3 reverse mode: needs the structured-box description (tables.nx/ny/nz/closed/boff)");
@@ -1435,7 +1444,8 @@ static int o3_adjoint_supported(const fgb_ortho3 *b, bool with_scalar) {
     if (b->opt.corrector_steps < 1 || b->opt.corrector_steps > 8) return set_err(FGB_E_ARG, "D = 3 reverse mode: 1..8 corrector steps");
     return FGB_OK;
 }
-// fgb_ortho3_piso_substep (all environments active) that additionally records the tape of the backward pass
+// fgb_ortho3_piso_substep for the environments of tp->active (NULL: all) that additionally records the tape of the backward pass; a
+// skipped environment keeps u, p (and T) bit for bit (every kernel and solve skips it, the final u <- ures copy is masked)
 static int o3_record_impl(fgb_ortho3 *b, float *u, float *p, const float *bvel, const float *src, const float *dt,
                           const fgb_ortho3_tape *tp, const fgb_tape_scalar *stp, fgb_stream_t s) {
     if (!b || !u || !p || !bvel || !dt || !tp) return set_err(FGB_E_ARG, "fgb_ortho3_piso_substep_record: null argument");
@@ -1445,35 +1455,36 @@ static int o3_record_impl(fgb_ortho3 *b, float *u, float *p, const float *bvel, 
     cudaStream_t st = STREAM(s);
     const size_t BN = (size_t)b->B * b->t.NS, BNB = (size_t)b->B * (b->t.NB > 0 ? b->t.NB : 1);
     const int C = b->opt.corrector_steps;
+    const int32_t *act = tp->active;
     if ((rc = o3_copy(tp->u_in, u, 3 * BN * 4, st))) return rc;
     if ((rc = o3_copy(tp->bvel_in, bvel, 3 * BNB * 4, st))) return rc;
     if ((rc = o3_copy(tp->dt, dt, (size_t)b->B * 4, st))) return rc;
     if (stp) {      // scalar transport with the incoming velocity first; the predictor / HbyA then read the new temperature (buoyancy)
         if ((rc = o3_copy(stp->T_in, b->sc.T, BN * 4, st))) return rc;
         if ((rc = o3_copy(stp->sbval_in, b->sc.sbval, BNB * 4, st))) return rc;
-        if ((rc = fgb_ortho3_advect_scalar(b, u, bvel, dt, nullptr, s))) return rc;
+        if ((rc = fgb_ortho3_advect_scalar(b, u, bvel, dt, act, s))) return rc;
         if ((rc = o3_copy(stp->T_out, b->sc.T, BN * 4, st))) return rc;
     }
     if (b->sgs_coef != 0.f) {     // per-cell viscosity of this substep: a CONSTANT of the graph, as in the reference (its Smagorinsky op has no
                                   // autograd wrapper: tcf_env.py:456-470 sets the block viscosity from a raw extension call)
         if (!tp->visc) return set_err(FGB_E_ARG, "fgb_ortho3_piso_substep_record: sub-grid model set, the tape needs a visc buffer");
-        if ((rc = fgb_ortho3_sgs_viscosity(b, u, bvel, nullptr, s))) return rc;
+        if ((rc = fgb_ortho3_sgs_viscosity(b, u, bvel, act, s))) return rc;
         if ((rc = o3_copy(tp->visc, b->visc, BN * 4, st))) return rc;
     }
-    if ((rc = fgb_ortho3_setup_advection(b, u, bvel, src, dt, nullptr, s))) return rc;
-    if ((rc = fgb_ortho3_solve_advection(b, 1, nullptr, s))) return rc;
+    if ((rc = fgb_ortho3_setup_advection(b, u, bvel, src, dt, act, s))) return rc;
+    if ((rc = fgb_ortho3_solve_advection(b, 1, act, s))) return rc;
     if ((rc = o3_copy(tp->ustar, b->ures, 3 * BN * 4, st))) return rc;
     if ((rc = o3_copy(tp->Coff, b->Coff, 6 * BN * 4, st))) return rc;
     if ((rc = o3_copy(tp->A, b->A, BN * 4, st))) return rc;
     for (int cs = 0; cs < C; ++cs) {
-        if ((rc = fgb_ortho3_setup_pressure(b, u, bvel, src, dt, cs == 0, nullptr, s))) return rc;
+        if ((rc = fgb_ortho3_setup_pressure(b, u, bvel, src, dt, cs == 0, act, s))) return rc;
         if ((rc = o3_copy(tp->hb + (size_t)cs * 3 * BN, b->hbya, 3 * BN * 4, st))) return rc;
-        if ((rc = fgb_ortho3_solve_pressure(b, p, 1, 0, b->opt.max_iter, cs, nullptr, s))) return rc;      // zero start, no residual reset
+        if ((rc = fgb_ortho3_solve_pressure(b, p, 1, 0, b->opt.max_iter, cs, act, s))) return rc;      // zero start, no residual reset
         if ((rc = o3_copy(tp->p + (size_t)cs * BN, p, BN * 4, st))) return rc;
-        if ((rc = fgb_ortho3_correct_velocity(b, p, b->ures, nullptr, s))) return rc;
+        if ((rc = fgb_ortho3_correct_velocity(b, p, b->ures, act, s))) return rc;
         if (cs + 1 < C && (rc = o3_copy(tp->u1 + (size_t)cs * 3 * BN, b->ures, 3 * BN * 4, st))) return rc;
     }
-    return o3_copy(u, b->ures, 3 * BN * 4, st);
+    return o3_copy_active(b, u, b->ures, 3 * BN, act, st);
 }
 extern "C" int fgb_ortho3_piso_substep_record(fgb_ortho3 *b, float *u, float *p, const float *bvel, const float *src, const float *dt,
                                               const fgb_ortho3_tape *tp, fgb_stream_t s) {
@@ -1489,7 +1500,8 @@ extern "C" size_t fgb_ortho3_adjoint_workspace_bytes(const fgb_ortho3_tables *t,
     const size_t BN = (size_t)B * (t->NS > 0 ? t->NS : t->N), BNB = (size_t)B * (t->NB > 0 ? t->NB : 1);
     return (size_t)(3 + 3 + 1 + 6 + 3 + 1 + 1 + 1 + 3 + 1 + 3) * align_up(BN * 4) + align_up(BNB * 4) + 8192;
 }
-// vector-Jacobian product of that substep: (u_out_bar, p_out_bar) -> (u_bar, bvel_bar), both overwritten
+// vector-Jacobian product of that substep: (u_out_bar, p_out_bar) -> (u_bar, bvel_bar), both overwritten; environments tp->active skips
+// are skipped by every adjoint kernel and transposed solve and get the identity cotangents (k_adj_inactive)
 static int o3_backward_impl(fgb_ortho3 *b, const fgb_ortho3_tape *tp, const fgb_tape_scalar *stp, const float *u_out_bar, const float *p_out_bar,
                             const float *T_out_bar, float *u_bar, float *bvel_bar, float *T_bar, float *sbval_bar, void *ws, size_t ws_bytes,
                             fgb_stream_t s) {
@@ -1502,6 +1514,7 @@ static int o3_backward_impl(fgb_ortho3 *b, const fgb_ortho3_tape *tp, const fgb_
     if (b->sgs_coef != 0.f && !tp->visc) return set_err(FGB_E_ARG, "fgb_ortho3_piso_substep_backward: sub-grid model set, the tape needs its visc buffer");
     cudaStream_t st = STREAM(s);
     const size_t B = b->B, NB = b->t.NB > 0 ? b->t.NB : 1, BN = B * b->t.NS;
+    const int32_t *act = tp->active;
     Carver c{(char *)ws, 0};
     float *unb = c.take<float>(3 * BN), *hbb = c.take<float>(3 * BN), *rAb = c.take<float>(BN), *Coffb = c.take<float>(6 * BN);
     float *Sbb = c.take<float>(3 * BN), *pb = c.take<float>(BN), *xb = c.take<float>(BN), *lam = c.take<float>(BN);
@@ -1514,37 +1527,37 @@ static int o3_backward_impl(fgb_ortho3 *b, const fgb_ortho3_tape *tp, const fgb_
     if ((rc = o3_copy(unb, u_out_bar, 3 * BN * 4, st))) return rc;
     if ((rc = o3_copy(pb, p_out_bar, BN * 4, st))) return rc;
     b->launches++;
-    k3_pressure_matrix<<<grid, O3_T, 0, st>>>(b->t, tp->A, nullptr, b->Poff, b->Pdiag);      // the pressure matrix of this substep (function of A only)
+    k3_pressure_matrix<<<grid, O3_T, 0, st>>>(b->t, tp->A, act, b->Poff, b->Pdiag);      // the pressure matrix of this substep (function of A only)
     LAUNCH_CHECK("k3_pressure_matrix (backward)");
     for (int cs = C - 1; cs >= 0; --cs) {
         const float *hb_c = tp->hb + (size_t)cs * 3 * BN, *p_c = tp->p + (size_t)cs * BN;
         const float *uprev = cs == 0 ? tp->ustar : tp->u1 + (size_t)(cs - 1) * 3 * BN;
         b->launches += 4;
-        k3_adj_correct<<<grid, O3_T, 0, st>>>(b->t, unb, p_c, tp->A, hbb, rAb, pb);
+        k3_adj_correct<<<grid, O3_T, 0, st>>>(b->t, unb, p_c, tp->A, hbb, rAb, pb, act);
         LAUNCH_CHECK("k3_adj_correct");
-        k3_adj_remove_mean<<<b->B, 1024, 0, st>>>(b->t.N, b->t.NS, pb, xb);
+        k3_adj_remove_mean<<<b->B, 1024, 0, st>>>(b->t.N, b->t.NS, pb, xb, act);
         LAUNCH_CHECK("k3_adj_remove_mean");
         {   // lam = P^-1 x_bar (P symmetric): the forward CG kernel, zero start, no residual reset, right-hand side xb
             T3 t = b->t; O3Slab sl = b->slab; int Bi = b->B; const float *poff = b->Poff, *pd = b->Pdiag, *rhs = xb; float *work = b->kry, *part = b->part;
-            float tol = b->opt.p_tol; int max_iter = b->opt.max_iter, zero_init = 1, reset_steps = 0, slot = 4; const int32_t *active = nullptr;
+            float tol = b->opt.p_tol; int max_iter = b->opt.max_iter, zero_init = 1, reset_steps = 0, slot = 4; const int32_t *active = act;
             int32_t *iters = b->iters; float *resid = b->resid; unsigned long long *itot = b->iter_total; float *out = lam;
             float *pmean = b->pmean;
             void *args[] = {&t, &sl, &Bi, &poff, &pd, &rhs, &out, &work, &part, &max_iter, &tol, &zero_init, &reset_steps, &slot, &active, &iters, &resid, &itot, &pmean};
             ce = cudaLaunchCooperativeKernel(b->cg_fused ? (void *)k3_cg_fused : (void *)k3_cg<0>, dim3(o3_coop_blocks(b)), dim3(O3_CT), args, 0, st);
             if (ce != cudaSuccess) return set_err(FGB_E_CUDA, "cudaLaunchCooperativeKernel(k3_cg, backward)", ce);
         }
-        k3_adj_pressure_rhs<<<grid, O3_T, 0, st>>>(b->t, lam, p_c, hbb, Fbb, rAb);
+        k3_adj_pressure_rhs<<<grid, O3_T, 0, st>>>(b->t, lam, p_c, hbb, Fbb, rAb, act);
         LAUNCH_CHECK("k3_adj_pressure_rhs");
         ZERO3(pb, BN);                         // the previous pressure does not enter this corrector (zero-started solve, orthogonal grid)
         ZERO3(uprevb, 3 * BN);
         b->launches++;
-        k3_adj_hbya<<<grid, O3_T, 0, st>>>(b->t, hbb, hb_c, tp->A, tp->Coff, uprev, tp->dt, rAb, u_bar, Sbb, Coffb, uprevb);
+        k3_adj_hbya<<<grid, O3_T, 0, st>>>(b->t, hbb, hb_c, tp->A, tp->Coff, uprev, tp->dt, rAb, u_bar, Sbb, Coffb, uprevb, act);
         LAUNCH_CHECK("k3_adj_hbya");
         float *tmp = unb; unb = uprevb; uprevb = tmp;       // gradient w.r.t. the velocity entering this corrector
     }
     {   // mu = C^-T ustar_bar
         T3 t = b->t; O3Slab sl = b->slab; int Bi = b->B; const float *coff = tp->Coff, *a = tp->A, *rhs = unb; float *x = mu, *work = b->kry, *part = b->part;
-        int maxit = b->opt.max_iter, zero_init = 1, transposed = 1; float tol = b->opt.adv_tol; const int32_t *active = nullptr;
+        int maxit = b->opt.max_iter, zero_init = 1, transposed = 1; float tol = b->opt.adv_tol; const int32_t *active = act;
         int32_t *iters = b->iters; float *resid = b->resid; unsigned long long *itot = b->iter_total;
         void *args[] = {&t, &sl, &Bi, &coff, &a, &rhs, &x, &work, &part, &maxit, &tol, &zero_init, &active, &iters, &resid, &itot, &transposed};
         b->launches++;
@@ -1552,9 +1565,9 @@ static int o3_backward_impl(fgb_ortho3 *b, const fgb_ortho3_tape *tp, const fgb_
         if (ce != cudaSuccess) return set_err(FGB_E_CUDA, "cudaLaunchCooperativeKernel(k3_bicgstab, transposed)", ce);
     }
     b->launches += 3;
-    k3_adj_advection<<<grid, O3_T, 0, st>>>(b->t, mu, tp->ustar, rAb, tp->A, tp->dt, Ab, Coffb, u_bar, Sbb);
+    k3_adj_advection<<<grid, O3_T, 0, st>>>(b->t, mu, tp->ustar, rAb, tp->A, tp->dt, Ab, Coffb, u_bar, Sbb, act);
     LAUNCH_CHECK("k3_adj_advection");
-    k3_adj_assemble<<<grid, O3_T, 0, st>>>(b->t, Ab, Coffb, Sbb, tp->bvel_in, u_bar, bvel_bar, Fbb, b->sgs_coef != 0.f ? tp->visc : nullptr);
+    k3_adj_assemble<<<grid, O3_T, 0, st>>>(b->t, Ab, Coffb, Sbb, tp->bvel_in, u_bar, bvel_bar, Fbb, b->sgs_coef != 0.f ? tp->visc : nullptr, act);
     LAUNCH_CHECK("k3_adj_assemble");
     if (stp) {
         // buoyancy + scalar transport (they ran BEFORE the predictor): T_new_bar from the source adjoint, one transposed scalar solve,
@@ -1562,28 +1575,30 @@ static int o3_backward_impl(fgb_ortho3 *b, const fgb_ortho3_tape *tp, const fgb_
         // the forward workspace (Coff / A / rhs are not read by this pass any more).
         float *Tnb = xb;
         b->launches += 4;
-        k3_adj_buoyancy<<<grid, O3_T, 0, st>>>(b->t, Sbb, T_out_bar, b->sc.beta, Tnb);
+        k3_adj_buoyancy<<<grid, O3_T, 0, st>>>(b->t, Sbb, T_out_bar, b->sc.beta, Tnb, act);
         LAUNCH_CHECK("k3_adj_buoyancy");
-        k3_setup_scalar<<<grid, O3_T, 0, st>>>(b->t, tp->u_in, stp->T_in, tp->bvel_in, stp->sbval_in, b->sc.kappa, tp->dt, nullptr, b->Coff, b->A, b->rhs);
+        k3_setup_scalar<<<grid, O3_T, 0, st>>>(b->t, tp->u_in, stp->T_in, tp->bvel_in, stp->sbval_in, b->sc.kappa, tp->dt, act, b->Coff, b->A, b->rhs);
         LAUNCH_CHECK("k3_setup_scalar (backward)");
         {   // lam = C_s^-T T_new_bar
             T3 t = b->t; O3Slab sl = b->slab; int Bi = b->B; const float *coff = b->Coff, *a = b->A, *rhs = Tnb; float *x = lam, *work = b->kry, *part = b->part;
-            int maxit = b->opt.max_iter, zero_init = 1, transposed = 1; float tol = b->opt.adv_tol; const int32_t *active = nullptr;
+            int maxit = b->opt.max_iter, zero_init = 1, transposed = 1; float tol = b->opt.adv_tol; const int32_t *active = act;
             int32_t *iters = b->iters; float *resid = b->resid; unsigned long long *itot = b->iter_total;
             void *args[] = {&t, &sl, &Bi, &coff, &a, &rhs, &x, &work, &part, &maxit, &tol, &zero_init, &active, &iters, &resid, &itot, &transposed};
             ce = cudaLaunchCooperativeKernel((b->bicg_fused ? (void *)k3_bicgstab<1, 1> : (void *)k3_bicgstab<1, 0>), dim3(o3_coop_blocks(b)), dim3(O3_CT), args, 0, st);
             if (ce != cudaSuccess) return set_err(FGB_E_CUDA, "cudaLaunchCooperativeKernel(k3_bicgstab<1>, transposed)", ce);
         }
         ZERO3(sbval_bar, B * NB);
-        k3_adj_scalar<<<grid, O3_T, 0, st>>>(b->t, lam, stp->T_out, tp->bvel_in, stp->sbval_in, b->sc.kappa, tp->dt, T_bar, sbval_bar, Fbb, u_bar);
+        k3_adj_scalar<<<grid, O3_T, 0, st>>>(b->t, lam, stp->T_out, tp->bvel_in, stp->sbval_in, b->sc.kappa, tp->dt, T_bar, sbval_bar, Fbb, u_bar, act);
         LAUNCH_CHECK("k3_adj_scalar");
     }
     if (b->t.NB > 0) {
-        k3_adj_bflux<<<dim3((unsigned)((b->t.NB + 127) / 128), b->B), 128, 0, st>>>(b->t, Fbb, bvel_bar);
+        k3_adj_bflux<<<dim3((unsigned)((b->t.NB + 127) / 128), b->B), 128, 0, st>>>(b->t, Fbb, bvel_bar, act);
         LAUNCH_CHECK("k3_adj_bflux");
     }
 #undef ZERO3
-    return FGB_OK;
+    if (act) b->launches++;
+    return launch_adj_inactive(act, b->B, 3, b->t.NS, u_out_bar, u_bar, nullptr, nullptr, stp ? T_out_bar : nullptr, stp ? T_bar : nullptr,
+                               (int)(3 * NB), bvel_bar, stp ? (int)NB : 0, stp ? sbval_bar : nullptr, st);
 }
 extern "C" int fgb_ortho3_piso_substep_backward(fgb_ortho3 *b, const fgb_ortho3_tape *tp, const float *u_out_bar, const float *p_out_bar,
                                                 float *u_bar, float *bvel_bar, void *ws, size_t ws_bytes, fgb_stream_t s) {
@@ -1661,6 +1676,15 @@ __global__ void k3_plan_substep(int B, double *__restrict__ remaining, float *__
         atomicAdd(&counters[0], 1);
     }
     dtv[b] = dt; active[b] = act;
+}
+
+// the planner of one round without a handle (differentiable rollouts plan per environment on the host's behalf: solver.py::cfl_substeps_per_env)
+extern "C" int fgb_plan_substep(int32_t B, const float *maxvel, double *remaining, float cfl, float *dt, int32_t *active, int32_t *nsub,
+                                int32_t *counter, fgb_stream_t s) {
+    if (B < 1 || !maxvel || !remaining || !dt || !active || !nsub || !counter) return set_err(FGB_E_ARG, "fgb_plan_substep: bad argument");
+    k3_plan_substep<<<(B + 127) / 128, 128, 0, STREAM(s)>>>(B, remaining, dt, active, nsub, maxvel, counter, cfl);
+    LAUNCH_CHECK("k3_plan_substep");
+    return FGB_OK;
 }
 
 // mean streamwise velocity of the first and last wall-normal cell layers -> wall shear stresses and the dynamic

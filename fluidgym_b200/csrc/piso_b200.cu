@@ -3037,8 +3037,10 @@ __device__ __forceinline__ void fluxes_adjoint(const Tab &t, int g, const int nb
 
 // adjoint of the corrector u_next = hb - rA * Minv^T grad(p):  hbb += unb ; rAb += -(g . unb) ; pb += grad^T(...)
 __global__ void __launch_bounds__(256) k_adj_correct(Tab t, const float *__restrict__ Unb, const float *__restrict__ P, const float *__restrict__ A,
-                                                      float *__restrict__ Hbb, float *__restrict__ rAb, float *__restrict__ Pb) {
+                                                      float *__restrict__ Hbb, float *__restrict__ rAb, float *__restrict__ Pb,
+                                                      const int32_t *__restrict__ active) {
     const int b = blockIdx.y;
+    if (active && !active[b]) return;   // skipped environment: identity cotangents from k_adj_inactive
     const int g = blockIdx.x * blockDim.x + threadIdx.x;
     const int N = t.N;
     if (g >= N) return;
@@ -3070,9 +3072,11 @@ __global__ void __launch_bounds__(256) k_adj_correct(Tab t, const float *__restr
 
 // x_bar = p_bar - mean(p_bar)   (adjoint of the mean removal), one CTA per environment
 template <int T>
-__global__ void __launch_bounds__(T) k_adj_remove_mean(int N, const float *__restrict__ Pb, float *__restrict__ Xb) {
+__global__ void __launch_bounds__(T) k_adj_remove_mean(int N, const float *__restrict__ Pb, float *__restrict__ Xb,
+                                                        const int32_t *__restrict__ active) {
     __shared__ double red[32 * 2 + 2];
     const int b = blockIdx.x;
+    if (active && !active[b]) return;   // skipped environment: identity cotangents from k_adj_inactive
     float acc[2] = {0.f, 0.f};
     for (int g = threadIdx.x; g < N; g += T) acc[0] += Pb[(size_t)b * N + g];
     block_reduce_sum<2>(acc, red);
@@ -3084,8 +3088,9 @@ __global__ void __launch_bounds__(T) k_adj_remove_mean(int N, const float *__res
 __global__ void __launch_bounds__(256) k_adj_pressure_rhs(Tab t, const float *__restrict__ Lam, const float *__restrict__ Pm /*p of this corrector*/,
                                                            const float *__restrict__ Pmean, const float *__restrict__ Pprev,
                                                            const float *__restrict__ A, float *__restrict__ Hbb, float *__restrict__ Fbb,
-                                                           float *__restrict__ rAb, float *__restrict__ Pprevb) {
+                                                           float *__restrict__ rAb, float *__restrict__ Pprevb, const int32_t *__restrict__ active) {
     const int b = blockIdx.y;
+    if (active && !active[b]) return;   // skipped environment: identity cotangents from k_adj_inactive
     const int g = blockIdx.x * blockDim.x + threadIdx.x;
     const int N = t.N, NB = t.NB;
     if (g >= N) return;
@@ -3132,8 +3137,10 @@ __global__ void __launch_bounds__(256) k_adj_pressure_rhs(Tab t, const float *__
 __global__ void __launch_bounds__(256) k_adj_hbya(Tab t, const float *__restrict__ Hbb, const float *__restrict__ Hb /*saved hb*/,
                                                    const float *__restrict__ A, const float *__restrict__ Coff, const float *__restrict__ Uprev,
                                                    const float *__restrict__ dtv, float *__restrict__ rAb, float *__restrict__ Ub,
-                                                   float *__restrict__ Sbb, float *__restrict__ Coffb, float *__restrict__ Uprevb) {
+                                                   float *__restrict__ Sbb, float *__restrict__ Coffb, float *__restrict__ Uprevb,
+                                                   const int32_t *__restrict__ active) {
     const int b = blockIdx.y;
+    if (active && !active[b]) return;   // skipped environment: identity cotangents from k_adj_inactive
     const int g = blockIdx.x * blockDim.x + threadIdx.x;
     const int N = t.N;
     if (g >= N) return;
@@ -3167,8 +3174,10 @@ __global__ void __launch_bounds__(256) k_adj_advection(Tab t, const float *__res
                                                         const float *__restrict__ A, const float *__restrict__ dtv, float *__restrict__ Ab,
                                                         float *__restrict__ Coffb, float *__restrict__ Ub, float *__restrict__ Sbb, float *__restrict__ Bvb,
                                                         float *__restrict__ NoTarget /* adjoint of the field the deferred term read: u_bar (first
-                                                        iteration) or the previous iterate's bar */, int first /* initialise A_bar from rA_bar */) {
+                                                        iteration) or the previous iterate's bar */, int first /* initialise A_bar from rA_bar */,
+                                                        const int32_t *__restrict__ active) {
     const int b = blockIdx.y;
+    if (active && !active[b]) return;   // skipped environment: identity cotangents from k_adj_inactive
     const int g = blockIdx.x * blockDim.x + threadIdx.x;
     const int N = t.N, NB = t.NB;
     if (g >= N) return;
@@ -3200,8 +3209,10 @@ __global__ void __launch_bounds__(256) k_adj_advection(Tab t, const float *__res
 
 // adjoint of the assembly (A, Coff from the face fluxes) and of the boundary sources
 __global__ void __launch_bounds__(256) k_adj_assemble(Tab t, const float *__restrict__ Ab, const float *__restrict__ Coffb, const float *__restrict__ Sbb,
-                                                       const float *__restrict__ Bvel, float *__restrict__ Ub, float *__restrict__ Bvb, float *__restrict__ Fbb) {
+                                                       const float *__restrict__ Bvel, float *__restrict__ Ub, float *__restrict__ Bvb, float *__restrict__ Fbb,
+                                                       const int32_t *__restrict__ active) {
     const int b = blockIdx.y;
+    if (active && !active[b]) return;   // skipped environment: identity cotangents from k_adj_inactive
     const int g = blockIdx.x * blockDim.x + threadIdx.x;
     const int N = t.N, NB = t.NB;
     if (g >= N) return;
@@ -3229,8 +3240,9 @@ __global__ void __launch_bounds__(256) k_adj_assemble(Tab t, const float *__rest
 }
 
 // adjoint of Fb(bvel): one thread per (boundary face, environment)
-__global__ void k_adj_bflux(Tab t, const float *__restrict__ Fbb, float *__restrict__ Bvb) {
+__global__ void k_adj_bflux(Tab t, const float *__restrict__ Fbb, float *__restrict__ Bvb, const int32_t *__restrict__ active) {
     const int b = blockIdx.y;
+    if (active && !active[b]) return;   // skipped environment: identity cotangents from k_adj_inactive
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
     const int NB = t.NB;
     if (j >= NB) return;
@@ -3244,8 +3256,9 @@ __global__ void k_adj_bflux(Tab t, const float *__restrict__ Fbb, float *__restr
 // S_b / det, so its adjoint is det * S_b_bar; with src = (0, beta * T_new):
 //   T_new_bar = T_out_bar + beta * det * S_b_bar[1]
 __global__ void __launch_bounds__(256) k_adj_buoyancy(Tab t, const float *__restrict__ Sbb, const float *__restrict__ Toutb, float beta,
-                                                       float *__restrict__ Tnb) {
+                                                       float *__restrict__ Tnb, const int32_t *__restrict__ active) {
     const int b = blockIdx.y;
+    if (active && !active[b]) return;   // skipped environment: identity cotangents from k_adj_inactive
     const int g = blockIdx.x * blockDim.x + threadIdx.x;
     const int N = t.N;
     if (g >= N) return;
@@ -3258,8 +3271,9 @@ __global__ void __launch_bounds__(256) k_adj_buoyancy(Tab t, const float *__rest
 __global__ void __launch_bounds__(256) k_adj_scalar(Tab t, const float *__restrict__ Lam, const float *__restrict__ Tnew,
                                                      const float *__restrict__ Bvel, const float *__restrict__ Sbval,
                                                      const float *__restrict__ dtv, float *__restrict__ Tinb, float *__restrict__ Sbvalb,
-                                                     float *__restrict__ Fbb, float *__restrict__ Ub) {
+                                                     float *__restrict__ Fbb, float *__restrict__ Ub, const int32_t *__restrict__ active) {
     const int b = blockIdx.y;
+    if (active && !active[b]) return;   // skipped environment: identity cotangents from k_adj_inactive
     const int g = blockIdx.x * blockDim.x + threadIdx.x;
     const int N = t.N, NB = t.NB;
     if (g >= N) return;
@@ -3285,6 +3299,36 @@ __global__ void __launch_bounds__(256) k_adj_scalar(Tab t, const float *__restri
         }
     }
     fluxes_adjoint(t, g, nb, flb, Ub + (size_t)b * 2 * N, nullptr);
+}
+
+// Cotangents of the environments a masked substep skipped (fgb_tape.active == 0): the substep is the identity there, so
+// u_bar = u_out_bar, p_prev_bar = p_out_bar, T_bar = T_out_bar, bvel_bar = 0, sbval_bar = 0.  Shared by the 2-D, box and extruded
+// reverse passes: nc velocity components and n cells per environment (p / T arrays optional), nbv boundary-velocity and nsb
+// boundary-scalar values per environment.  One thread per (index, environment) over max(nc * n, nbv, nsb).
+__global__ void k_adj_inactive(const int32_t *__restrict__ active, int nc, int n, const float *__restrict__ Uob, float *__restrict__ Ub,
+                               const float *__restrict__ Pob, float *__restrict__ Pb, const float *__restrict__ Tob, float *__restrict__ Tb,
+                               int nbv, float *__restrict__ Bvb, int nsb, float *__restrict__ Sbb) {
+    const int b = blockIdx.y;
+    if (active[b]) return;
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    const size_t nu = (size_t)nc * n;
+    if ((size_t)i < nu) Ub[b * nu + i] = Uob[b * nu + i];
+    if (i < n) {
+        if (Pb) Pb[(size_t)b * n + i] = Pob[(size_t)b * n + i];
+        if (Tb) Tb[(size_t)b * n + i] = Tob[(size_t)b * n + i];
+    }
+    if (i < nbv) Bvb[(size_t)b * nbv + i] = 0.f;
+    if (Sbb && i < nsb) Sbb[(size_t)b * nsb + i] = 0.f;
+}
+static int launch_adj_inactive(const int32_t *active, int B, int nc, int n, const float *uob, float *ub, const float *pob, float *pb,
+                               const float *tob, float *tb, int nbv, float *bvb, int nsb, float *sbb, cudaStream_t st) {
+    if (!active) return 0;
+    int m = nc * n;
+    if (nbv > m) m = nbv;
+    if (nsb > m) m = nsb;
+    k_adj_inactive<<<dim3((unsigned)((m + 255) / 256), (unsigned)B), 256, 0, st>>>(active, nc, n, uob, ub, pob, pb, tob, tb, nbv, bvb, nsb, sbb);
+    const cudaError_t ce = cudaGetLastError();
+    return ce == cudaSuccess ? 0 : set_err(FGB_E_CUDA, "k_adj_inactive launch", ce);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -3719,9 +3763,10 @@ static int copy_async(void *dst, const void *src, size_t bytes, cudaStream_t st)
     return ce == cudaSuccess ? FGB_OK : set_err(FGB_E_CUDA, "cudaMemcpyAsync (tape)", ce);
 }
 
-// fgb_piso_substep that additionally records the tape the backward pass needs (every environment active).
+// fgb_piso_substep that additionally records the tape the backward pass needs, for the environments of tp->active (NULL: all).
 // C = corrector_steps, n_adv / n_p = advect / pressure non-orthogonal iterations (1 / 1 on the orthogonal path).
-// sc / stp: passive scalar + buoyancy (RBC), both or neither.
+// sc / stp: passive scalar + buoyancy (RBC), both or neither.  A skipped environment is the identity: every kernel and solve
+// leaves its u, p (and T) alone, the final u <- ures copy is masked; its tape rows hold whatever the copies found and are never read.
 static int record_impl(fgb_batch *b, float *u, float *p, const float *bvel, const float *dt, const fgb_tape *tp,
                        const fgb_scalar *sc, const fgb_tape_scalar *stp, fgb_stream_t s) {
     const fgb_options &o = b->opt;
@@ -3734,6 +3779,7 @@ static int record_impl(fgb_batch *b, float *u, float *p, const float *bvel, cons
         return set_err(FGB_E_ARG, "fgb_piso_substep_record: needs cg_impl 3 or 6 and correctors x pressure iterations <= 8");
     cudaStream_t st = STREAM(s);
     const size_t B = b->B, N = b->t.N, NB = b->t.NB;
+    const int32_t *act = tp->active;
     int rc;
     if ((rc = copy_async(tp->u_in, u, 2 * B * N * 4, st))) return rc;
     if ((rc = copy_async(tp->p_in, p, B * N * 4, st))) return rc;
@@ -3747,16 +3793,16 @@ static int record_impl(fgb_batch *b, float *u, float *p, const float *bvel, cons
         if ((rc = copy_async(stp->sbval_in, sc->sbval, B * NB * 4, st))) return rc;
         {
             ProfScope ps(b, CLS_ASM, st);
-            k_setup_scalar<<<cell_grid(b), 256, 0, st>>>(b->t, u, sc->T, bvel, sc->sbval, dt, nullptr, b->Coff, b->A, b->rhs);
+            k_setup_scalar<<<cell_grid(b), 256, 0, st>>>(b->t, u, sc->T, bvel, sc->sbval, dt, act, b->Coff, b->A, b->rhs);
             LAUNCH_CHECK("k_setup_scalar");
         }
         {
             ProfScope ps(b, CLS_BICG, st);
-            if ((rc = run_bicgstab<1>(b, b->rhs, sc->T, 1, nullptr, st))) return rc;
+            if ((rc = run_bicgstab<1>(b, b->rhs, sc->T, 1, act, st))) return rc;
         }
         if ((rc = copy_async(stp->T_out, sc->T, B * N * 4, st))) return rc;
         b->launches++;
-        k_buoyancy<<<cell_grid(b), 256, 0, st>>>(sc->T, sc->beta, (int)N, nullptr, sc->src);
+        k_buoyancy<<<cell_grid(b), 256, 0, st>>>(sc->T, sc->beta, (int)N, act, sc->src);
         LAUNCH_CHECK("k_buoyancy");
         src = sc->src;
     }
@@ -3765,26 +3811,30 @@ static int record_impl(fgb_batch *b, float *u, float *p, const float *bvel, cons
     // so that env.step(differentiable=True) reproduces the reference's differentiable run, which on the airfoil differs visibly from
     // its plain run (the deferred-correction pressure solves restart from zero and stop at residual ~4e-4).
     for (int k = 0; k < n_adv; ++k) {
-        if ((rc = fgb_setup_advection(b, u, k == 0 ? u : b->ures, bvel, src, dt, nullptr, s))) return rc;
-        if ((rc = fgb_solve_advection(b, 1, nullptr, s))) return rc;
+        if ((rc = fgb_setup_advection(b, u, k == 0 ? u : b->ures, bvel, src, dt, act, s))) return rc;
+        if ((rc = fgb_solve_advection(b, 1, act, s))) return rc;
         if ((rc = copy_async(tp->ustar + (size_t)k * 2 * B * N, b->ures, 2 * B * N * 4, st))) return rc;
     }
     if ((rc = copy_async(tp->Coff, b->Coff, 4 * B * N * 4, st))) return rc;
     if ((rc = copy_async(tp->A, b->A, B * N * 4, st))) return rc;
-    if ((rc = fgb_setup_pressure_matrix(b, nullptr, s))) return rc;
+    if ((rc = fgb_setup_pressure_matrix(b, act, s))) return rc;
     for (int cs = 0; cs < C; ++cs) {
         for (int ps = 0; ps < n_p; ++ps) {
             const int q = cs * n_p + ps;
-            if ((rc = fgb_setup_pressure_rhs(b, u, bvel, src, p, dt, ps == 0, nullptr, s))) return rc;
-            if ((rc = solve_pressure_slot(b, p, 1, reset, o.max_iter, q, nullptr, s))) return rc;
+            if ((rc = fgb_setup_pressure_rhs(b, u, bvel, src, p, dt, ps == 0, act, s))) return rc;
+            if ((rc = solve_pressure_slot(b, p, 1, reset, o.max_iter, q, act, s))) return rc;
             if ((rc = copy_async(tp->p + (size_t)q * B * N, p, B * N * 4, st))) return rc;
             if ((rc = copy_async(tp->pmean + (size_t)q * B, b->pmean + (size_t)q * B, B * 4, st))) return rc;
         }
         if ((rc = copy_async(tp->hb + (size_t)cs * 2 * B * N, b->hbya, 2 * B * N * 4, st))) return rc;
-        if ((rc = fgb_correct_velocity(b, p, b->ures, nullptr, s))) return rc;
+        if ((rc = fgb_correct_velocity(b, p, b->ures, act, s))) return rc;
         if (cs + 1 < C && (rc = copy_async(tp->u1 + (size_t)cs * 2 * B * N, b->ures, 2 * B * N * 4, st))) return rc;
     }
-    return copy_async(u, b->ures, 2 * B * N * 4, st);
+    if (!act) return copy_async(u, b->ures, 2 * B * N * 4, st);
+    b->launches++;
+    k_copy_active<<<dim3((unsigned)((2 * N + 255) / 256), b->B), 256, 0, st>>>(b->ures, u, (int)(2 * N), act);
+    LAUNCH_CHECK("k_copy_active (record)");
+    return FGB_OK;
 }
 extern "C" int fgb_piso_substep_record(fgb_batch *b, float *u, float *p, const float *bvel, const float *dt, const fgb_tape *tp,
                                        fgb_stream_t s) {
@@ -3804,7 +3854,8 @@ extern "C" size_t fgb_adjoint_workspace_bytes(const fgb_tables *t, int32_t B) {
 }
 
 // Reverse pass of fgb_piso_substep_record.  u_out_bar / p_out_bar: incoming gradients; u_bar, p_prev_bar, bvel_bar
-// are OVERWRITTEN with the gradients w.r.t. the inputs of the substep.  ws: >= fgb_adjoint_workspace_bytes.
+// are OVERWRITTEN with the gradients w.r.t. the inputs of the substep.  ws: >= fgb_adjoint_workspace_bytes.  Environments that
+// tp->active skips are skipped by every adjoint kernel and transposed solve and get the identity cotangents (k_adj_inactive).
 static int backward_impl(fgb_batch *b, const fgb_tape *tp, const fgb_tape_scalar *stp, float beta, const float *u_out_bar,
                          const float *p_out_bar, const float *T_out_bar, float *u_bar, float *p_prev_bar, float *bvel_bar,
                          float *T_bar, float *sbval_bar, void *ws, size_t ws_bytes, fgb_stream_t s) {
@@ -3816,6 +3867,7 @@ static int backward_impl(fgb_batch *b, const fgb_tape *tp, const fgb_tape_scalar
     if (!b->t.rev) return set_err(FGB_E_ARG, "fgb_piso_substep_backward: tables.rev missing");
     cudaStream_t st = STREAM(s);
     const size_t B = b->B, N = b->t.N, NB = b->t.NB, BN = B * N;
+    const int32_t *act = tp->active;
     Carver c{(char *)ws, 0};
     float *unb = c.take<float>(2 * BN), *hbb = c.take<float>(2 * BN), *rAb = c.take<float>(BN), *Coffb = c.take<float>(4 * BN);
     float *Sbb = c.take<float>(2 * BN), *pb = c.take<float>(BN), *xb = c.take<float>(BN), *lam = c.take<float>(BN);
@@ -3833,37 +3885,37 @@ static int backward_impl(fgb_batch *b, const fgb_tape *tp, const fgb_tape_scalar
     if ((rc = copy_async(pb, p_out_bar, BN * 4, st))) return rc;
     // the pressure matrix of this substep (function of A only)
     b->launches++;
-    k_setup_pressure_matrix<<<grid, 256, 0, st>>>(b->t, tp->A, nullptr, b->Poff, b->Pdiag);
+    k_setup_pressure_matrix<<<grid, 256, 0, st>>>(b->t, tp->A, act, b->Poff, b->Pdiag);
     LAUNCH_CHECK("k_setup_pressure_matrix (backward)");
     for (int cs = C - 1; cs >= 0; --cs) {
         const float *hb_c = tp->hb + (size_t)cs * 2 * BN;
         const float *uprev = cs == 0 ? tp->ustar + (size_t)(n_adv - 1) * 2 * BN : tp->u1 + (size_t)(cs - 1) * 2 * BN;
         b->launches++;
         // u_next = hb - rA grad(p of the last pressure iteration): hbb = unb, rAb +=, pb += grad^T
-        k_adj_correct<<<grid, 256, 0, st>>>(b->t, unb, tp->p + (size_t)(cs * n_p + n_p - 1) * BN, tp->A, hbb, rAb, pb);
+        k_adj_correct<<<grid, 256, 0, st>>>(b->t, unb, tp->p + (size_t)(cs * n_p + n_p - 1) * BN, tp->A, hbb, rAb, pb, act);
         LAUNCH_CHECK("k_adj_correct");
         for (int ps = n_p - 1; ps >= 0; --ps) {
             const int q = cs * n_p + ps;
             // the pressure the deferred term of this solve read: previous iteration, previous corrector, or the input
             const float *pprev = q == 0 ? tp->p_in : tp->p + (size_t)(q - 1) * BN;
             b->launches++;
-            k_adj_remove_mean<256><<<b->B, 256, 0, st>>>((int)N, pb, xb);
+            k_adj_remove_mean<256><<<b->B, 256, 0, st>>>((int)N, pb, xb, act);
             LAUNCH_CHECK("k_adj_remove_mean");
             {   // lam = P^-T x_bar
                 ProfScope psc(b, CLS_CG, st);
-                rc = cg_cluster_mb_any(b, b->Poff, b->Pdiag, xb, lam, 1, 0, b->opt.max_iter, 5, nullptr, 1 | 2, nullptr, st);
+                rc = cg_cluster_mb_any(b, b->Poff, b->Pdiag, xb, lam, 1, 0, b->opt.max_iter, 5, act, 1 | 2, nullptr, st);
                 if (rc == 1) return set_err(FGB_E_ARG, "fgb_piso_substep_backward: grid too large for the on-chip transposed solve");
                 if (rc) return rc;
             }
             ZERO(pb2, BN);                 // becomes the gradient w.r.t. pprev
             b->launches++;
-            k_adj_pressure_rhs<<<grid, 256, 0, st>>>(b->t, lam, tp->p + (size_t)q * BN, tp->pmean + (size_t)q * B, pprev, tp->A, hbb, Fbb, rAb, pb2);
+            k_adj_pressure_rhs<<<grid, 256, 0, st>>>(b->t, lam, tp->p + (size_t)q * BN, tp->pmean + (size_t)q * B, pprev, tp->A, hbb, Fbb, rAb, pb2, act);
             LAUNCH_CHECK("k_adj_pressure_rhs");
             float *tmp = pb; pb = pb2; pb2 = tmp;      // the previous iterate enters only through that deferred term
         }
         ZERO(uprevb, 2 * BN);
         b->launches++;
-        k_adj_hbya<<<grid, 256, 0, st>>>(b->t, hbb, hb_c, tp->A, tp->Coff, uprev, tp->dt, rAb, u_bar, Sbb, Coffb, uprevb);
+        k_adj_hbya<<<grid, 256, 0, st>>>(b->t, hbb, hb_c, tp->A, tp->Coff, uprev, tp->dt, rAb, u_bar, Sbb, Coffb, uprevb, act);
         LAUNCH_CHECK("k_adj_hbya");
         float *tmp = unb; unb = uprevb; uprevb = tmp;   // gradient w.r.t. the velocity entering this corrector
     }
@@ -3873,19 +3925,19 @@ static int backward_impl(fgb_batch *b, const fgb_tape *tp, const fgb_tape_scalar
     for (int k = n_adv - 1; k >= 0; --k) {
         {   // mu = C^-T x_k_bar
             ProfScope psc(b, CLS_BICG, st);
-            rc = bicgstab_cluster_any<2>(b, tp->Coff, tp->A, xb_cur, mu, 1, nullptr, 1, st);
+            rc = bicgstab_cluster_any<2>(b, tp->Coff, tp->A, xb_cur, mu, 1, act, 1, st);
             if (rc == 1) return set_err(FGB_E_ARG, "fgb_piso_substep_backward: grid too large for the on-chip transposed solve");
             if (rc) return rc;
         }
         if (k > 0) ZERO(xb_prev, 2 * BN);
         b->launches++;
         k_adj_advection<<<grid, 256, 0, st>>>(b->t, mu, tp->ustar + (size_t)k * 2 * BN, rAb, tp->A, tp->dt, Ab, Coffb, u_bar, Sbb, bvel_bar,
-                                              k > 0 ? xb_prev : u_bar, k == n_adv - 1);
+                                              k > 0 ? xb_prev : u_bar, k == n_adv - 1, act);
         LAUNCH_CHECK("k_adj_advection");
         float *tmp = xb_cur; xb_cur = xb_prev; xb_prev = tmp;
     }
     b->launches += 2;
-    k_adj_assemble<<<grid, 256, 0, st>>>(b->t, Ab, Coffb, Sbb, tp->bvel_in, u_bar, bvel_bar, Fbb);
+    k_adj_assemble<<<grid, 256, 0, st>>>(b->t, Ab, Coffb, Sbb, tp->bvel_in, u_bar, bvel_bar, Fbb, act);
     LAUNCH_CHECK("k_adj_assemble");
     if (stp) {
         // buoyancy + scalar transport (they ran BEFORE the predictor): T_new_bar from the source adjoint, one transposed
@@ -3893,24 +3945,26 @@ static int backward_impl(fgb_batch *b, const fgb_tape *tp, const fgb_tape_scalar
         // rebuilt from the taped inputs into the forward workspace (Coff / A / rhs are not read by this pass).
         float *Tnb = xb;
         b->launches += 3;
-        k_adj_buoyancy<<<grid, 256, 0, st>>>(b->t, Sbb, T_out_bar, beta, Tnb);
+        k_adj_buoyancy<<<grid, 256, 0, st>>>(b->t, Sbb, T_out_bar, beta, Tnb, act);
         LAUNCH_CHECK("k_adj_buoyancy");
-        k_setup_scalar<<<grid, 256, 0, st>>>(b->t, tp->u_in, stp->T_in, tp->bvel_in, stp->sbval_in, tp->dt, nullptr, b->Coff, b->A, b->rhs);
+        k_setup_scalar<<<grid, 256, 0, st>>>(b->t, tp->u_in, stp->T_in, tp->bvel_in, stp->sbval_in, tp->dt, act, b->Coff, b->A, b->rhs);
         LAUNCH_CHECK("k_setup_scalar (backward)");
         {
             ProfScope psc(b, CLS_BICG, st);
-            rc = bicgstab_cluster_any<1>(b, b->Coff, b->A, Tnb, lam, 1, nullptr, 1, st);
+            rc = bicgstab_cluster_any<1>(b, b->Coff, b->A, Tnb, lam, 1, act, 1, st);
             if (rc == 1) return set_err(FGB_E_ARG, "fgb_piso_substep_backward_scalar: grid too large for the on-chip transposed solve");
             if (rc) return rc;
         }
         ZERO(sbval_bar, B * NB);
-        k_adj_scalar<<<grid, 256, 0, st>>>(b->t, lam, stp->T_out, tp->bvel_in, stp->sbval_in, tp->dt, T_bar, sbval_bar, Fbb, u_bar);
+        k_adj_scalar<<<grid, 256, 0, st>>>(b->t, lam, stp->T_out, tp->bvel_in, stp->sbval_in, tp->dt, T_bar, sbval_bar, Fbb, u_bar, act);
         LAUNCH_CHECK("k_adj_scalar");
     }
-    k_adj_bflux<<<dim3((unsigned)((NB + 127) / 128), b->B), 128, 0, st>>>(b->t, Fbb, bvel_bar);
+    k_adj_bflux<<<dim3((unsigned)((NB + 127) / 128), b->B), 128, 0, st>>>(b->t, Fbb, bvel_bar, act);
     LAUNCH_CHECK("k_adj_bflux");
 #undef ZERO
-    return FGB_OK;
+    if (act) b->launches++;
+    return launch_adj_inactive(act, b->B, 2, (int)N, u_out_bar, u_bar, p_out_bar, p_prev_bar, stp ? T_out_bar : nullptr, stp ? T_bar : nullptr,
+                               (int)(2 * NB), bvel_bar, stp ? (int)NB : 0, stp ? sbval_bar : nullptr, st);
 }
 extern "C" int fgb_piso_substep_backward(fgb_batch *b, const fgb_tape *tp, const float *u_out_bar, const float *p_out_bar,
                                          float *u_bar, float *p_prev_bar, float *bvel_bar, void *ws, size_t ws_bytes, fgb_stream_t s) {

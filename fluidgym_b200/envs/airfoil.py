@@ -53,7 +53,9 @@ class Airfoil2DEnv(EpisodeLifecycle, DifferentiableRollout, InitialDomains, Rend
 
     def __init__(self, n_envs: int = 1, reynolds_number=3e3, dt=0.05, step_length=0.25, adaptive_cfl=0.8, episode_length=300,
                  attack_angle_deg=10.0, device="cuda:0", cg_impl=6, compiled=None, cl_cd_ref=0.0, randomize_initial_state=False,
-                 enable_actions=True, use_marl=False, differentiable=False, load_initial_domain=False, initial_domains_path=None):
+                 enable_actions=True, use_marl=False, differentiable=False, load_initial_domain=False, initial_domains_path=None,
+                 per_env_substeps: bool = False):
+        self.per_env_substeps = bool(per_env_substeps)
         if attack_angle_deg < 0.0 or attack_angle_deg > 20.0:
             raise ValueError("Attack angle must be between 0 and 20 degrees.")
         if use_marl:
@@ -265,6 +267,7 @@ class Airfoil2DEnv(EpisodeLifecycle, DifferentiableRollout, InitialDomains, Rend
         acc = torch.zeros(self.n_envs, 2, device=self.device)
         nsub = 0
         free = self.free_mask.bool()
+        self._begin_substep_count()
         for _ in range(self.n_sim_steps):
             last = last + self.action_smoothing_alpha * (action - last)
             if self.enable_actions:

@@ -43,8 +43,9 @@ class Airfoil3DEnv(SpanwiseExtrudedEnv):
     def __init__(self, n_envs: int = 1, n_agents=4, reynolds_number=3e3, dt=0.05, adaptive_cfl=0.8, step_length=0.25, episode_length=200,
                  attack_angle_deg=10.0, local_obs_window=1, use_marl=False, local_reward_weight=0.5, local_2d_obs=False, init_from_2d=False,
                  device="cuda:0", cl_cd_ref=0.0, randomize_initial_state=False, enable_actions=True, load_initial_domain=False,
-                 initial_domains_path=None, compiled=None, solver_cls=None, res_z=None, differentiable=False):
-        self.differentiable = bool(differentiable)       # reverse mode of the extruded substep (SpanwiseExtrudedEnv._advance_differentiable)
+                 initial_domains_path=None, compiled=None, solver_cls=None, res_z=None, differentiable=False, per_env_substeps: bool = False):
+        self.differentiable = bool(differentiable)
+        self.per_env_substeps = bool(per_env_substeps)       # reverse mode of the extruded substep (SpanwiseExtrudedEnv._advance_differentiable)
         if res_z is not None:
             self.res_z = int(res_z)                                     # tests only: the reference's value is fixed
         if n_agents < 1 or self.res_z % n_agents != 0:

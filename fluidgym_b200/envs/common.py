@@ -13,7 +13,7 @@ import torch
 
 from .. import native
 from ..sensors import cell_centres
-from ..solver import _ptr, cfl_substeps
+from ..solver import _ptr, cfl_substeps, cfl_substeps_per_env
 
 
 def build_wall_tables(cd, spec, ring, device, scale: float):
@@ -76,7 +76,9 @@ class EpisodeLifecycle:
     _reset_called = False
     _seed = None
     _n_steps = 0
-    last_substeps = 0
+    last_substeps = 0               # substep rounds launched by the last step (every environment's count in plain mode)
+    last_substeps_per_env = None    # int64 [B]: each environment's substeps in the last per-environment differentiable step
+    per_env_substeps = False        # differentiable mode: every environment follows its own CFL plan (see _substep_rounds)
     _dstate = None          # differentiable mode: the state tensors carried with their autograd history
 
     @property
@@ -127,6 +129,20 @@ class EpisodeLifecycle:
         """fluid_env.py ``detach()``: cut the autograd graph at the current state."""
         if self._dstate is not None:
             self._dstate = tuple(t.detach() for t in self._dstate)
+
+    def _begin_substep_count(self):
+        """start of a differentiable step: ``last_substeps_per_env`` counts from zero with per-environment plans, else it is None"""
+        self.last_substeps_per_env = torch.zeros(self.n_envs, dtype=torch.int64, device=self.device) if self.per_env_substeps else None
+
+    def _substep_rounds(self, max_velocity_env):
+        """The substep rounds of one solver step of a differentiable rollout with ``per_env_substeps``: every environment follows its own
+        adaptive CFL plan (``solver.cfl_substeps_per_env``, the plan plain mode uses), so an environment of a batch takes the substeps it
+        would take alone.  ``max_velocity_env()`` -> float32 [B] of the current state.  Yields ``(dt [B], active [B])``; environments with
+        ``active == 0`` have used up their time and must pass through the round unchanged."""
+        s = self.solver
+        for dtv, act in cfl_substeps_per_env(s.lib, self.n_envs, self.dt, self.cfl, max_velocity_env, self.device, s.stream):
+            self.last_substeps_per_env += act
+            yield dtv, act
 
 
 class DifferentiableRollout:
@@ -182,7 +198,7 @@ class DifferentiableRollout:
         return bv * scale[:, None, :]
 
     def _outflow_torch(self, u, bv, dt, bc_tol=1e-5):
-        """k_plan_substep's boundary part (SIM.py:188-224, 282-393).  The reference runs update_advective_boundaries entirely
+        """k_plan_substep's boundary part (SIM.py:188-224, 282-393); ``dt`` a float or a per-environment [B, 1, 1] tensor.  The reference runs update_advective_boundaries entirely
         under ``torch.no_grad()`` (SIM.py:232), including the setVelocity of the relaxed and rescaled outflow values: the outflow
         faces carry no gradient (neither to the adjacent cells nor to their previous values), all other faces keep theirs."""
         tb = self._diff_tables()
@@ -217,18 +233,26 @@ class DifferentiableRollout:
     def _single_step_differentiable(self, u, p, bv):
         """Simulation.single_step with the adaptive CFL plan of SIM.py:2004-2031; the plan itself is not
         differentiated (the reference computes it from detached maxima as well).  One common substep size is
-        used for the batch (the most restrictive environment decides)."""
+        used for the batch (the most restrictive environment decides), or with ``per_env_substeps`` every
+        environment's own plan (environments that are done keep their state and boundary values)."""
         from ..autograd import piso_substep
         s = self.solver
         mvb = torch.empty(self.n_envs, device=self.device)
+        tol = getattr(self, "bc_tol", 1e-5)
 
-        def max_velocity():
+        def max_velocity_env():
             native.check(self.lib.fgb_max_velocity(s.handle, _ptr(u.detach().contiguous()), _ptr(bv.detach().contiguous()), _ptr(mvb),
                                                    s.stream), "fgb_max_velocity")
-            return float(mvb.max())
+            return mvb
         nsub = 0
-        for ts in cfl_substeps(self.dt, self.cfl, max_velocity):
-            bv = self._outflow_torch(u, bv, ts, getattr(self, "bc_tol", 1e-5))
+        if self.per_env_substeps:
+            for dtv, act in self._substep_rounds(max_velocity_env):
+                bv = torch.where(act.bool()[:, None, None], self._outflow_torch(u, bv, dtv[:, None, None], tol), bv)
+                u, p = piso_substep(s, u, p, bv, dtv, active=act)
+                nsub += 1
+            return u, p, bv, nsub
+        for ts in cfl_substeps(self.dt, self.cfl, lambda: float(max_velocity_env().max())):
+            bv = self._outflow_torch(u, bv, ts, tol)
             u, p = piso_substep(s, u, p, bv, ts)
             nsub += 1
         return u, p, bv, nsub

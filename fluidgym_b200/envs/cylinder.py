@@ -95,9 +95,10 @@ class CylinderJet2DEnv(EpisodeLifecycle, DifferentiableRollout, InitialDomains, 
     def __init__(self, n_envs: int = 1, reynolds_number=1e2, resolution=24, dt=1e-2, adaptive_cfl=0.8, step_length=0.25,
                  episode_length=80, lift_penalty=1.0, device="cuda:0", cg_impl=11, compiled=None, cd_ref=0.0,
                  randomize_initial_state=False, enable_actions=True, use_marl=False, differentiable=False, load_initial_domain=False,
-                 initial_domains_path=None):
+                 initial_domains_path=None, per_env_substeps: bool = False):
         if use_marl:
             raise ValueError("CylinderJet2D is a single-agent environment (n_agents == 1)")
+        self.per_env_substeps = bool(per_env_substeps)
         self.n_envs = int(n_envs)
         self.resolution, self.dt, self.cfl = int(resolution), float(dt), float(adaptive_cfl)
         self.step_length, self.episode_length = float(step_length), int(episode_length)
@@ -290,6 +291,7 @@ class CylinderJet2DEnv(EpisodeLifecycle, DifferentiableRollout, InitialDomains, 
         a = action.reshape(self.n_envs)
         acc = torch.zeros(self.n_envs, 2, device=self.device)
         nsub = 0
+        self._begin_substep_count()
         for _ in range(self.n_sim_steps):
             if self.enable_actions:
                 last = last + self.action_smoothing_alpha * (a - last)

@@ -160,7 +160,8 @@ class SpanwiseExtrudedEnv(EpisodeLifecycle, InitialDomainsExtruded, Renderable):
     # ---- differentiable mode: one autograd node per substep (autograd.PISOSubstepExtruded, CUDA adjoint of the extruded path); the
     # boundary hooks, the jets and the wall forces around it are functional torch expressions with the graph cut where the reference
     # cuts it: update_advective_boundaries runs entirely under no_grad (SIM.py:232), balance_boundary_fluxes computes its scale under
-    # no_grad and applies it outside (SIM.py:191-224).  One common substep size for the batch (the most restrictive environment decides).
+    # no_grad and applies it outside (SIM.py:191-224).  One common substep size for the batch (the most restrictive environment decides), or
+    # with per_env_substeps every environment's own plan (EpisodeLifecycle._substep_rounds).
     differentiable = False
 
     def mark_state_differentiable(self):
@@ -204,7 +205,20 @@ class SpanwiseExtrudedEnv(EpisodeLifecycle, InitialDomainsExtruded, Renderable):
                 return float(torch.stack([(mi[0] * u4[:, 0] + mi[1] * u4[:, 1]).abs().max(), (mi[2] * u4[:, 0] + mi[3] * u4[:, 1]).abs().max(),
                                           u4[:, 2].abs().max() / s.hz, (bm[0] * bv[:, 0] + bm[1] * bv[:, 1]).abs().max(),
                                           (bm[2] * bv[:, 0] + bm[3] * bv[:, 1]).abs().max(), bv[:, 2].abs().max() / s.hz]).max())
+
+        def max_velocity_env():                     # the same maxima per environment (ExtrudedStepping.max_velocity of u, bv)
+            with torch.no_grad():
+                u4, mi, bm = u.view(self.n_envs, 3, self.nz, s.N2), st["minv"], st["b_minv"]
+                return torch.stack([(mi[0] * u4[:, 0] + mi[1] * u4[:, 1]).abs().amax(dim=(1, 2)), (mi[2] * u4[:, 0] + mi[3] * u4[:, 1]).abs().amax(dim=(1, 2)),
+                                    u4[:, 2].abs().amax(dim=(1, 2)) / s.hz, (bm[0] * bv[:, 0] + bm[1] * bv[:, 1]).abs().amax(dim=(1, 2)),
+                                    (bm[2] * bv[:, 0] + bm[3] * bv[:, 1]).abs().amax(dim=(1, 2)), bv[:, 2].abs().amax(dim=(1, 2)) / s.hz]).amax(dim=0)
         nsub = 0
+        if self.per_env_substeps:
+            for dtv, act in self._substep_rounds(max_velocity_env):
+                bv = torch.where(act.bool()[:, None, None, None], self._outflow_fn(u, bv, dtv, self.bc_tol), bv)
+                u, p = piso_substep_extruded(s, u, p, bv, dtv, active=act)
+                nsub += 1
+            return u, p, bv, nsub
         for ts in cfl_substeps(self.dt, self.cfl, max_velocity):                                   # SIM.py:2004-2031
             dtv = torch.full((self.n_envs,), ts, device=self.device)
             bv = self._outflow_fn(u, bv, dtv, self.bc_tol)
@@ -222,6 +236,7 @@ class SpanwiseExtrudedEnv(EpisodeLifecycle, InitialDomainsExtruded, Renderable):
         cls_ = torch.zeros_like(cds)
         jf = self.jet_faces.long()
         nsub = 0
+        self._begin_substep_count()
         for _ in range(self.n_sim_steps):
             last = last + self.action_smoothing_alpha * (a - last)
             if self.enable_actions:
@@ -289,9 +304,10 @@ class CylinderJet3DEnv(SpanwiseExtrudedEnv):
     def __init__(self, n_envs: int = 1, n_jets=8, reynolds_number=1e2, resolution=24, dt=1e-2, adaptive_cfl=0.8, step_length=0.25,
                  episode_length=80, lift_penalty=1.0, local_obs_window=3, use_marl=False, local_reward_weight=0.8, local_2d_obs=False,
                  device="cuda:0", cd_ref=0.0, randomize_initial_state=False, enable_actions=True, load_initial_domain=False,
-                 initial_domains_path=None, compiled=None, solver_cls=None, differentiable=False):
+                 initial_domains_path=None, compiled=None, solver_cls=None, differentiable=False, per_env_substeps: bool = False):
         self.load_domain_on_reset, self.initial_domains_path = bool(load_initial_domain), initial_domains_path
         self.differentiable = bool(differentiable)
+        self.per_env_substeps = bool(per_env_substeps)
         if n_jets < 1 or resolution % n_jets != 0:
             raise ValueError("n_agents must be a positive integer that evenly dividescircle_resolution_angular.")
         if local_2d_obs and not use_marl:

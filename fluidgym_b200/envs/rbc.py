@@ -50,7 +50,8 @@ class RBC2DEnv(EpisodeLifecycle, InitialDomains, Renderable):
                  adaptive_cfl=0.8, step_length=1.0, episode_length=200, local_obs_window=11, local_reward_weight=0.2,
                  uniform_grid=False, aspect_ratio=1.0, use_marl=False, device="cuda:0", cg_impl=6, nu_ref=0.0,
                  randomize_initial_state=False, enable_actions=True, load_initial_domain=False, initial_domains_path=None,
-                 differentiable=False):
+                 differentiable=False, per_env_substeps: bool = False):
+        self.per_env_substeps = bool(per_env_substeps)
         self.n_envs = int(n_envs)
         self.Ra, self.Pr = float(rayleigh_number), float(prandtl_number)
         self.n_heaters, self.heater_width = int(n_heaters), int(resolution)
@@ -263,7 +264,8 @@ class RBC2DEnv(EpisodeLifecycle, InitialDomains, Renderable):
     # One autograd node per substep (scalar transport + buoyancy + PISO, fluidgym_b200.autograd.PISOSubstepScalar backed by
     # the CUDA adjoint); the heater profile (rbc_env_2d.py:210-282) and the Nusselt sums (rbc_env_base.py:491-539) around it
     # are torch expressions, as in the reference.  The CFL plan is taken from detached maxima with one common substep size
-    # for the batch (the most restrictive environment decides): solver.cfl_substeps.
+    # for the batch (the most restrictive environment decides): solver.cfl_substeps; with per_env_substeps every environment
+    # follows its own plan (EpisodeLifecycle._substep_rounds).
     def _advance_differentiable(self, action):
         from ..autograd import piso_substep_scalar
         s = self.solver
@@ -276,12 +278,18 @@ class RBC2DEnv(EpisodeLifecycle, InitialDomains, Renderable):
         bv = s.bvel
         mvb = torch.empty(self.n_envs, device=self.device)
 
-        def max_velocity():
+        def max_velocity_env():
             native.check(self.lib.fgb_max_velocity(s.handle, _ptr(u.detach().contiguous()), _ptr(bv), _ptr(mvb), s.stream), "fgb_max_velocity")
-            return float(mvb.max())
+            return mvb
         nsub = 0
+        self._begin_substep_count()
         for _ in range(self.n_sim_steps):
-            for ts in cfl_substeps(self.dt, self.cfl, max_velocity):                 # SIM.py:2004-2031
+            if self.per_env_substeps:
+                for dtv, act in self._substep_rounds(max_velocity_env):
+                    u, p, T = piso_substep_scalar(s, u, p, bv, T, sb, dtv, self.buoyancy_factor, active=act)
+                    nsub += 1
+                continue
+            for ts in cfl_substeps(self.dt, self.cfl, lambda: float(max_velocity_env().max())):                 # SIM.py:2004-2031
                 u, p, T = piso_substep_scalar(s, u, p, bv, T, sb, ts, self.buoyancy_factor)
                 nsub += 1
         self._dstate = (u, p, T, sb)

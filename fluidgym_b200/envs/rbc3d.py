@@ -68,7 +68,8 @@ class RBC3DEnv(EpisodeLifecycle, InitialDomains3D, Renderable):
                  adaptive_cfl=0.8, step_length=1.0, episode_length=200, local_obs_window=3, local_reward_weight=0.0015,
                  uniform_grid=False, aspect_ratio=1.0, use_marl=True, device="cuda:0", nu_ref=0.0, randomize_initial_state=False,
                  enable_actions=True, load_initial_domain=False, initial_domains_path=None, transforms=None, btransforms=None,
-                 differentiable=False):
+                 differentiable=False, per_env_substeps: bool = False):
+        self.per_env_substeps = bool(per_env_substeps)
         self.n_envs = int(n_envs)
         self.differentiable = bool(differentiable)
         self.load_domain_on_reset, self.initial_domains_path = bool(load_initial_domain), initial_domains_path
@@ -312,7 +313,8 @@ class RBC3DEnv(EpisodeLifecycle, InitialDomains3D, Renderable):
 
     # ---- differentiable mode: one autograd node per substep (autograd.PISOSubstepScalar3D, CUDA adjoint of the D = 3 box path); the
     # heater profile and the Nusselt integrals around it are torch expressions, as in the reference.  The CFL plan is taken from
-    # detached maxima with one common substep size for the batch (the most restrictive environment decides).
+    # detached maxima with one common substep size for the batch (the most restrictive environment decides), or with per_env_substeps
+    # every environment's own plan (EpisodeLifecycle._substep_rounds).
     def mark_state_differentiable(self):
         """envs/util/diff_tools.py:8-22: (velocity, temperature) leaves of the incoming state"""
         s = self.solver
@@ -335,8 +337,18 @@ class RBC3DEnv(EpisodeLifecycle, InitialDomains3D, Renderable):
         def max_velocity():
             with torch.no_grad():
                 return float(torch.maximum((minv * u).abs().max(), (b_minv * bv).abs().max()))
+
+        def max_velocity_env():
+            with torch.no_grad():
+                return torch.maximum((minv * u).abs().amax(dim=(1, 2)), (b_minv * bv).abs().amax(dim=(1, 2)))
         nsub = 0
+        self._begin_substep_count()
         for _ in range(self.n_sim_steps):
+            if self.per_env_substeps:
+                for dtv, act in self._substep_rounds(max_velocity_env):
+                    u, p, T = piso_substep_scalar_3d(s, u, p, bv, T, sb, dtv, active=act)
+                    nsub += 1
+                continue
             for ts in cfl_substeps(self.dt, self.cfl, max_velocity):                 # SIM.py:2004-2031
                 u, p, T = piso_substep_scalar_3d(s, u, p, bv, T, sb, ts)
                 nsub += 1

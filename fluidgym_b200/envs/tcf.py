@@ -50,7 +50,9 @@ class TCF3DEnv(EpisodeLifecycle, InitialDomains3D, Renderable):
     def __init__(self, n_envs: int = 1, resolution_y=65, resolution_x_z=64, actor_size=2, L=np.pi, D=np.pi / 2, reynolds_number_wall=180,
                  adaptive_cfl=0.1, step_length=0.6, episode_length=1000, local_obs_window=1, local_reward_weight=0.0, use_marl=True,
                  C_smag=0.0, use_van_driest=False, init_with_noise=False, device="cuda:0", tau_ref=1.0, randomize_initial_state=False,
-                 enable_actions=True, domain=None, load_initial_domain=False, initial_domains_path=None, differentiable=False):
+                 enable_actions=True, domain=None, load_initial_domain=False, initial_domains_path=None, differentiable=False,
+                 per_env_substeps: bool = False):
+        self.per_env_substeps = bool(per_env_substeps)
         if init_with_noise:
             raise NotImplementedError("init_with_noise needs the reference's optional simplex-noise extension; start from a state instead")
         self.n_envs = int(n_envs)
@@ -272,16 +274,25 @@ class TCF3DEnv(EpisodeLifecycle, InitialDomains3D, Renderable):
 
     def _single_step_differentiable(self, u, p, bv):
         """Simulation.single_step with the adaptive CFL plan (SIM.py:2004-2031, k3_plan_substep); the plan is not differentiated.
-        One common substep size for the batch (the most restrictive environment decides)."""
+        One common substep size for the batch (the most restrictive environment decides), or with ``per_env_substeps`` every
+        environment's own plan."""
         from ..autograd import piso_substep_3d
         s = self.solver
         minv = s._tab["minv"].reshape(1, 3, -1)
         b_minv = s._tab["b_minv"].reshape(1, 3, -1)
+        nsub = 0
+        if self.per_env_substeps:
+            def max_velocity_env():
+                with torch.no_grad():
+                    return torch.maximum((minv * u).abs().amax(dim=(1, 2)), (b_minv * bv).abs().amax(dim=(1, 2)))
+            for dtv, act in self._substep_rounds(max_velocity_env):
+                u, p = piso_substep_3d(s, u, p, bv, dtv, self._forcing_torch(u), active=act)
+                nsub += 1
+            return u, p, nsub
 
         def max_velocity():
             with torch.no_grad():
                 return float(torch.maximum((minv * u).abs().max(), (b_minv * bv).abs().max()))
-        nsub = 0
         for ts in cfl_substeps(self.dt, self.cfl, max_velocity):
             u, p = piso_substep_3d(s, u, p, bv, ts, self._forcing_torch(u))
             nsub += 1
@@ -311,6 +322,7 @@ class TCF3DEnv(EpisodeLifecycle, InitialDomains3D, Renderable):
                 hi = torch.stack([hi[:, 0], -1 * self._action_to_control(a[:, half:].reshape(self.n_envs, self.nax, self.naz)), hi[:, 2]], dim=1)
                 bv = torch.cat([bv[:, :, :self._face_hi.start], hi, bv[:, :, self._face_hi.stop:]], dim=2)
         tb, tt, nsub = [], [], 0
+        self._begin_substep_count()
         for _ in range(self.n_sim_steps):
             u, p, n = self._single_step_differentiable(u, p, bv)
             nsub += n

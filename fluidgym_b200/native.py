@@ -31,11 +31,11 @@ class Tables(C.Structure):
 
 
 class Tape(C.Structure):
-    _fields_ = [(k, C.c_void_p) for k in ("u_in", "p_in", "bvel_in", "dt", "Coff", "A", "ustar", "hb", "p", "pmean", "u1")]
+    _fields_ = [(k, C.c_void_p) for k in ("u_in", "p_in", "bvel_in", "dt", "Coff", "A", "ustar", "hb", "p", "pmean", "u1", "active")]
 
 
 class Ortho3Tape(C.Structure):
-    _fields_ = [(k, C.c_void_p) for k in ("u_in", "bvel_in", "dt", "Coff", "A", "ustar", "hb", "p", "u1", "visc")]
+    _fields_ = [(k, C.c_void_p) for k in ("u_in", "bvel_in", "dt", "Coff", "A", "ustar", "hb", "p", "u1", "visc", "active")]
 
 
 class ScalarTape(C.Structure):
@@ -85,7 +85,7 @@ EXPORTS = ["fgb_last_error", "fgb_version", "fgb_workspace_bytes", "fgb_batch_cr
            "fgb_ortho3_solve_pressure", "fgb_ortho3_correct_velocity", "fgb_ortho3_piso_substep", "fgb_ortho3_make_divergence_free",
            "fgb_ortho3_sim_step", "fgb_ortho3_wall_rows", "fgb_ipc_alloc", "fgb_ipc_open", "fgb_ipc_close", "fgb_ipc_free",
            "fgb_ortho3_set_slab", "fgb_ortho3_slab_error", "fgb_ortho3_set_scalar", "fgb_ortho3_advect_scalar", "fgb_ortho3_set_sgs", "fgb_ortho3_sgs_viscosity", "fgb_ortho3_velocity_gradients", "fgb_ortho3_piso_substep_record", "fgb_ortho3_adjoint_workspace_bytes", "fgb_ortho3_piso_substep_backward", "fgb_ortho3_piso_substep_record_scalar", "fgb_ortho3_piso_substep_backward_scalar", "fgb_extruded3_piso_substep_record", "fgb_extruded3_adjoint_workspace_bytes", "fgb_extruded3_piso_substep_backward", "fgb_sample_sensors_n", "fgb_extruded3_piso_substep", "fgb_extruded3_make_divergence_free",
-           "fgb_extruded3_balance_fluxes", "fgb_extruded3_update_outflow", "fgb_extruded3_max_velocity", "fgb_extruded3_wall_forces", "fgb_extruded3_apply_jets", "fgb_render_gather", "fgb_render_colour"]
+           "fgb_extruded3_balance_fluxes", "fgb_extruded3_update_outflow", "fgb_extruded3_max_velocity", "fgb_extruded3_wall_forces", "fgb_extruded3_apply_jets", "fgb_render_gather", "fgb_render_colour", "fgb_plan_substep"]
 
 
 def lib_path() -> str:
@@ -220,6 +220,7 @@ def load():
     L.fgb_extruded3_max_velocity.argtypes = [C.POINTER(Extruded3Tables), i32, vp, vp, vp, vp]
     L.fgb_extruded3_apply_jets.argtypes = [C.POINTER(Extruded3Tables), i32, vp, vp, i32, vp, vp, i32, vp, vp, f32, vp]
     L.fgb_extruded3_wall_forces.argtypes = [C.POINTER(Extruded3Tables), i32, C.POINTER(Wall), vp, vp, vp, vp, vp]
+    L.fgb_plan_substep.argtypes = [i32, vp, vp, f32, vp, vp, vp, vp, vp]
     L.fgb_ipc_alloc.argtypes = [C.c_size_t, C.POINTER(vp), C.c_char_p]
     L.fgb_ipc_open.argtypes = [C.c_char_p, C.POINTER(vp)]
     L.fgb_ipc_close.argtypes = [vp]

@@ -36,12 +36,36 @@ def cfl_substep(remaining: float, cfl: float, max_vel: float) -> float:
 def cfl_substeps(dt: float, cfl: float, max_velocity):
     """The substeps of one solver step of length ``dt``: yields each size rounded to float32 (what the substep kernels take).
     ``max_velocity()`` returns the maximum velocity of the batch as a Python float and is called before every substep, so one
-    common size serves the whole batch (the most restrictive environment decides)."""
+    common size serves the whole batch (the most restrictive environment decides).  ``cfl_substeps_per_env`` plans every
+    environment on its own."""
     remaining = float(dt)
     while remaining > 0.0 and not abs(remaining) <= 1e-8:
         ts = cfl_substep(remaining, cfl, max_velocity())
         remaining -= ts
         yield float(np.float32(ts))
+
+
+def cfl_substeps_per_env(lib, B: int, dt: float, cfl: float, max_velocity, device, stream):
+    """The per-environment counterpart of ``cfl_substeps``: every environment follows its own adaptive CFL plan through one solver
+    step of length ``dt``, as ``fgb_sim_step`` plans plain steps.  ``max_velocity()`` returns the maximum velocity of every environment
+    (float32 [B] on ``device``) and is called before every round; the plan of the round comes from ``fgb_plan_substep`` (the same
+    arithmetic as ``cfl_substep``, float64 remainders on the device).  Yields ``(dt, active)`` per round -- float32 [B] substep sizes,
+    0 for environments whose time is used up, and the int32 [B] mask of the environments that take the substep -- until no
+    environment has time left.  The only host read is the round's 4-byte count of active environments, which also ends the loop
+    (``lib``: the loaded library; ``stream``: the ctypes stream handle the solver launches on)."""
+    remaining = torch.full((B,), float(dt), dtype=torch.float64, device=device)
+    nsub = torch.zeros(B, dtype=torch.int32, device=device)
+    count = torch.zeros(1, dtype=torch.int32, device=device)
+    while True:
+        mv = max_velocity().to(device=device, dtype=torch.float32).contiguous()
+        dtv = torch.empty(B, dtype=torch.float32, device=device)
+        active = torch.empty(B, dtype=torch.int32, device=device)
+        count.zero_()
+        native.check(lib.fgb_plan_substep(B, _ptr(mv), _ptr(remaining), float(cfl), _ptr(dtv), _ptr(active), _ptr(nsub), _ptr(count), stream),
+                     "fgb_plan_substep")
+        if int(count.item()) == 0:
+            return
+        yield dtv, active
 
 
 def cluster_shape(N: int, cg_impl: int = 6):

@@ -277,8 +277,12 @@ typedef struct fgb_tape {      /* C = corrector_steps, n_adv / n_p = advect / pr
     float *p;        /* [C*n_p][B][N]     pressure after every solve (mean removed) */
     float *pmean;    /* [C*n_p][B]        the removed means */
     float *u1;       /* [max(C-1,1)][B][2][N]  velocity after every corrector but the last */
+    const int32_t *active; /* [B] (0 = skip this environment) or NULL = every environment active.  Read by the recording and the
+                              backward call: a skipped environment is the identity (its outputs equal its inputs bit for bit, its
+                              cotangents are u_bar = u_out_bar, p_prev_bar = p_out_bar, T_bar = T_out_bar, bvel_bar = sbval_bar = 0)
+                              and its tape rows are neither written meaningfully nor read. */
 } fgb_tape;
-/* forward substep (non-orthogonal path, no passive scalar, all environments active, C * n_p <= 8) + tape */
+/* forward substep (non-orthogonal path, no passive scalar, the environments of tape->active, C * n_p <= 8) + tape */
 int fgb_piso_substep_record(fgb_batch *b, float *u, float *p, const float *bvel, const float *dt, const fgb_tape *tape,
                             fgb_stream_t s);
 /* bytes of scratch fgb_piso_substep_backward[_scalar] needs */
@@ -402,8 +406,10 @@ typedef struct fgb_ortho3_tape {
     float *u1;       /* [max(C-1,1)][B][3][N]  velocity after every corrector but the last */
     float *visc;     /* [B][N] per-cell viscosity of the substep when a sub-grid model is set (fgb_ortho3_set_sgs), else NULL: a constant of
                       * the graph, as in the reference, whose Smagorinsky op has no autograd wrapper */
+    const int32_t *active; /* [B] (0 = skip this environment) or NULL = every environment active; as fgb_tape.active (identity
+                              cotangents u_bar = u_out_bar, T_bar = T_out_bar, bvel_bar = sbval_bar = 0) */
 } fgb_ortho3_tape;
-/* forward substep of the D = 3 box (as fgb_ortho3_piso_substep) that also fills the tape (the forward() of the reference's autograd
+/* forward substep of the D = 3 box (as fgb_ortho3_piso_substep for the environments of tape->active) that also fills the tape (the forward() of the reference's autograd
  * Functions, PISOtorch_diff.py:624-1808) + bytes of scratch the backward needs */
 int fgb_ortho3_piso_substep_record(fgb_ortho3 *b, float *u, float *p, const float *bvel, const float *src, const float *dt,
                                    const fgb_ortho3_tape *tape, fgb_stream_t s);
@@ -430,6 +436,14 @@ int fgb_ortho3_sim_step(fgb_ortho3 *b, float *u, float *p, const float *bvel, fl
  * acc [B][2] (optional): += (tau_lo, tau_hi) */
 int fgb_ortho3_wall_rows(fgb_ortho3 *b, const float *u, const int32_t *rows, int n_row, float d_lo, float d_hi, int set_forcing,
                          float *acc, fgb_stream_t s);
+
+/* Adaptive CFL plan of one round (SIM.py:2004-2031, the arithmetic of fgb_sim_step's planner), one thread per environment, no solver
+ * handle: for every environment with time left (remaining > 0 and |remaining| > 1e-8) dt = the next substep size from maxvel and cfl,
+ * remaining -= dt, nsub += 1, active = 1 and counter[0] += 1; finished environments get dt = 0, active = 0.  maxvel [B] float, remaining
+ * [B] double, dt [B] float, active / nsub [B] int32, counter [1] int32 (not cleared by this call): all device pointers.  Lets a caller
+ * drive per-environment substeps of its own (differentiable rollouts: fluidgym_b200/solver.py::cfl_substeps_per_env). */
+int fgb_plan_substep(int32_t B, const float *maxvel, double *remaining, float cfl, float *dt, int32_t *active, int32_t *nsub,
+                     int32_t *counter, fgb_stream_t s);
 
 /* ---- slab decomposition of one large 3-D domain over the GPUs of a node (one process per GPU) -------------------------
  * Every rank owns nz/world z-planes.  All device memory the solver touches lives in ONE symmetric allocation per rank
