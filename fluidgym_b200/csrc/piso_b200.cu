@@ -14,6 +14,7 @@
 #include <string.h>
 #include <math.h>
 #include <new>
+#include <type_traits>
 
 #include "fluidgym_b200.h"
 
@@ -1541,8 +1542,15 @@ __global__ void __launch_bounds__(T, MINB) k_cg_cluster_mb(Tab t, const float *_
 // arrays safe: a CTA can only start exchange n+1 after every warp of every CTA has contributed to exchange n, i.e.
 // has consumed exchange n-1.  The best iterate (CG.cu:335-352) is kept in global scratch (written, never read, unless
 // the solve fails), thread-major and coalesced.
+// LAZY (cg_impl 11; false = cg_impl 13, the eager order) moves the bookkeeping that does not feed the recurrence off the
+// chain between the two exchanges, with the same floating-point operations on the same values (bit-identical results):
+//   * x += alpha p is deferred into the next direction update, which loads p_old for p = r + beta p anyway; between
+//     exchanges A and B only r is updated.  Every exit that leaves with the current iterate applies the update first;
+//   * the best iterate is stored only when it is about to be lost: on the first non-improving iteration after an
+//     improving run the registers (not yet advanced) still hold it.  A failed solve whose last iteration improved takes
+//     it from the registers.
 // ------------------------------------------------------------------------------------------------
-template <int T, int CPT, int CS, int MINB>
+template <int T, int CPT, int CS, int MINB, bool LAZY>
 __global__ void __launch_bounds__(T, MINB) k_cg_strip(Tab t, const float *__restrict__ Poff, const float *__restrict__ Pdiag,
                                                     const float *__restrict__ Rhs, float *__restrict__ Xout,
                                                     int maxit, float tol, int zero_init, int reset_steps, int slot,
@@ -1581,7 +1589,9 @@ __global__ void __launch_bounds__(T, MINB) k_cg_strip(Tab t, const float *__rest
     const float *rgp = rs + th1.y;                     // first remote ghost row of this thread in the receive buffer
     const uint32_t rm = (uint32_t)th1.z;               // remote ghost rows of this thread (bit k)
     const int32_t *cellp = t.st_cell + ((size_t)rank * T + tid) * CPT;
-    float *bestp = best + ((size_t)b * CS + rank) * T * CPT + tid;
+    // LAZY: volatile, or the compiler forwards the stored best iterate to the reload at the failure exit in CPT registers
+    // that stay live across the whole loop (and push the iteration into spills)
+    typename std::conditional<LAZY, volatile float, float>::type *bestp = best + ((size_t)b * CS + rank) * T * CPT + tid;
     const uint32_t bytesA = CS * 4u, bytesB = CS * 4u + 4u * (uint32_t)t.st_cnt[4 * rank];
     if (tid == 0) {
         mbar_init(mb_addr, 1); mbar_init(mb_addr + 8, 1);
@@ -1686,7 +1696,9 @@ __global__ void __launch_bounds__(T, MINB) k_cg_strip(Tab t, const float *__rest
         for (int k = 0; k < CPT; ++k) vp[k * S] = x[k];
         mirror_local_ghosts();
     };
-    auto new_direction = [&](float beta) {             // p = r + beta p in place in vs; remote ghost rows use the residual they received
+    // p = r + beta p in place in vs; remote ghost rows use the residual they received.  advance_x: also the deferred
+    // x += alpha p of the LAZY order, from the same load of p_old (ghost replicas too, so they stay equal to their owners)
+    auto new_direction = [&](float beta, float alpha, bool advance_x) {
         if (rm) {                                      // (r of a ghost row is zero otherwise: its coefficients are)
             int n = 0;
 #pragma unroll
@@ -1696,6 +1708,10 @@ __global__ void __launch_bounds__(T, MINB) k_cg_strip(Tab t, const float *__rest
         for (int k = 0; k < CPT; ++k) ap[k] = vp[k * S];   // (loads first: the stores below would otherwise serialise them; A p is dead here)
 #pragma unroll
         for (int k = 0; k < CPT; ++k) vp[k * S] = fmaf(beta, ap[k], r[k]);
+        if (advance_x) {
+#pragma unroll
+            for (int k = 0; k < CPT; ++k) x[k] = fmaf(alpha, ap[k], x[k]);
+        }
         if (rm) {
 #pragma unroll
             for (int k = 0; k < CPT; ++k) if (rm & (1u << k)) r[k] = 0.f;
@@ -1734,9 +1750,12 @@ __global__ void __launch_bounds__(T, MINB) k_cg_strip(Tab t, const float *__rest
 #pragma unroll
         for (int k = 0; k < CPT; ++k) bestp[k * T] = x[k];
         float rho = residual_norm2();
-        new_direction(0.f);                            // p = r (vs holds zeros or x0: 0 * finite + r)
+        new_direction(0.f, 0.f, false);                // p = r (vs holds zeros or x0: 0 * finite + r)
         float bestc = 0.f, lastc = 0.f; int best_it = -1, rising = 0;
         bool take_best = false;
+        bool pending = false;                          // LAZY: the best iterate is x + alpha p of this iteration, not stored yet
+        bool advance = false;                          // LAZY: the loop left with the current iterate, x += alpha p is still due
+        float alpha = 0.f;
         int until_reset = reset_steps > 0 ? reset_steps - 1 : -1;   // iterations left before the next residual reset
         for (int i = 0; i < maxit; ++i) {
             if (until_reset == 0) {
@@ -1749,14 +1768,14 @@ __global__ void __launch_bounds__(T, MINB) k_cg_strip(Tab t, const float *__rest
                 for (int k = 0; k < CPT; ++k) { const int c = cellp[k]; r[k] = (c >= 0 ? f[c] : 0.f) - ap[k]; }
                 __syncthreads();
                 rho = residual_norm2();
-                new_direction(0.f);
+                new_direction(0.f, 0.f, false);
             }
             --until_reset;
             const float pap = exchange(spmv(), 0u, parA, bytesA);
-            const float alpha = rho / pap;
+            alpha = rho / pap;
 #pragma unroll
             for (int k = 0; k < CPT; ++k) {
-                x[k] = fmaf(alpha, vp[k * S], x[k]);
+                if (!LAZY) x[k] = fmaf(alpha, vp[k * S], x[k]);
                 r[k] = fmaf(-alpha, ap[k], r[k]);
             }
             const float rr2 = residual_norm2();
@@ -1768,6 +1787,13 @@ __global__ void __launch_bounds__(T, MINB) k_cg_strip(Tab t, const float *__rest
             if (!stop) {
                 if (i == 0 || crit < bestc) {
                     bestc = crit; best_it = i;
+                    if (LAZY) pending = true;
+                    else {
+#pragma unroll
+                        for (int k = 0; k < CPT; ++k) bestp[k * T] = x[k];
+                    }
+                } else if (LAZY && pending) {          // x is not advanced yet: it is the iterate of best_it
+                    pending = false;
 #pragma unroll
                     for (int k = 0; k < CPT; ++k) bestp[k * T] = x[k];
                 }
@@ -1777,15 +1803,22 @@ __global__ void __launch_bounds__(T, MINB) k_cg_strip(Tab t, const float *__rest
                 else if (i == maxit - 1 || rising >= 100) stop = 2;
             }
             asm volatile("" : "+r"(stop));             // opaque: keeps the compiler from threading the exits apart again
-            if (stop) { take_best = stop == 2; break; }
+            if (stop) {
+                take_best = stop == 2 && !pending;     // (pending: this iteration improved, best_it == i, bestc == crit)
+                advance = LAZY && !take_best;
+                break;
+            }
             const float beta = rr2 / rho;
             rho = rr2;
-            new_direction(beta);
+            new_direction(beta, alpha, LAZY);
         }
         if (take_best) {
 #pragma unroll
             for (int k = 0; k < CPT; ++k) x[k] = bestp[k * T];
             used = best_it; fin = bestc;
+        } else if (advance) {
+#pragma unroll
+            for (int k = 0; k < CPT; ++k) x[k] = fmaf(alpha, vp[k * S], x[k]);
         }
     }
     float mean = 0.f;
@@ -1812,7 +1845,8 @@ __global__ void __launch_bounds__(T, MINB) k_cg_strip(Tab t, const float *__rest
 // An exchange is split in a non-blocking start (warp partials -> the LAST arriving warp of the CTA adds them in fixed order and
 // pushes one value to every CTA of the cluster) and a finish (wait on the transaction barrier, add the CS totals in rank
 // order), so the flight time of one system's reduction is covered by the other system's arithmetic.  Arithmetic, operation
-// order and stopping rules per system are those of k_cg_strip (bit-identical results); the two systems converge independently,
+// order and stopping rules per system are those of k_cg_strip with the eager bookkeeping order; results are NOT bit-identical to
+// cg_impl 11, whose layout (17 rows per thread, half the CTAs) sums the dot products in another order.  The two systems converge independently,
 // the faster one idles until both are done.  Same tables (strip_plan.py) with the shape (T, CPT) of this kernel.
 // ------------------------------------------------------------------------------------------------
 template <int E> struct EnvTag { static constexpr int value = E; };
@@ -3447,18 +3481,18 @@ static int launch_cg_cluster_mb(fgb_batch *b, const float *poff, const float *pd
     return FGB_OK;
 }
 
-template <int T, int CPT, int CS, int MINB>
+template <int T, int CPT, int CS, int MINB, bool LAZY>
 static int launch_cg_strip(fgb_batch *b, const float *poff, const float *pdiag, const float *rhs, float *p_out, int zero_init,
                            int reset_steps, int max_iter, int slot, const int32_t *active, int flags, float *mean_out,
                            cudaStream_t st) {
     if (b->t.st_cs != CS || b->t.st_T != T || b->t.st_cpt != CPT) return 1;
     if ((size_t)CS * T * CPT > (size_t)KRY_VECS * b->t.N)
-        return set_err(FGB_E_ARG, "cg_impl 11: domain too small for the best-iterate scratch (use cg_impl 6)");
+        return set_err(FGB_E_ARG, "cg_impl 11/13: domain too small for the best-iterate scratch (use cg_impl 6)");
     const size_t smem = ((size_t)5 * CPT * T + (size_t)b->t.st_slots + (size_t)b->t.st_gmax + (size_t)2 * CS + 2 * (T / 32) + 2) * sizeof(float) + 4 * 8 +
                         ((size_t)b->t.st_remax + (size_t)b->t.st_lemax) * 8;
     if (smem > 227 * 1024 || (b->t.st_slots & 3) || (b->t.st_gmax & 1))
-        return set_err(FGB_E_ARG, "cg_impl 11: strip plan does not fit in shared memory");
-    auto kern = k_cg_strip<T, CPT, CS, MINB>;
+        return set_err(FGB_E_ARG, "cg_impl 11/13: strip plan does not fit in shared memory");
+    auto kern = k_cg_strip<T, CPT, CS, MINB, LAZY>;
     cudaError_t ce = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (ce != cudaSuccess) return set_err(FGB_E_CUDA, "cudaFuncSetAttribute(k_cg_strip)", ce);
     if (CS > 8) {
@@ -3477,24 +3511,25 @@ static int launch_cg_strip(fgb_batch *b, const float *poff, const float *pdiag, 
     return FGB_OK;
 }
 
-template <int T, int CPT, int MINB>
+template <int T, int CPT, int MINB, bool LAZY>
 static int cg_strip_cs(fgb_batch *b, const float *poff, const float *pdiag, const float *rhs, float *p_out, int zero_init,
                        int reset_steps, int max_iter, int slot, const int32_t *active, int flags, float *mean_out, cudaStream_t st) {
-    int rc = launch_cg_strip<T, CPT, 1, MINB>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
-    if (rc == 1) rc = launch_cg_strip<T, CPT, 2, MINB>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
-    if (rc == 1) rc = launch_cg_strip<T, CPT, 4, MINB>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
-    if (rc == 1) rc = launch_cg_strip<T, CPT, 8, MINB>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
-    if (rc == 1) rc = launch_cg_strip<T, CPT, 16, MINB>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
+    int rc = launch_cg_strip<T, CPT, 1, MINB, LAZY>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
+    if (rc == 1) rc = launch_cg_strip<T, CPT, 2, MINB, LAZY>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
+    if (rc == 1) rc = launch_cg_strip<T, CPT, 4, MINB, LAZY>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
+    if (rc == 1) rc = launch_cg_strip<T, CPT, 8, MINB, LAZY>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
+    if (rc == 1) rc = launch_cg_strip<T, CPT, 16, MINB, LAZY>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
     return rc;
 }
 // instantiated shapes = fluidgym_b200/strip_plan.py::SHAPES: 4 / 2 / 1 co-resident CTAs per SM, 8 320 cells per SM in every case
+template <bool LAZY>
 static int cg_strip_any(fgb_batch *b, const float *poff, const float *pdiag, const float *rhs, float *p_out, int zero_init,
                         int reset_steps, int max_iter, int slot, const int32_t *active, int flags, float *mean_out, cudaStream_t st) {
-    int rc = cg_strip_cs<480, 17, 1>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
-    if (rc == 1) rc = cg_strip_cs<256, 17, 2>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
-    if (rc == 1) rc = cg_strip_cs<896, 9, 1>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
-    if (rc == 1) rc = cg_strip_cs<640, 13, 1>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
-    if (rc == 1) rc = cg_strip_cs<320, 13, 2>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
+    int rc = cg_strip_cs<480, 17, 1, LAZY>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
+    if (rc == 1) rc = cg_strip_cs<256, 17, 2, LAZY>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
+    if (rc == 1) rc = cg_strip_cs<896, 9, 1, LAZY>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
+    if (rc == 1) rc = cg_strip_cs<640, 13, 1, LAZY>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
+    if (rc == 1) rc = cg_strip_cs<320, 13, 2, LAZY>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
     return rc;
 }
 
@@ -3539,7 +3574,7 @@ static int cg_strip2_any(fgb_batch *b, const float *poff, const float *pdiag, co
     return rc;
 }
 
-static inline bool uses_halo_plan(int cg_impl) { return cg_impl == 6 || cg_impl == 11 || cg_impl == 12; }
+static inline bool uses_halo_plan(int cg_impl) { return cg_impl == 6 || cg_impl == 11 || cg_impl == 12 || cg_impl == 13; }
 
 static int cg_cluster_mb_any(fgb_batch *b, const float *poff, const float *pdiag, const float *rhs, float *p_out, int zero_init,
                              int reset_steps, int max_iter, int slot, const int32_t *active, int flags, float *mean_out, cudaStream_t st) {
@@ -3548,9 +3583,13 @@ static int cg_cluster_mb_any(fgb_batch *b, const float *poff, const float *pdiag
         if (rc == 1) return set_err(FGB_E_ARG, "cg_impl 12: no k_cg_strip2 instantiation for the shape (st_T, st_cpt, st_cs) of this strip plan");
         return rc;
     }
-    if (b->opt.cg_impl == 11 && b->t.st_thread && b->t.st_cell && b->t.st_rexp && b->t.st_lexp && b->t.st_cnt) {
-        const int rc = cg_strip_any(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
-        if (rc == 1) return set_err(FGB_E_ARG, "cg_impl 11: no k_cg_strip instantiation for the shape (st_T, st_cpt, st_cs) of this strip plan");
+    // 11: k_cg_strip with the iterate update deferred and the best iterate stored lazily; 13: the same kernel with the eager
+    // bookkeeping order (bit-identical results, kept for A/B measurements and as the in-tree reference of the reorder)
+    if ((b->opt.cg_impl == 11 || b->opt.cg_impl == 13) && b->t.st_thread && b->t.st_cell && b->t.st_rexp && b->t.st_lexp && b->t.st_cnt) {
+        const int rc = b->opt.cg_impl == 11
+            ? cg_strip_any<true>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st)
+            : cg_strip_any<false>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
+        if (rc == 1) return set_err(FGB_E_ARG, "cg_impl 11/13: no k_cg_strip instantiation for the shape (st_T, st_cpt, st_cs) of this strip plan");
         return rc;
     }
     if (b->opt.cg_impl == 8) {       // as 6 with 256-thread CTAs of 1792 cells, TWO co-resident CTAs per SM (of different environments):
@@ -3568,7 +3607,7 @@ static int cg_cluster_mb_any(fgb_batch *b, const float *poff, const float *pdiag
         if (rc == 1) rc = launch_cg_cluster_mb<16, 12, true, 256>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
         return rc;
     }
-    if (uses_halo_plan(b->opt.cg_impl)) {   // pushed halos: same cluster-size rule, gathers from local shared memory (11 without a strip plan = 6)
+    if (uses_halo_plan(b->opt.cg_impl)) {   // pushed halos: same cluster-size rule, gathers from local shared memory (11 / 13 without a strip plan = 6)
         int rc = launch_cg_cluster_mb<2, 6, true>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
         if (rc == 1) rc = launch_cg_cluster_mb<4, 7, true>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);
         if (rc == 1) rc = launch_cg_cluster_mb<8, 7, true>(b, poff, pdiag, rhs, p_out, zero_init, reset_steps, max_iter, slot, active, flags, mean_out, st);

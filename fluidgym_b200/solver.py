@@ -164,10 +164,11 @@ class BatchedPISO:
             self.tables.scalar_viscosity = float(cd.scalar_visc)
         else:
             self._tab["Cd_s"] = self._tab["sb_neumann"] = None
-        plan = halo_plan(np.asarray(cd.nbr), cd.N, 6 if cg_impl in (11, 12) else cg_impl)
+        plan = halo_plan(np.asarray(cd.nbr), cd.N, 6 if cg_impl in (11, 12, 13) else cg_impl)
         self.halo = plan
         self.strip = None
-        if cg_impl in (11, 12):              # register-blocked strip layout of the pressure CG (strip_plan.py); 6 when it does not apply
+        if cg_impl in (11, 12, 13):          # register-blocked strip layout of the pressure CG (strip_plan.py); 6 when it does not apply
+            # 13: k_cg_strip with the eager bookkeeping order of round 2 (bit-identical to 11, kept for A/B runs)
             from .strip_plan import pair_shape, plan_for_domain
             # 12: two environments per cluster (k_cg_strip2), half the rows per thread and environment
             sp = self.strip = plan_for_domain(cd, None, *pair_shape()) if cg_impl == 12 else plan_for_domain(cd)
