@@ -117,24 +117,35 @@ typedef struct fgb_options {
     int32_t nonortho;               /* 1: flags CENTER_MATRIX|DIRECT_MATRIX|DIAGONAL_RHS, 0: orthogonal */
     float adv_tol, p_tol;           /* 1e-5, 1e-5 : ||r||_2/sqrt(N) absolute (SIM.py:1096-1098)          */
     int32_t max_iter;               /* 5000 */
-    int32_t cg_impl;                /* 0: one CTA per environment, vectors in global memory
+    int32_t cg_impl;                /* pressure CG (and whether the advection BiCGStab runs on chip: 0 = never).
+                                       Every on-chip variant takes the smallest cluster that holds the grid and falls
+                                       through to 0 when none does (the pressure solve; BiCGStab likewise), except:
+                                       11 / 13 fail (FGB_E_ARG) on a grid smaller than the best-iterate scratch
+                                       (cluster x threads x rows per thread > 12 N), 12 fails on a strip plan it
+                                       has no instantiation for (1 or 16 CTAs).
+                                       0: one CTA per environment, vectors in global memory
                                        1: thread-block cluster per environment, vectors on chip,
                                           textbook recurrence (3 cluster barriers / iteration)
                                        2: as 1 with A*p from the recurrence Ap <- A*r + beta*Ap
                                           (mathematically identical, 2 cluster barriers / iteration)
                                        3: as 1 without cluster barriers: st.async + mbarrier transactions
                                           for the reductions, remote mbarrier arrive for the p hand-shake
-                                          (default, fastest)
                                        4: as 3 with x/r/p/neighbour table in shared memory, 2x cells per CTA
                                        5: as 4 with two co-resident CTAs per SM
                                        6: as 3 with PUSHED halos (tables.cg_slot/cg_exp): after updating the
                                           search direction every CTA st.async-es the cells its neighbours need into
                                           their shared memory, all stencil gathers become plain ld.shared
+                                          (default of BatchedPISO, RBC2D and Airfoil2D)
+                                       7: as 6 with 256-thread CTAs and twice the cells per thread
+                                       8: as 6 with 256-thread CTAs of 1792 cells, two co-resident CTAs per SM
                                        11: register-blocked strip layout (tables.st_*): TWO cross-CTA exchanges per
                                           iteration instead of three (the residual of the ghost cells travels with the
                                           partial sums of <r,r>, ghost replicas update p and x themselves), no per-cell
-                                          neighbour addresses, north/south neighbours in registers (default where the
-                                          domain has a strip plan; 6 otherwise)                                 */
+                                          neighbour addresses, north/south neighbours in registers (default of the
+                                          cylinder environments; 6 where the domain has no strip plan)
+                                       12: as 11 with two environments per cluster (k_cg_strip2, 2 / 4 / 8-CTA plans
+                                          only; any other plan is an error)
+                                       13: as 11 with the eager bookkeeping order (bit-identical to 11)          */
 } fgb_options;
 
 /* message of the last failed fgb_* call of the calling thread (the analogue of the reference's TORCH_CHECK text, BIND.cpp) */

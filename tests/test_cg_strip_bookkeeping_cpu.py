@@ -2,12 +2,15 @@
 the <p,Ap> and <r,r> reductions and stores every improving iterate as the best one; cg_impl 11 (LAZY) defers x += alpha p into
 the next direction update (same p_old, same operands), stores the best iterate only on the first non-improving iteration after
 an improving run (the registers are not advanced yet then) and applies the pending update on every exit that leaves with the
-current iterate.  Both orders are written here in float32 numpy with the same expressions, including the residual reset, the
-100-rising-steps cut-off and the iteration cap: solution, iteration count, criterion and best iterate must be bit-identical.
+current iterate.  Both orders are run here in float32 with the same expressions (oracle/krylov_eval.py, which the GPU tests
+also run in float64 as the reference of the kernels), including the residual reset, the 100-rising-steps cut-off and the
+iteration cap: solution, iteration count, criterion and best iterate must be bit-identical.
 (The GPU check of the kernels themselves: tests/test_gpu_cg_strip_lazy.py.)"""
 import numpy as np
 import pytest
 import scipy.sparse as sp
+
+import krylov_eval as ke
 
 f32 = np.float32
 
@@ -29,123 +32,21 @@ def _poisson(n, seed, consistent=True):
     return A, ((b - b.mean()) if consistent else b).astype(f32)
 
 
-def _crit(rr, n):
-    return f32(np.sqrt(rr)) * f32(1.0 / np.sqrt(f32(n)))
-
-
-def _start(A, f, x0):
-    x = x0.copy()
-    r = f.copy() if not x.any() else (f - A @ x).astype(f32)
-    return x, r, x.copy(), np.dot(r, r), r.copy()                          # x, r, best (x0 stored), rho, p
-
-
 def strip_cg_eager(A, f, x0, tol, reset_steps, maxit):
-    """statement order of k_cg_strip<..., LAZY = false> (cg_impl 13)"""
-    n = f.size
-    x, r, best, rho, p = _start(A, f, x0)
-    bestc = lastc = f32(0); best_it, rising, used, fin = -1, 0, -1, f32(0)
-    take_best = False
-    until_reset = reset_steps - 1 if reset_steps > 0 else -1
-    for i in range(maxit):
-        if until_reset == 0:
-            until_reset = reset_steps
-            r = (f - A @ x).astype(f32); rho = np.dot(r, r); p = r.copy()
-        until_reset -= 1
-        ap = (A @ p).astype(f32)
-        alpha = f32(rho / np.dot(p, ap))
-        x = (x + alpha * p).astype(f32)
-        r = (r - alpha * ap).astype(f32)
-        rr = np.dot(r, r)
-        crit = _crit(rr, n)
-        stop = 0 if np.isfinite(crit) else 1
-        used, fin = i, crit
-        if not stop:
-            if i == 0 or crit < bestc:
-                bestc, best_it, best = crit, i, x.copy()
-            rising = rising + 1 if (i > 0 and crit >= lastc) else 0
-            lastc = crit
-            if crit < tol:
-                stop = 1
-            elif i == maxit - 1 or rising >= 100:
-                stop = 2
-        if stop:
-            take_best = stop == 2
-            break
-        beta = f32(rr / rho); rho = rr
-        p = (r + beta * p).astype(f32)
-    if take_best:
-        x = best.copy(); used, fin = best_it, bestc
-    return x, used, fin, best
+    """statement order of k_cg_strip<..., LAZY = false> (cg_impl 13), mean kept"""
+    r = ke.cg(A, f, x0, tol, reset_steps, maxit, dtype=f32, flags=2)
+    return r.x, r.used, f32(r.fin), r.best
 
 
 def strip_cg_lazy(A, f, x0, tol, reset_steps, maxit):
-    """statement order of k_cg_strip<..., LAZY = true> (cg_impl 11)"""
-    n = f.size
-    x, r, best, rho, p = _start(A, f, x0)
-    bestc = lastc = f32(0); best_it, rising, used, fin = -1, 0, -1, f32(0)
-    take_best = pending = advance = False
-    alpha = f32(0)
-    until_reset = reset_steps - 1 if reset_steps > 0 else -1
-    for i in range(maxit):
-        if until_reset == 0:
-            until_reset = reset_steps
-            r = (f - A @ x).astype(f32); rho = np.dot(r, r); p = r.copy()
-        until_reset -= 1
-        ap = (A @ p).astype(f32)
-        alpha = f32(rho / np.dot(p, ap))
-        r = (r - alpha * ap).astype(f32)                                   # x waits for the direction update
-        rr = np.dot(r, r)
-        crit = _crit(rr, n)
-        stop = 0 if np.isfinite(crit) else 1
-        used, fin = i, crit
-        if not stop:
-            if i == 0 or crit < bestc:
-                bestc, best_it = crit, i
-                pending = True
-            elif pending:                                                  # x is still the iterate of best_it
-                pending = False
-                best = x.copy()
-            rising = rising + 1 if (i > 0 and crit >= lastc) else 0
-            lastc = crit
-            if crit < tol:
-                stop = 1
-            elif i == maxit - 1 or rising >= 100:
-                stop = 2
-        if stop:
-            take_best = stop == 2 and not pending
-            advance = not take_best
-            break
-        beta = f32(rr / rho); rho = rr
-        p_old = p
-        p = (r + beta * p_old).astype(f32)
-        x = (x + alpha * p_old).astype(f32)
-    if take_best:
-        x = best.copy(); used, fin = best_it, bestc
-    elif advance:
-        x = (x + alpha * p).astype(f32)
-    return x, used, fin, (x if pending else best)
+    """statement order of k_cg_strip<..., LAZY = true> (cg_impl 11), mean kept"""
+    r = ke.cg(A, f, x0, tol, reset_steps, maxit, dtype=f32, flags=2, lazy=True)
+    return r.x, r.used, f32(r.fin), r.best
 
 
 def _history(A, f, x0, reset_steps, maxit):
     """criterion of every iteration of an uncapped, unconverging run (both orders share the recurrence)"""
-    crits = []
-    n = f.size
-    x, r, _, rho, p = _start(A, f, x0)
-    until_reset = reset_steps - 1 if reset_steps > 0 else -1
-    for _ in range(maxit):
-        if until_reset == 0:
-            until_reset = reset_steps
-            r = (f - A @ x).astype(f32); rho = np.dot(r, r); p = r.copy()
-        until_reset -= 1
-        ap = (A @ p).astype(f32)
-        alpha = f32(rho / np.dot(p, ap))
-        x = (x + alpha * p).astype(f32)
-        r = (r - alpha * ap).astype(f32)
-        rr = np.dot(r, r)
-        crits.append(_crit(rr, n))
-        beta = f32(rr / rho); rho = rr
-        p = (r + beta * p).astype(f32)
-    return np.array(crits)
+    return ke.cg_history(A, f, x0, reset_steps, maxit, dtype=f32)[0]
 
 
 def _x0(n, warm, seed):
